@@ -55,7 +55,13 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--main-only", action="store_true",
                     help="only the timed step (for ncu runs): skips the variants, latency, e2e and CPU legs; prints a short line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy: a fixed, "
+                         "seeded sample of PSD rows, peak bins and decimated channels, at most 64 MB in all")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def peaks():
@@ -91,6 +97,42 @@ def synth_tile(nchan, S, seed):
     out[:, 0::2] += car
     out[:, 1::2] += sar
     return out
+
+
+def sample_rows(nrows, ncols, itemsize, budget, seed):
+    """A fixed, seeded set of rows (ascending) and a leading run of columns of an nrows x ncols
+    output, together at most `budget` bytes."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    k = int(min(nrows, max(1, budget // max(1, ncols * itemsize))))
+    rows = np.sort(rng.choice(nrows, k, replace=False))
+    return rows, int(min(ncols, budget // (k * itemsize)))
+
+
+# bytes per dumped file as stored (PSD float32, peak bins and decimated rows float64):
+# 60 MiB = 62.9e6 bytes in all, which leaves room for the .npy headers under 64 MB
+DUMP_BUDGET = {"psd": 24 << 20, "peak_bin": 4 << 20, "ds": 32 << 20}
+
+
+def dump_plan(batch, n, nchan, nds):
+    """{name: (rows, cols, itemsize)}: the sample dump_outputs takes of each output of the pump,
+    PSD [batch][n+2], peak bins [batch] and decimated rows [nchan][nds] complex."""
+    shapes = {"psd": (batch, n + 2, 4), "peak_bin": (batch, 1, 8), "ds": (nchan, nds, 16)}
+    return {k: sample_rows(r, c, size, DUMP_BUDGET[k], seed) + (size,)
+            for seed, (k, (r, c, size)) in enumerate(shapes.items(), 1)}
+
+
+def dump_outputs(out_dir, bank, d_psd, d_peak, batch, n):
+    """What the caller of jsdr_pump_receive_s16 receives from the last step, sampled by dump_plan."""
+    os.makedirs(out_dir, exist_ok=True)
+    ds = bank.read_ds()
+    plan = dump_plan(batch, n, ds.shape[0], ds.shape[1])
+    rows, cols, _ = plan["psd"]
+    psd = np.stack([d_psd.download(np.float32, cols, offset=int(r) * (n + 2) * 4) for r in rows])
+    rows, _, _ = plan["peak_bin"]
+    peak = d_peak.download(np.int32, batch)[rows].astype(np.float64)
+    rows, cols, _ = plan["ds"]
+    for name, v in (("psd", psd), ("peak_bin", peak), ("ds", ds[rows, :cols])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(v))
 
 
 class ClockSampler:
@@ -347,6 +389,8 @@ def main():
     ctx.profile(False)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, bank, d_psd, d_peak, batch, n)
     fft_ms = kern["fft"][0] / max(kern["fft"][1], 1)
     mix_ms = kern["mixdecim"][0] / max(kern["mixdecim"][1], 1)
     scout_ms = kern["scout"][0] / max(kern["scout"][1], 1)

@@ -26,14 +26,21 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback():
-    """Without a CUDA device context creation must fail, not fall back."""
-    lib = jsdrcuda.lib()
-    n = ctypes.c_int(-1)
-    rc = lib.jsdr_device_count(ctypes.byref(n))
-    if rc == 0 and n.value > 0:
-        pytest.skip("a GPU is present")
-    with pytest.raises(jsdrcuda.JsdrError):
-        jsdrcuda.Context(0)
+    """Without a CUDA device context creation must fail, not fall back.  In a child process
+    that sees no device (CUDA_VISIBLE_DEVICES empty), so that a machine with a GPU checks it too."""
+    import subprocess
+    import sys
+    code = r"""
+import jsdrcuda as J
+try:
+    J.Context(0)
+except J.JsdrError as e:
+    print("REFUSED", e)
+"""
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="",
+               PYTHONPATH=os.pathsep.join([os.path.dirname(os.path.dirname(jsdrcuda.__file__)), os.environ.get("PYTHONPATH", "")]))
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, timeout=300)
+    assert r.returncode == 0 and "REFUSED" in r.stdout, (r.returncode, r.stdout[-2000:], r.stderr[-2000:])
 
 
 def test_host_side_helpers_need_no_device():

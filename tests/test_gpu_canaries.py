@@ -51,8 +51,10 @@ def _dev(ctx, a):
                                      (32768, 3), (65536, 2)])
 @pytest.mark.parametrize("fmt", ["s16", "f32"])
 def test_fft_outputs_stay_inside(ctx, n, batch, fmt):
-    if not J.fft_supported(n):
-        pytest.skip(f"no plan for N={n}")
+    if not J.fft_supported(n):                 # no plan (777 = 3 * 7 * 37): refused before anything is written
+        with pytest.raises(J.JsdrError):
+            J.fft(ctx, None, J.AudioDescriptor(96000), max_batch=batch, n=n)
+        return
     rng = np.random.default_rng(n + batch)
     if fmt == "s16":
         x = rng.integers(-20000, 20000, (batch, 2 * n)).astype(np.int16)

@@ -2,7 +2,8 @@
 every FFM downcall descriptor in JsdrCuda.java names an exported symbol and has the argument
 count and the scalar/pointer kinds of the C ABI (taken from the ctypes signatures, which
 tests/test_abi.py ties to include/jsdrcuda.h); the patches against the reference are
-insert-only; and, where the reference checkout is present, they apply cleanly."""
+insert-only and well-formed; and, given a java-sdr checkout in JAVA_SDR_REFERENCE, they apply
+cleanly.  The upstream sources themselves are not vendored in this repository."""
 import os
 import re
 import shutil
@@ -15,7 +16,7 @@ import jsdrcuda as J
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 JAVA = os.path.join(ROOT, "java-sdr_b200", "java")
 SRC = os.path.join(JAVA, "com", "ashbysoft", "java_sdr")
-REF = "/root/reference"
+REF = os.environ.get("JAVA_SDR_REFERENCE", "")
 
 
 def _descriptors():
@@ -59,7 +60,35 @@ def test_patches_are_insert_only():
         assert not any(l.startswith("-") for l in body), f"{f} removes reference lines"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF) or shutil.which("patch") is None, reason="reference checkout not present")
+def test_patch_hunks_are_well_formed():
+    """What patch(1) checks before it reads the file it patches: every hunk holds exactly the
+    lines its header counts, and each hunk's new start is its old start shifted by the lines
+    the hunks before it insert."""
+    for f in ("fft.java.patch", "FUNcubeBPSKDemod.java.patch", "FECDecoder.java.patch"):
+        lines = open(os.path.join(JAVA, "patches", f)).read().splitlines()
+        assert lines[0].startswith("--- ") and lines[1].startswith("+++ "), f
+        i, shift, hunks = 2, 0, 0
+        while i < len(lines):
+            m = re.fullmatch(r"@@ -(\d+)(?:,(\d+))? \+(\d+)(?:,(\d+))? @@.*", lines[i])
+            assert m, f"{f}:{i + 1}: expected a hunk header"
+            o0, oc, n0, nc = int(m[1]), int(m[2] or 1), int(m[3]), int(m[4] or 1)
+            assert n0 == o0 + shift, f"{f}:{i + 1}: new start {n0}, expected {o0 + shift}"
+            i += 1
+            ro, rn = oc, nc
+            while ro > 0 or rn > 0:
+                assert i < len(lines), f"{f}: hunk ends early"
+                tag = lines[i][:1] or " "            # an empty line is blank context
+                assert tag in " +-", f"{f}:{i + 1}: not a hunk line"
+                ro -= tag != "+"
+                rn -= tag != "-"
+                assert ro >= 0 and rn >= 0, f"{f}:{i + 1}: more lines than the header counts"
+                i += 1
+            shift += nc - oc
+            hunks += 1
+        assert hunks, f
+
+
+@pytest.mark.skipif(not os.path.isdir(REF) or shutil.which("patch") is None, reason="needs a java-sdr checkout in JAVA_SDR_REFERENCE")
 def test_patches_apply_to_the_reference(tmp_path):
     for f in ("fft.java", "FUNcubeBPSKDemod.java", "FECDecoder.java"):
         shutil.copy(os.path.join(REF, f), tmp_path / f)

@@ -156,9 +156,7 @@ int jsdr_bpsk_set_precision(jsdr_bpsk *b, int precision);
 /* Kernel choice for the tuner + decimator (results are identical): AUTO picks the
  * streaming kernel (one lane per channel) for banks of >= 32 channels of s16 input
  * and the tile kernel (one CTA per channel tile) otherwise. */
-enum { JSDR_KERNEL_AUTO = 0, JSDR_KERNEL_TILE = 1, JSDR_KERNEL_STREAM = 2,
-       JSDR_KERNEL_PRING = 3 /* the streaming kernel with a period ring staged by bulk (TMA-engine) copies:
-                                identical results, measured slower; s16 input, rate/9600 = 20, aligned blocks */ };
+enum { JSDR_KERNEL_AUTO = 0, JSDR_KERNEL_TILE = 1, JSDR_KERNEL_STREAM = 2 };
 int jsdr_bpsk_set_kernel(jsdr_bpsk *b, int mode);
 /* replace the 27-tap decimator low-pass (BASELINE config 4 uses 64 taps); resets
  * the decimator history like a fresh instance */

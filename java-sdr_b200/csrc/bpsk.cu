@@ -513,7 +513,6 @@ __global__ void k_tuner_tail(const MixParams p)
 }  // namespace bpsk
 }  // namespace jsdr
 #include "bpsk_stream.cuh"
-#include "bpsk_stream2.cuh"
 namespace jsdr {
 namespace bpsk {
 
@@ -1088,27 +1087,6 @@ int launch_stream_shape(jsdr_bpsk *b, const stream::Params &sp)
     return launched(ctx, "k_mixdecim_stream");
 }
 
-// The period-ring form (bpsk_stream2.cuh): s16 input, D % 4 == 0, every period 16-byte aligned.
-template <int PREC, int NTAPS, int DD>
-int launch_pring_shape(jsdr_bpsk *b, const stream::Params &sp)
-{
-    jsdr_ctx *ctx = b->ctx;
-    constexpr int W = stream::kPWarps;
-    auto kern = stream::k_mixdecim_pring<PREC, NTAPS, DD>;
-    constexpr size_t smem = stream::p_smem_bytes<DD>();
-    static PerDeviceFlag attr_done;
-    JSDR_TRY(attr_done.once(ctx->device, [&]() -> int {
-        JSDR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        return JSDR_OK;
-    }));
-    const int warps = sp.ncw * sp.nseg;
-    const int grid = std::min((warps + W - 1) / W, sp.grid);
-    JSDR_CUDA(cudaMemsetAsync(sp.work_counter, 0, sizeof(unsigned), ctx->stream));
-    ProfScope prof(ctx, JSDR_K_MIXDECIM, ctx->stream);
-    kern<<<grid, W * 32, smem, ctx->stream>>>(sp);
-    return launched(ctx, "k_mixdecim_pring");
-}
-
 template <int FMT>
 int launch_stream(jsdr_bpsk *b, const MixParams &mp, int S)
 {
@@ -1155,22 +1133,6 @@ int launch_stream(jsdr_bpsk *b, const MixParams &mp, int S)
         sp.tapsf[k] = (float)sp.taps[k];
     }
     const bool f32 = b->precision == JSDR_PREC_F32;
-    if constexpr (FMT == FMT_S16) {
-        // The period-ring form staged by bulk (TMA-engine) copies, bpsk_stream2.cuh: bit-identical
-        // but SLOWER than the chunk ring (5.03 against 3.90 ms per 2^31 samples in the pump; 4.60 ms
-        // with 16-byte cp.async copies instead of the bulk ones), so it only runs when asked for:
-        // jsdr_bpsk_set_kernel(JSDR_KERNEL_PRING) or JSDR_PRING=1.  It needs every period to start
-        // on a 16-byte boundary in every row; otherwise the chunk ring runs.
-        static int use_pring = -1;
-        if (use_pring < 0) use_pring = env_int("JSDR_PRING", 0, 1, 0);
-        const bool aligned = ((reinterpret_cast<size_t>(sp.in) & 15) == 0) && ((sp.chan_stride & 3) == 0) &&
-                             (((sp.n0 + 1) & 3) == 0);
-        if ((use_pring || b->kernel_mode == JSDR_KERNEL_PRING) && aligned && mp.D == 20 && (sp.ic | sp.qc) == 0) {
-            if (b->ntaps == 27)
-                return f32 ? launch_pring_shape<stream::PREC_F32, 27, 20>(b, sp) : launch_pring_shape<stream::PREC_F64, 27, 20>(b, sp);
-            return f32 ? launch_pring_shape<stream::PREC_F32, 64, 20>(b, sp) : launch_pring_shape<stream::PREC_F64, 64, 20>(b, sp);
-        }
-    }
     if (b->ntaps == 27 && mp.D == 10)
         return f32 ? launch_stream_shape<FMT, stream::PREC_F32, 27, 10>(b, sp) : launch_stream_shape<FMT, stream::PREC_F64, 27, 10>(b, sp);
     if (b->ntaps == 27 && mp.D == 20)
@@ -1331,7 +1293,7 @@ int bpsk_receive(jsdr_bpsk *b, const void *in, int S, long long chan_stride, int
     if (NO > 0 && b->kernel_mode != JSDR_KERNEL_TILE) {
         // many channels: the streaming kernel (bpsk_stream.cuh); needs a compiled (taps, D) shape
         const bool shape_ok = (b->ntaps == 27 && D == 10) || (b->ntaps == 27 && D == 20) || (b->ntaps == 64 && D == 20);
-        const bool want = b->kernel_mode == JSDR_KERNEL_STREAM || b->kernel_mode == JSDR_KERNEL_PRING || (nchan >= 32 && NO >= 64) ||
+        const bool want = b->kernel_mode == JSDR_KERNEL_STREAM || (nchan >= 32 && NO >= 64) ||
                           (b->precision == JSDR_PREC_F32 && nchan >= 8);
         if (shape_ok && want) {
             JSDR_TRY(launch_stream<FMT>(b, mp, P.S));
@@ -1634,7 +1596,7 @@ try {
 
 extern "C" int jsdr_bpsk_set_kernel(jsdr_bpsk *b, int mode)
 try {
-    JSDR_REQUIRE(b && mode >= JSDR_KERNEL_AUTO && mode <= JSDR_KERNEL_PRING, JSDR_EINVAL, "bad kernel mode");
+    JSDR_REQUIRE(b && mode >= JSDR_KERNEL_AUTO && mode <= JSDR_KERNEL_STREAM, JSDR_EINVAL, "bad kernel mode");
     b->kernel_mode = mode;
     return JSDR_OK;
 } JSDR_CATCH_ALL

@@ -32,10 +32,7 @@ namespace jsdr {
 namespace bpsk {
 namespace stream {
 
-#ifndef JSDR_STREAM_WARPS
-#define JSDR_STREAM_WARPS 16
-#endif
-constexpr int kWarps = JSDR_STREAM_WARPS;   // s16 input: 16 warps (one CTA per SM: 231552 B of shared memory, 128 registers); the macro is an occupancy probe
+constexpr int kWarps = 16;            // s16 input: one CTA per SM (231552 B of shared memory, 128 registers); fewer warps do not help (DESIGN.md §9)
 constexpr int kWarpsF32 = 8;          // float input: the ring rows are twice as wide
 constexpr int kMaxTaps = 64;
 enum { PREC_F64 = 0, PREC_F32 = 1 };
@@ -255,11 +252,7 @@ __device__ __forceinline__ void period_body(const Params &p, const typename Raw<
 }
 
 template <int FMT, int PREC, int NTAPS, int DD, int W>
-#ifdef JSDR_STREAM_MAXNREG      // (experiment: leave registers for a co-resident phase-scout warp)
-__global__ void __maxnreg__(JSDR_STREAM_MAXNREG) k_mixdecim_stream(const Params p)
-#else
 __global__ void __launch_bounds__(W * 32, 1) k_mixdecim_stream(const Params p)
-#endif
 {
     typedef typename Raw<FMT>::type raw_t;
     constexpr int NQ = (NTAPS + DD - 1) / DD;          // live outputs per sample

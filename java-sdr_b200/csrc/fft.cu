@@ -1,7 +1,5 @@
 // fft.cu — host side of the fft.java replacement (jsdr_fft_* in jsdrcuda.h).
-#include <cstring>
 #include <math.h>
-#include <stdio.h>
 #include <stdlib.h>
 
 #include <algorithm>
@@ -23,16 +21,9 @@ namespace fft {
 JSDR_FFT_PLANS(DECL)
 #undef DECL
 
-int launch_split_n8192(jsdr_ctx *ctx, const Args &a, int in_fmt, int out_mode, cudaStream_t st);
-int launch_split_n9600(jsdr_ctx *ctx, const Args &a, int in_fmt, int out_mode, cudaStream_t st);
 int launch_split_n16384(jsdr_ctx *ctx, const Args &a, int in_fmt, int out_mode, cudaStream_t st);
 
 typedef int (*launch_fn)(jsdr_ctx *, const Args &, int, int, cudaStream_t);
-// measured (profiles/r02_fft_split.txt): 32768 as 2 x 16384 beats the four-step pair (0.278 / 0.424
-// against 0.256 / 0.355 of peak for s16 / float input); 16384 as 2 x 8192 and 19200 as 2 x 9600 do
-// not beat their whole-block plans (the second read and conversion of every sample and the
-// strided stores cost what the second CTA per SM gains)
-static const char kDefaultSplit[] = "32768";
 struct PlanEntry { int n; launch_fn fn; };
 static const PlanEntry kPlans[] = {
 #define ROW(N, T, G, R0, R1, R2, R3) {N, launch_n##N},
@@ -50,23 +41,11 @@ static const PlanEntry *find_plan(int n)
 
 // Lengths that run as a split plan: two CTAs per block, each an n/2-point plan behind one
 // radix-2 decimation-in-frequency step folded into its loads (fft_kernel, SPLIT = 2).
-// JSDR_FFT_SPLIT="19200,16384" overrides the default list, "0" turns it off (A/B measurements).
-static launch_fn split_plan(int n)
-{
-    static const char *env = getenv("JSDR_FFT_SPLIT");
-    const char *list = env ? env : kDefaultSplit;
-    char want[16];
-    snprintf(want, sizeof(want), "%d", n);
-    const char *hit = strstr(list, want);
-    const size_t len = strlen(want);
-    if (!hit || (hit != list && hit[-1] != ',') || (hit[len] != 0 && hit[len] != ',')) return nullptr;
-    switch (n) {
-    case 16384: return launch_split_n8192;
-    case 19200: return launch_split_n9600;
-    case 32768: return launch_split_n16384;
-    }
-    return nullptr;
-}
+// Measured (profiles/r02_fft_split.txt): 32768 as 2 x 16384 beats the four-step pair (0.278 / 0.424
+// against 0.256 / 0.355 of peak for s16 / float input); 16384 as 2 x 8192 and 19200 as 2 x 9600 do
+// not beat their whole-block plans (the second read and conversion of every sample and the
+// strided stores cost what the second CTA per SM gains).
+static launch_fn split_plan(int n) { return n == 32768 ? launch_split_n16384 : nullptr; }
 
 // ---- lengths without a single-CTA plan: fft_generic.cuh stages + a PSD pass -------------
 __global__ void __launch_bounds__(256) k_generic_load(const void *__restrict__ in, float2 *__restrict__ out, long long total,

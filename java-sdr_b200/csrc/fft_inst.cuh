@@ -1,8 +1,6 @@
 // fft_inst.cuh — one translation unit per FFT length includes this with
 // JSDR_FFT_N etc. defined, so the plans compile in parallel.
 #pragma once
-#include <stdlib.h>
-
 #include <algorithm>
 
 #include "fft_kernels.cuh"
@@ -15,11 +13,8 @@ static int launch_one(jsdr_ctx *ctx, const Args &a, cudaStream_t st)
 {
     static PerDeviceFlag attr_done;
     auto kern = fft_kernel<P, IN, OUT, SPLIT>;
-    // JSDR_FFT_EXTRA_SMEM_KB: unused shared memory added to every CTA (occupancy experiments only)
-    static const size_t extra = []() { const char *e = getenv("JSDR_FFT_EXTRA_SMEM_KB"); return e ? (size_t)std::max(0, atoi(e)) * 1024 : (size_t)0; }();
-    constexpr size_t base = (P::PERSIST && IN == IN_S16 && SPLIT == 1) ? P::SMEM_PERSIST
+    constexpr size_t smem = (P::PERSIST && IN == IN_S16 && SPLIT == 1) ? P::SMEM_PERSIST
                           : (P::TW_SMEM_NP && SPLIT == 1) ? P::SMEM_TW : P::SMEM;   // + twiddle tables
-    const size_t smem = std::min(base + extra, (size_t)227 * 1024);
     JSDR_TRY(attr_done.once(ctx->device, [&]() -> int {
         JSDR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         return JSDR_OK;

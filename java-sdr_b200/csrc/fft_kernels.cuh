@@ -163,11 +163,7 @@ __device__ __forceinline__ float2 cmul_w(float2 a)
 //   w = c*(1 + i*t):  u = b + t*(i*b);  a + c*u;  a - c*u        (|c| >= |s|, t = s/c)
 //   w = s*(i + t'):   u = i*b + t'*b;   a + s*u;  a - s*u        (otherwise,  t' = c/s)
 // (the multiply-add form of Linzer & Feig / Goedecker).  A 64-point DFT is 482 packed
-// instructions this way against 546 with the twiddles multiplied out; JSDR_FFT_FUSED_TW=0
-// builds the multiplied-out form for comparison.
-#ifndef JSDR_FFT_FUSED_TW
-#define JSDR_FFT_FUSED_TW 1
-#endif
+// instructions this way against 546 with the twiddles multiplied out.
 
 constexpr int pick_factor(int r)
 {
@@ -309,7 +305,6 @@ struct Dft<R, false> {
     template <int K, int RR>
     static __device__ __forceinline__ void run_tw(float2 *v)
     {
-#if JSDR_FFT_FUSED_TW
         static_assert(RR % R == 0, "sub-transform length divides the outer one");
         float2 t[R];
         static_for<0, B>([&](auto nn2) {
@@ -330,35 +325,6 @@ struct Dft<R, false> {
 #pragma unroll
             for (int k2 = 0; k2 < B; k2++) v[k1 + A * k2] = b[k2];
         });
-#else
-        if constexpr (mod_pos(K, RR) != 0) {
-            static_for<1, R>([&](auto nn) {
-                constexpr int n = decltype(nn)::value;
-                v[n] = cmul_w<K * n, RR>(v[n]);
-            });
-        }
-        float2 t[R];
-        static_for<0, B>([&](auto nn2) {
-            constexpr int n2 = decltype(nn2)::value;
-            float2 a[A];
-#pragma unroll
-            for (int n1 = 0; n1 < A; n1++) a[n1] = v[B * n1 + n2];
-            Dft<A>::run(a);
-            static_for<0, A>([&](auto kk1) {
-                constexpr int k1 = decltype(kk1)::value;
-                t[k1 * B + n2] = cmul_w<n2 * k1, R>(a[k1]);
-            });
-        });
-#pragma unroll
-        for (int k1 = 0; k1 < A; k1++) {
-            float2 b[B];
-#pragma unroll
-            for (int n2 = 0; n2 < B; n2++) b[n2] = t[k1 * B + n2];
-            Dft<B>::run(b);
-#pragma unroll
-            for (int k2 = 0; k2 < B; k2++) v[k1 + A * k2] = b[k2];
-        }
-#endif
     }
     static __device__ __forceinline__ void run(float2 *v) { run_tw<0, R>(v); }
 };
@@ -413,13 +379,7 @@ struct Plan {
     // hide the load phase behind other CTAs' butterflies.  Those plans run persistent CTAs that
     // fetch the next block's pass-0 samples into registers before the last pass of the current
     // one (s16 input: one register per sample).
-#ifndef JSDR_FFT_NO_PERSIST
-#define JSDR_FFT_NO_PERSIST 0
-#endif
-#ifndef JSDR_FFT_PERSIST_MIN_KB
-#define JSDR_FFT_PERSIST_MIN_KB 113
-#endif
-    static constexpr bool PERSIST = !JSDR_FFT_NO_PERSIST && (G_ == 1) && (N_ >= 9600) && (SMEM > JSDR_FFT_PERSIST_MIN_KB * 1024);   // one CTA per SM (113) or two (70: N = 9600)
+    static constexpr bool PERSIST = (G_ == 1) && (N_ >= 9600) && (SMEM > 113 * 1024);   // one CTA per SM (at two, N = 9600 is faster as ordinary CTAs)
     // CTAs per SM the kernel is compiled for: what shared memory allows, at the register budget
     // the largest register DFT needs.  Radix <= 16 fits 48 registers (4096 = 16^3 then keeps five
     // CTAs per SM instead of slipping to four); radix 32 fits 80, and a 256-thread CTA at 81..88
@@ -430,31 +390,24 @@ struct Plan {
     static constexpr int MINB_SMEM = (int)((227 * 1024) / (SMEM + 1024));
     static constexpr int MINB_REGS = 65536 / (T_ * REG_BUDGET);
     static constexpr int MINB_FIT = (MINB_SMEM < MINB_REGS ? MINB_SMEM : MINB_REGS) < 1 ? 1 : (MINB_SMEM < MINB_REGS ? MINB_SMEM : MINB_REGS);
-    static constexpr int MINB = PERSIST ? (MINB_SMEM > 1 ? MINB_SMEM : 0) : (RMAX > 32 || (RMAX & (RMAX - 1)) != 0) ? 0 : MINB_FIT;
+    static constexpr int MINB = (PERSIST || RMAX > 32 || (RMAX & (RMAX - 1)) != 0) ? 0 : MINB_FIT;
     // Persistent plans keep the twiddle bases of every pass in shared memory behind the block (the
     // block leaves room: one CTA per SM): R0 values for the first middle pass, R0*R1 for the
     // second, ML for the last -- a shared-memory load where every butterfly waited for L2.
-#ifndef JSDR_FFT_TW_SMEM
-#define JSDR_FFT_TW_SMEM 1
-#endif
     static constexpr int TW1 = (K >= 3) ? R0_ : 0;
     static constexpr int TW2 = (K >= 4) ? R0_ * R1_ : 0;
     static constexpr int TW_ELEMS = TW1 + TW2 + ML;
-    static constexpr bool TW_SMEM = JSDR_FFT_TW_SMEM && PERSIST && (SMEM + TW_ELEMS * sizeof(float2) + 2048 <= 227 * 1024);
+    static constexpr bool TW_SMEM = PERSIST && (SMEM + TW_ELEMS * sizeof(float2) + 2048 <= 227 * 1024);
     static constexpr size_t SMEM_PERSIST = SMEM + (TW_SMEM ? TW_ELEMS * sizeof(float2) : 0);
     // The same tables for the ordinary (one CTA per block) three- and four-pass plans, where they
     // cost no CTA per SM: each thread fetches its share into registers before pass 0 and stores
     // it to shared memory behind pass 0, so the fetch hides behind the pass-0 loads.
-#ifndef JSDR_FFT_TW_SMEM_NP
-#define JSDR_FFT_TW_SMEM_NP 1
-#endif
     static constexpr int TW_PER_THREAD = (TW_ELEMS + T_ - 1) / T_;
     // (N >= 8192 only: measured +5.7 % at 8192 and +4.3 % at 9600 for s16 input; at 4800 the extra
     // registers cost a CTA per SM, -8 %, and 2048 / 4410 do not move)
-    static constexpr bool TW_SMEM_NP = JSDR_FFT_TW_SMEM_NP && !PERSIST && G_ == 1 && K >= 3 && N_ >= 8192 && TW_PER_THREAD <= 4 &&
+    static constexpr bool TW_SMEM_NP = !PERSIST && G_ == 1 && K >= 3 && N_ >= 8192 && TW_PER_THREAD <= 4 &&
                                        (int)((227 * 1024) / (SMEM + TW_ELEMS * sizeof(float2) + 1024)) == (int)((227 * 1024) / (SMEM + 1024));
     static constexpr size_t SMEM_TW = SMEM + TW_ELEMS * sizeof(float2);
-    static constexpr bool PACK_IN = true;
     static constexpr bool GROUP_IN = true;
     static constexpr int NB0 = N_ / R0_;
     static constexpr int PRE_IT = (NB0 + T_ - 1) / T_;        // pass-0 butterflies per thread
@@ -492,39 +445,21 @@ __device__ __forceinline__ float lg2_approx(float x)
     return r;
 }
 
-// exact s16 pair -> float pair; three forms, chosen at build time (-DJSDR_FFT_CVT=n):
-//   2 (default)  sign-extend on the ALU (PRMT with sign replication / arithmetic shift) and
-//                I2FP.F32.S32: four instructions per pair and nothing on the FMA pipe, the one
-//                this kernel saturates (0.5-2 % faster than form 0);
-//   1            I2F.S16 straight from the halves: two instructions, but on the XU pipe next to
-//                MUFU.LG2 (2-3 % slower than form 0);
-//   0            bias to unsigned, splice into the mantissa of 2^23, subtract 2^23 + 32768 with
-//                one FADD2.
+// exact s16 pair -> float pair: sign-extend on the ALU (PRMT with sign replication, arithmetic
+// shift) and I2FP.F32.S32, four instructions per pair and nothing on the FMA pipe, the one this
+// kernel saturates.  It is 0.5-2 % faster than biasing to unsigned, splicing into the mantissa of
+// 2^23 and subtracting 2^23 + 32768 with one FADD2; I2F.S16 straight from the halves is two
+// instructions, but on the XU pipe next to MUFU.LG2, and 2-3 % slower than the splice.
+// (prmt in PTX: selector bit 3 replicates the chosen byte's sign; __byte_perm masks it off.)
 // The 1/32767 of JavaAudio.java:283 is folded into cf (the transform is linear).
-#ifndef JSDR_FFT_CVT
-#define JSDR_FFT_CVT 2
-#endif
-template <bool PACK>
 __device__ __forceinline__ float2 s16_bits_to_float(uint32_t w)
 {
-#if JSDR_FFT_CVT == 1
-    return make_float2((float)(short)(w & 0xffffu), (float)(short)(w >> 16));
-#elif JSDR_FFT_CVT == 2
-    // sign-extend on the ALU (PRMT with sign replication, arithmetic shift), I2FP.F32.S32
-    // (prmt in PTX: selector bit 3 replicates the chosen byte's sign; __byte_perm masks it off)
     float a, b;
     int lo;
     asm("prmt.b32 %0, %1, 0, 0x9910;" : "=r"(lo) : "r"(w));
     asm("cvt.rn.f32.s32 %0, %1;" : "=f"(a) : "r"(lo));
     asm("cvt.rn.f32.s32 %0, %1;" : "=f"(b) : "r"((int)w >> 16));
     return make_float2(a, b);
-#else
-    w ^= 0x80008000u;
-    const float2 b = make_float2(__uint_as_float(__byte_perm(w, 0x4b000000u, 0x7410)),
-                                 __uint_as_float(__byte_perm(w, 0x4b000000u, 0x7432)));
-    if constexpr (PACK) return cadd(b, make_float2(-8421376.0f, -8421376.0f));
-    else return make_float2(b.x - 8421376.0f, b.y - 8421376.0f);
-#endif
 }
 
 template <class P, int IN>
@@ -539,9 +474,7 @@ __device__ __forceinline__ float2 load_sample(const Args &a, long blk, int n)
         if (a.ic | a.qc) {   // uniform branch: the correction is normally zero
             w = (((w & 0xffffu) + (unsigned)a.ic) & 0xffffu) | ((((w >> 16) + (unsigned)a.qc) & 0xffffu) << 16);
         }
-        // exact s16 -> float without the conversion pipe: bias to unsigned, splice into
-        // the mantissa of 2^23, subtract 2^23 + 32768
-        return s16_bits_to_float<P::PACK_IN>(w);
+        return s16_bits_to_float(w);
     }
 }
 
@@ -604,18 +537,12 @@ __global__ void __launch_bounds__(P::T, P::MINB) fft_kernel(const Args a)
     // "prefetch" stalled every warp in front of the last pass (ncu source page: STL, long scoreboard,
     // 8 % of all stall samples).  Those plans ask for the next block with one bulk L2 prefetch
     // instead, as the non-persistent plans do, and load pass 0 from L2.
-#ifndef JSDR_FFT_REGPF_MAX_IT
-#define JSDR_FFT_REGPF_MAX_IT 1
-#endif
-    constexpr bool PREFETCH = PERSIST && (P::PRE_IT <= JSDR_FFT_REGPF_MAX_IT) && (P::MINB_SMEM < 2);   // (two CTAs per SM: no room for pre[])
+    constexpr bool PREFETCH = PERSIST && P::PRE_IT == 1;
     constexpr bool L2_NEXT = PERSIST && !PREFETCH;
     // ... and fetch BOTH rounds of their own pass 0 before the first butterfly (the shared-memory
     // stores of round one would otherwise hold back the loads of round two): pre[] then lives
     // only inside pass 0 and stays in registers.
-#ifndef JSDR_FFT_EARLY_LOADS
-#define JSDR_FFT_EARLY_LOADS 1
-#endif
-    constexpr bool EARLY = JSDR_FFT_EARLY_LOADS && IN == IN_S16 && SPLIT == 1 && P::G == 1 && !PREFETCH &&
+    constexpr bool EARLY = IN == IN_S16 && SPLIT == 1 && P::G == 1 && !PREFETCH &&
                            P::PRE_IT >= 2 && P::PRE_IT * P::R0 <= 40;       // (19200: 2 x 16; 4410: 2 x 10)
     constexpr bool PRE = PREFETCH || EARLY;
 
@@ -757,8 +684,8 @@ __global__ void __launch_bounds__(P::T, P::MINB) fft_kernel(const Args a)
                         }
 #pragma unroll
                         for (int i = 0; i < CHK; i++) {
-                            va[i] = s16_bits_to_float<P::PACK_IN>(wa[i]);
-                            vb[i] = s16_bits_to_float<P::PACK_IN>(wb[i]);
+                            va[i] = s16_bits_to_float(wa[i]);
+                            vb[i] = s16_bits_to_float(wb[i]);
                         }
                     } else {
                         const float2 *src = reinterpret_cast<const float2 *>(a.in) + rblk * NR + c;
@@ -797,7 +724,7 @@ __global__ void __launch_bounds__(P::T, P::MINB) fft_kernel(const Args a)
                         w[m] = (((w[m] & 0xffffu) + (unsigned)a.ic) & 0xffffu) | ((((w[m] >> 16) + (unsigned)a.qc) & 0xffffu) << 16);
                 }
 #pragma unroll
-                for (int m = 0; m < R0; m++) v[m] = s16_bits_to_float<P::PACK_IN>(w[m]);
+                for (int m = 0; m < R0; m++) v[m] = s16_bits_to_float(w[m]);
             } else {
 #pragma unroll
                 for (int m = 0; m < R0; m++) v[m] = load_sample<P, IN>(a, blk, c + m * NB0);

@@ -29,7 +29,7 @@ HEADER = os.path.join(os.path.dirname(_ROOT), "include", "jsdrcuda.h")
 
 MEM_HOST, MEM_DEVICE = 0, 1
 PREC_F64, PREC_F32 = 0, 1
-KERNEL_AUTO, KERNEL_TILE, KERNEL_STREAM, KERNEL_PRING = 0, 1, 2, 3
+KERNEL_AUTO, KERNEL_TILE, KERNEL_STREAM = 0, 1, 2
 INT_MIN = -2147483648
 
 

@@ -92,7 +92,8 @@ def test_bad_arguments_on_live_handles(ctx):
     for st in (0, 4, -1):
         refused(L.jsdr_bpsk_set_stages, b.h, st)
     refused(L.jsdr_bpsk_set_precision, b.h, 2)
-    refused(L.jsdr_bpsk_set_kernel, b.h, 9)
+    for mode in (3, 9):
+        refused(L.jsdr_bpsk_set_kernel, b.h, mode)
     taps = np.ones(200)
     for nt in (0, -1, 129):
         refused(L.jsdr_bpsk_set_ds_filter, b.h, p(taps), nt)

@@ -13,7 +13,6 @@ import pytest
 
 import jsdrcuda as J
 import oracle as O
-from oracle import siggen
 from test_gpu_parity import check_psd
 
 pytestmark = pytest.mark.gpu
@@ -178,39 +177,6 @@ def test_waterfall_rows_more_than_65535(ctx):
     pix = J.waterfall_rows(ctx, psd, width)
     for r in (0, 65535, 65536, rows - 1):
         assert np.array_equal(pix[r], O.waterfall_row(psd[r], width)), r
-
-
-@pytest.mark.parametrize("ntaps", [27, 64])
-def test_period_ring_kernel_bit_exact(ctx, ntaps):
-    """JSDR_KERNEL_PRING (bpsk_stream2.cuh: period ring staged by bulk copies tracked with
-    mbarriers) against the chunk-ring streaming kernel and the oracle: identical bits, over
-    blocks whose lengths keep every period 16-byte aligned (multiples of 4) and one that does
-    not (the library then falls back to the chunk ring by itself)."""
-    rate, nchan = 192000, 70                       # two full warps of channels and a partial one
-    rng = np.random.default_rng(900 + ntaps)
-    tun = rng.uniform(2000, rate * 0.47, nchan)
-    tun[3] = 0.0
-    tun[5] = rate * 0.4999
-    taps = siggen.lowpass_taps(64, 4800.0, rate) if ntaps == 64 else None
-    banks = {}
-    for k in (J.KERNEL_STREAM, J.KERNEL_PRING):
-        b = J.FUNcubeBPSKDemod(ctx, None, J.AudioDescriptor(rate), tuning=tun, stages=1, max_block=8192)
-        if taps is not None:
-            b.set_ds_filter(taps)
-        b.set_kernel(k)
-        banks[k] = b
-    orcs = {c: O.Bpsk(rate, tun[c], ds_taps=taps, stages=1) for c in (0, 3, 5, 31, 32, 69)}
-    for S in (4096, 8192, 1280, 20, 4, 8188, 777, 4096):
-        raw = rng.integers(-32768, 32768, (nchan, 2 * S)).astype(np.int16)
-        out = {}
-        for k, b in banks.items():
-            b.receive_raw(raw)
-            out[k] = b.read_ds()
-        assert np.array_equal(out[J.KERNEL_PRING], out[J.KERNEL_STREAM]), S
-        for c, o in orcs.items():
-            assert np.array_equal(out[J.KERNEL_PRING][c], o.receive(O.s16_to_float(raw[c]))["ds"]), (S, c)
-    for b in banks.values():
-        b.close()
 
 
 def test_pump_waterfall_argument_errors(ctx):

@@ -150,7 +150,7 @@ __global__ void __launch_bounds__(1024) k_tput(double *out, long long *cyc, doub
 
 // ---------------------------------------------------------------- small bulk copies
 // every lane copies `bytes` from its own row with cp.async.bulk onto one mbarrier per warp, waits,
-// repeats: the staging pattern of bpsk_stream2.cuh
+// repeats: the staging pattern of the period-ring decimator that was measured and dropped (DESIGN.md §9)
 __global__ void __launch_bounds__(512) k_bulk(const uint32_t *in, long long row_stride, int bytes, int reps, long long *cyc,
                                               unsigned *sink)
 {

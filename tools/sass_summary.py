@@ -11,7 +11,6 @@ BUILD = os.path.join(ROOT, "java-sdr_b200", "csrc", "build")
 KERNELS = [
     ("fft_n4096.o", r"fft_kernelINS0_4PlanILi4096.*Li1ELi0E", "fft_kernel<Plan<4096,64,1,64,64>, IN_S16, OUT_PSD>"),
     ("bpsk.o", r"k_mixdecim_streamILi1ELi0ELi64ELi20ELi16E", "k_mixdecim_stream<S16, F64, 64 taps, D=20, 16 warps>"),
-    ("bpsk.o", r"k_mixdecim_pringILi0ELi64ELi20E", "k_mixdecim_pring<F64, 64 taps, D=20> (opt-in: period ring staged by bulk copies)"),
     ("bpsk.o", r"k_tuner_scoutILi1E", "k_tuner_scout<1>"),
     ("fec.o", r"k_fec_decode", "k_fec_decode"),
 ]

@@ -213,6 +213,13 @@ int jsdr_demod_get_weights(jsdr_demod *d, int chan, float w[21]);
 int jsdr_demod_set_flags(jsdr_demod *d, int dofir, int dodwn);
 int jsdr_demod_receive_f32(jsdr_demod *d, const float *iq, int nsamples, int64_t chan_stride,
                            float *out /* nchan*2*nsamples */, int mem);
+/* The same on s16 IQ of the IRawHandler contract (what the dongle delivers): each sample is
+ * converted on the device as JavaAudio does before it calls its handlers (JavaAudio.java:276-293,
+ * ic/qc added with 16-bit wrap, then (float)s/32767f), so the result equals receive_f32 on the
+ * converted floats bit for bit.  chan_stride counts complex samples (0: one shared stream).
+ * The delay line holds converted floats: s16 and f32 calls may alternate on one handle. */
+int jsdr_demod_receive_s16(jsdr_demod *d, const int16_t *raw, int nsamples, int64_t chan_stride,
+                           int ic, int qc, float *out /* nchan*2*nsamples */, int mem);
 
 /* The detectors, AGC and s16 narrowing that follow the FIR + NCO in demod.receive
  * (demod.java:405-481): mode 0 off, 1 raw (I), 2 AM (envelope minus its running mean),
@@ -223,6 +230,9 @@ int jsdr_demod_receive_f32(jsdr_demod *d, const float *iq, int nsamples, int64_t
 int jsdr_demod_set_mode(jsdr_demod *d, int mode, int doagc);
 int jsdr_demod_receive_audio_f32(jsdr_demod *d, const float *iq, int nsamples, int64_t chan_stride,
                                  int16_t *audio, float *max_avg /* nchan*2 */, int mem);
+/* The whole of demod.receive on s16 IQ, converted as in jsdr_demod_receive_s16. */
+int jsdr_demod_receive_audio_s16(jsdr_demod *d, const int16_t *raw, int nsamples, int64_t chan_stride,
+                                 int ic, int qc, int16_t *audio, float *max_avg /* nchan*2 */, int mem);
 
 /* -------------------------------------------------------------- waterfall.java
  * paintLine (waterfall.java:90-107) for `rows` published "fft-psd" rows (float[n+2]
@@ -288,6 +298,15 @@ int jsdr_pump_receive_s16(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nbl
 int jsdr_pump_waterfall_s16(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks,
                             int ic, int qc, int width, uint32_t peak_rgb, int32_t *pixels,
                             float *peak, int32_t *peak_bin, int mem);
+/* JavaAudio.run's whole fan-out (JavaAudio.java:298-304): fft + demod + tuner bank over one
+ * resident [nchan][nblocks*n] batch.  PSD, peak bins and the bank's outputs are those of
+ * jsdr_pump_receive_s16; the demod handler (d->nchan == b->nchan, nblocks*n within its
+ * max_block_samples) gives what nblocks successive jsdr_demod_receive_audio_s16 calls of n samples
+ * per channel give, in its current mode and flags.
+ * audio is [nchan][nblocks*n]; max_avg (nullable) is [nchan][nblocks][2], one pair per block. */
+int jsdr_pump_demod_s16(jsdr_fft *f, jsdr_bpsk *b, jsdr_demod *d, const int16_t *raw, int nblocks,
+                        int ic, int qc, float *psd, int32_t *peak_bin,
+                        int16_t *audio, float *max_avg, int mem);
 
 #ifdef __cplusplus
 }

@@ -103,17 +103,6 @@ struct RawT<FMT_F32> { typedef float2 type; };
 template <>
 struct RawT<FMT_S16> { typedef uint32_t type; };
 
-// (float)s / 32767f, correctly rounded, without the generic division.  s/32767 = s*2^-15 repeated
-// with period 15 bits, so it never comes within 2^-39 (relative) of a float rounding boundary,
-// and 1/32767 split as r_hi + r_lo (two floats, 48 bits) gives the correctly rounded quotient
-// in one multiply and one FMA: q = fma(s, r_hi, s*r_lo).  Checked exhaustively against IEEE
-// division for all 65536 inputs (tests/test_oracle.py).
-__device__ __forceinline__ float s16_over_32767(float x)
-{
-    const float r_hi = 3.0518509447574615e-05f, r_lo = 2.8422576792141996e-14f;
-    return __fmaf_rn(x, r_hi, __fmul_rn(x, r_lo));
-}
-
 template <int FMT>
 __device__ __forceinline__ void raw_to_iq(typename RawT<FMT>::type w, int ic, int qc, double &i, double &q)
 {
@@ -121,11 +110,9 @@ __device__ __forceinline__ void raw_to_iq(typename RawT<FMT>::type w, int ic, in
         i = (double)w.x;            // :372-373 (double)buf[n*2]
         q = (double)w.y;
     } else {
-        // JavaAudio.java:281-288: s += (short)ic (16-bit wrap); (float)s/(float)Short.MAX_VALUE
-        short si = (short)((int)(w & 0xffffu) + ic);
-        short sq = (short)((int)(w >> 16) + qc);
-        i = (double)s16_over_32767((float)si);
-        q = (double)s16_over_32767((float)sq);
+        const float2 f = s16_iq_to_float2(w, ic, qc);   // common.cuh
+        i = (double)f.x;
+        q = (double)f.y;
     }
 }
 
@@ -1755,15 +1742,22 @@ struct PumpPixels {          // jsdr_pump_waterfall_s16: pixel rows and the two 
     int32_t *pixels;         // [batch][width]
     float *peak;             // [batch][2]: psd[N] (peak Hz), psd[N+1] (peak dB)
 };
+struct PumpDemod {           // jsdr_pump_demod_s16: the demod handler beside the other two
+    jsdr_demod *d;
+    int16_t *audio;          // [nchan][nblocks*n]
+    float *max_avg;          // nullable: [nchan][nblocks][2]
+};
 struct PumpJob {
     jsdr_fft *f;
-    int batch, ic, qc;
+    int batch, ic, qc, S;
     float *d_psd;
     int32_t *d_peak;
     const PumpPixels *px;    // device-resident pixel path: paintLine and the maxima behind the FFT
+    const PumpDemod *dm;     // device-resident demod path: FIR + NCO and detectors behind the FFT
 };
 // runs inside bpsk_receive after its fork, so that the next block's phase replay (side stream)
-// starts beside this FFT and not behind it
+// starts beside this FFT and not behind it; the demod kernels follow the FFT there, ahead of
+// the bank's wait for this block's tuner-phase replay
 int pump_fft(void *user, const void *d_in)
 {
     PumpJob *j = static_cast<PumpJob *>(user);
@@ -1775,6 +1769,9 @@ int pump_fft(void *user, const void *d_in)
         JSDR_CUDA(cudaMemcpy2DAsync(j->px->peak, 2 * sizeof(float), j->d_psd + f->n, (f->n + 2) * sizeof(float),
                                     2 * sizeof(float), (size_t)j->batch, cudaMemcpyDeviceToDevice, ctx->stream));
     }
+    if (j->dm)
+        JSDR_TRY(jsdr_pump_demod_run(j->dm->d, static_cast<const int16_t *>(d_in), j->S, f->n, j->ic, j->qc,
+                                     j->dm->audio, j->dm->max_avg));
     return JSDR_OK;
 }
 }  // namespace
@@ -1783,7 +1780,7 @@ int pump_fft(void *user, const void *d_in)
 // blocks go to the fft handler and to the tuner bank.
 namespace {
 int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int ic, int qc, float *psd,
-                 int32_t *peak_bin, int mem, const PumpPixels *px);
+                 int32_t *peak_bin, int mem, const PumpPixels *px, const PumpDemod *dm = nullptr);
 }  // namespace
 
 extern "C" int jsdr_pump_receive_s16(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks,
@@ -1791,6 +1788,26 @@ extern "C" int jsdr_pump_receive_s16(jsdr_fft *f, jsdr_bpsk *b, const int16_t *r
 try {
     JSDR_REQUIRE(psd, JSDR_EINVAL, "null argument");
     return pump_receive(f, b, raw, nblocks, ic, qc, psd, peak_bin, mem, nullptr);
+} JSDR_CATCH_ALL
+
+// JavaAudio.run's whole fan-out (JavaAudio.java:298-304): the fft handler, the demod handler and
+// the tuner bank over one resident batch.  The demod part equals nblocks successive demod.receive
+// calls of n samples per channel.
+extern "C" int jsdr_pump_demod_s16(jsdr_fft *f, jsdr_bpsk *b, jsdr_demod *d, const int16_t *raw, int nblocks,
+                                   int ic, int qc, float *psd, int32_t *peak_bin, int16_t *audio, float *max_avg,
+                                   int mem)
+try {
+    JSDR_REQUIRE(f && b && d && raw && psd && audio, JSDR_EINVAL, "null argument");
+    JSDR_REQUIRE(mem == JSDR_MEM_HOST || mem == JSDR_MEM_DEVICE, JSDR_EINVAL, "bad mem");
+    JSDR_REQUIRE(d->ctx == f->ctx && d->ctx == b->ctx, JSDR_EINVAL, "handlers belong to different contexts");
+    JSDR_REQUIRE(d->nchan == b->nchan, JSDR_EINVAL, "the demod and the bank need the same channel count");
+    JSDR_REQUIRE(nblocks > 0, JSDR_EINVAL, "nblocks must be positive");
+    JSDR_REQUIRE((long long)nblocks * f->n <= d->max_block, JSDR_EINVAL, "nblocks*n exceeds the demod's max_block_samples");
+    // (bpsk_receive's own refusal would come after the demod had consumed the block)
+    JSDR_REQUIRE(!b->dofft || (long long)nblocks * f->n == b->max_block, JSDR_EINVAL,
+                 "auto-tune needs whole blocks of max_block_samples");
+    const PumpDemod dm = {d, audio, max_avg};
+    return pump_receive(f, b, raw, nblocks, ic, qc, psd, peak_bin, mem, nullptr, &dm);
 } JSDR_CATCH_ALL
 
 // The same fan-out with waterfall.java's paintLine (:90-107) chained behind every block's PSD on
@@ -1808,7 +1825,7 @@ try {
 
 namespace {
 int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int ic, int qc, float *psd,
-                 int32_t *peak_bin, int mem, const PumpPixels *px)
+                 int32_t *peak_bin, int mem, const PumpPixels *px, const PumpDemod *dm)
 {
     JSDR_REQUIRE(f && b && raw, JSDR_EINVAL, "null argument");
     JSDR_REQUIRE(f->ctx == b->ctx, JSDR_EINVAL, "handlers belong to different contexts");
@@ -1824,11 +1841,15 @@ int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int
     job.batch = (int)batch;
     job.ic = ic;                                   // JavaAudio.java:281-288: both handlers see the corrected samples
     job.qc = qc;
+    job.S = (int)S;
     job.px = nullptr;
+    job.dm = nullptr;
     const size_t psd_elems = (size_t)batch * (f->n + 2);
+    if (dm) JSDR_TRY(jsdr_pump_demod_fork(dm->d, (int)S));   // the car replay starts beside everything below
     if (mem == JSDR_MEM_DEVICE && !px) {
         job.d_psd = psd;
         job.d_peak = peak_bin;
+        job.dm = dm;
         b->in_pump = 1;
         const int rc = bpsk_receive<FMT_S16>(b, raw, (int)S, S, ic, qc, mem, pump_fft, &job);
         b->in_pump = 0;
@@ -1903,6 +1924,21 @@ int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int
         }
         if (peak_bin)
             JSDR_CUDA(cudaMemcpyAsync(peak_bin + blk0, f->d_peak + blk0, sizeof(int32_t) * nblk,
+                                      cudaMemcpyDeviceToHost, ctx->copy_out));
+    }
+    if (dm) {   // the whole batch is in (the main stream waited for every chunk): demod, audio down beside the bank
+        jsdr_demod *d = dm->d;
+        int16_t *d_audio = nullptr;
+        float *d_ma = nullptr;
+        JSDR_TRY(jsdr_pump_demod_staging(d, (int)S, nblocks, &d_audio, &d_ma));
+        JSDR_TRY(jsdr_pump_demod_run(d, static_cast<const int16_t *>(b->d_in), (int)S, f->n, ic, qc, d_audio,
+                                     dm->max_avg ? d_ma : nullptr));
+        JSDR_CUDA(cudaEventRecord(d->ev_audio_ready, ctx->stream));
+        JSDR_CUDA(cudaStreamWaitEvent(ctx->copy_out, d->ev_audio_ready, 0));
+        JSDR_CUDA(cudaMemcpyAsync(dm->audio, d_audio, sizeof(int16_t) * (size_t)b->nchan * S, cudaMemcpyDeviceToHost,
+                                  ctx->copy_out));
+        if (dm->max_avg)
+            JSDR_CUDA(cudaMemcpyAsync(dm->max_avg, d_ma, sizeof(float) * 2 * (size_t)b->nchan * nblocks,
                                       cudaMemcpyDeviceToHost, ctx->copy_out));
     }
     b->in_pump = 1;

@@ -201,7 +201,7 @@ __device__ __forceinline__ void period_body(const Params &p, const typename Raw<
             double xi, xq;
             if constexpr (FMT == FMT_S16) {
                 // (float)s / 32767f, correctly rounded (JavaAudio.java:283): fma(s, r_hi, s*r_lo), the
-                // s16_over_32767 of bpsk.cu on both halves at once
+                // s16_over_32767 of common.cuh on both halves at once
                 const float2 q2 = fma2(f2, make_float2(3.0518509447574615e-05f, 3.0518509447574615e-05f),
                                        mul2(f2, make_float2(2.8422576792141996e-14f, 2.8422576792141996e-14f)));
                 xi = (double)q2.x;

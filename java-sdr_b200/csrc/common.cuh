@@ -196,6 +196,26 @@ __device__ __forceinline__ void stg_stream_f2(float2 *p, float2 v)
 {
     asm volatile("st.global.cs.v2.f32 [%0], {%1,%2};" ::"l"(p), "f"(v.x), "f"(v.y));
 }
+
+// (float)s / 32767f, correctly rounded, without the generic division.  s/32767 = s*2^-15 repeated
+// with period 15 bits, so it never comes within 2^-39 (relative) of a float rounding boundary,
+// and 1/32767 split as r_hi + r_lo (two floats, 48 bits) gives the correctly rounded quotient
+// in one multiply and one FMA: q = fma(s, r_hi, s*r_lo).  Checked exhaustively against IEEE
+// division for all 65536 inputs (tests/test_oracle.py).
+__device__ __forceinline__ float s16_over_32767(float x)
+{
+    const float r_hi = 3.0518509447574615e-05f, r_lo = 2.8422576792141996e-14f;
+    return __fmaf_rn(x, r_hi, __fmul_rn(x, r_lo));
+}
+
+// One s16le (I, Q) word of the IRawHandler contract to the floats JavaAudio hands its
+// IAudioHandlers (JavaAudio.java:281-288): s += (short)ic (16-bit wrap); (float)s/(float)Short.MAX_VALUE
+__device__ __forceinline__ float2 s16_iq_to_float2(uint32_t w, int ic, int qc)
+{
+    const short si = (short)((int)(w & 0xffffu) + ic);
+    const short sq = (short)((int)(w >> 16) + qc);
+    return make_float2(s16_over_32767((float)si), s16_over_32767((float)sq));
+}
 #endif
 
 }  // namespace jsdr

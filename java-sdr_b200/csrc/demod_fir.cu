@@ -9,6 +9,7 @@
 #include <math.h>
 #include <string.h>
 
+#include <type_traits>
 #include <vector>
 
 #include "handles.h"
@@ -114,19 +115,39 @@ __device__ __forceinline__ void nco_sincos(float car, float *sn_out, float *cs_o
 }
 
 struct DemodParams {
-    const float2 *in;
+    const void *in;            // float2 IQ, or s16 (I, Q) words for k_demod_s16
     long long chan_stride;
     int S, nchan;
     const float *w;            // [nchan][21]
     const float *phi;
     const float *chunk_car;
-    const float2 *hist_in;     // [nchan][20], entry k is local sample k-20
+    const float2 *hist_in;     // [nchan][20], entry k is local sample k-20 (converted floats)
     float2 *hist_out;
     float2 *out;               // [nchan][S]
     int dofir, dodwn;
+    int ic, qc;                // s16 input: JavaAudio's I/Q corrections (JavaAudio.java:281-288)
 };
 
-__global__ void __launch_bounds__(kThreads) k_demod(const DemodParams p)
+// Input sample n >= 0 of channel row `src` as the float IQ demod.receive sees: the f32 row
+// itself, or the s16 word converted as JavaAudio does before it calls its handlers.
+template <bool S16>
+__device__ __forceinline__ float2 demod_input(const DemodParams &p, const void *src, int n)
+{
+    if constexpr (S16) return s16_iq_to_float2(static_cast<const uint32_t *>(src)[n], p.ic, p.qc);
+    else return static_cast<const float2 *>(src)[n];
+}
+
+template <bool S16>
+__device__ __forceinline__ const void *demod_row(const DemodParams &p, int ch)
+{
+    using T = typename std::conditional<S16, uint32_t, float2>::type;
+    return static_cast<const T *>(p.in) + (long long)ch * p.chan_stride;
+}
+
+// k_demod and k_demod_s16: the input form only changes how a sample is staged into sX (each
+// sample is converted once there, not once per tap); the FIR and the NCO see floats either way.
+template <bool S16>
+__device__ __forceinline__ void demod_tile(const DemodParams &p)
 {
     __shared__ __align__(16) float2 sX[kTile + kHist + 4];   // (+4: the last thread's 128-bit reads stay inside)
     __shared__ float sCar[kTile + kTile / kChunk];
@@ -134,11 +155,11 @@ __global__ void __launch_bounds__(kThreads) k_demod(const DemodParams p)
     const int tid = threadIdx.x, ch = blockIdx.y;
     const int t0 = blockIdx.x * kTile;
     const int cnt = min(kTile, p.S - t0);
-    const float2 *src = p.in + (long long)ch * p.chan_stride;
+    const void *src = demod_row<S16>(p, ch);
     if (tid < kTaps) sW[tid] = p.w[ch * kTaps + tid];
     for (int i = tid; i < cnt + kHist; i += kThreads) {
         int n = t0 - kHist + i;
-        sX[i] = (n < 0) ? p.hist_in[(size_t)ch * kHist + kHist + n] : src[n];
+        sX[i] = (n < 0) ? p.hist_in[(size_t)ch * kHist + kHist + n] : demod_input<S16>(p, src, n);
     }
     if (p.dodwn) {
         // one thread per checkpoint chunk replays car (:427-429); padded so lanes
@@ -212,13 +233,19 @@ __global__ void __launch_bounds__(kThreads) k_demod(const DemodParams p)
     }
 }
 
+__global__ void __launch_bounds__(kThreads) k_demod(const DemodParams p) { demod_tile<false>(p); }
+__global__ void __launch_bounds__(kThreads) k_demod_s16(const DemodParams p) { demod_tile<true>(p); }
+
+// The delay line holds converted floats whatever the input form, so that s16 and f32 blocks
+// may alternate on one handle.
+template <bool S16>
 __global__ void k_demod_tail(const DemodParams p)
 {
     const int ch = blockIdx.x, k = threadIdx.x;
     if (k >= kHist) return;
-    const float2 *src = p.in + (long long)ch * p.chan_stride;
+    const void *src = demod_row<S16>(p, ch);
     int n = p.S - kHist + k;
-    p.hist_out[(size_t)ch * kHist + k] = (n < 0) ? p.hist_in[(size_t)ch * kHist + k + p.S] : src[n];
+    p.hist_out[(size_t)ch * kHist + k] = (n < 0) ? p.hist_in[(size_t)ch * kHist + k + p.S] : demod_input<S16>(p, src, n);
 }
 
 // ------------------------------------------------------------------ fir.java
@@ -375,7 +402,9 @@ try {
     if (e == cudaSuccess) e = cudaMalloc(&d->d_chunk_car, sizeof(float) * nc * d->max_chunks);
     if (e == cudaSuccess) e = cudaMalloc(&d->d_hist[0], sizeof(float2) * kHist * nc);
     if (e == cudaSuccess) e = cudaMalloc(&d->d_hist[1], sizeof(float2) * kHist * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&d->d_lilq, sizeof(float2) * nc);
+    if (e == cudaSuccess) e = cudaMalloc(&d->d_lilq, sizeof(float2) * 2 * nc);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&d->ev_car_ready, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&d->ev_audio_ready, cudaEventDisableTiming);
     if (e != cudaSuccess) {
         set_error("jsdr_demod_create: %s", cudaGetErrorString(e));
         jsdr_demod_destroy(d);
@@ -387,7 +416,7 @@ try {
     cudaMemsetAsync(d->d_car, 0, sizeof(float) * nc, ctx->stream);
     cudaMemsetAsync(d->d_hist[0], 0, sizeof(float2) * kHist * nc, ctx->stream);
     cudaMemsetAsync(d->d_hist[1], 0, sizeof(float2) * kHist * nc, ctx->stream);
-    cudaMemsetAsync(d->d_lilq, 0, sizeof(float2) * nc, ctx->stream);
+    cudaMemsetAsync(d->d_lilq, 0, sizeof(float2) * 2 * nc, ctx->stream);
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     *out = d;
     return JSDR_OK;
@@ -398,10 +427,14 @@ try {
     if (!d) return JSDR_OK;
     d->ctx->bind();
     cudaStreamSynchronize(d->ctx->side);
+    cudaStreamSynchronize(d->ctx->side2);
+    cudaStreamSynchronize(d->ctx->copy_out);
     cudaStreamSynchronize(d->ctx->stream);
     void *ptrs[] = {d->d_w, d->d_phi, d->d_car, d->d_chunk_car, d->d_hist[0], d->d_hist[1], d->d_in, d->d_out,
                     d->d_lilq, d->d_det, d->d_audio};
     for (void *p : ptrs) cudaFree(p);
+    if (d->ev_car_ready) cudaEventDestroy(d->ev_car_ready);
+    if (d->ev_audio_ready) cudaEventDestroy(d->ev_audio_ready);
     delete d;
     return JSDR_OK;
 } JSDR_CATCH_ALL
@@ -460,33 +493,28 @@ try {
 
 namespace {
 
-// FIR + NCO of one block for every channel; the result stays on the device in *d_result
-// ([nchan][S] float2: `out` itself for device calls, the staging buffer for host calls).
-int demod_run(jsdr_demod *d, const float *iq, int S, int64_t chan_stride, float *out, int mem, float2 **d_result)
+// The car replay of S samples (k_car_scout) on `side`, forked from the main stream (so it follows
+// the previous k_demod of this handle, which read the checkpoints it overwrites) and joined back
+// through `join`, which the main stream waits on before k_demod.
+int demod_car_fork(jsdr_demod *d, int S, cudaEvent_t fork, cudaStream_t side, cudaEvent_t join)
+{
+    jsdr_ctx *ctx = d->ctx;
+    JSDR_CUDA(cudaEventRecord(fork, ctx->stream));
+    JSDR_CUDA(cudaStreamWaitEvent(side, fork, 0));
+    k_car_scout<<<(d->nchan + 127) / 128, 128, 0, side>>>(d->d_phi, d->d_car, d->d_chunk_car, d->nchan, S);
+    JSDR_TRY(launched(ctx, "k_car_scout"));
+    JSDR_CUDA(cudaEventRecord(join, side));
+    return JSDR_OK;
+}
+
+// k_demod (or k_demod_s16) and the delay-line update over S samples per channel of device input
+// d_in into d_out, on the main stream behind `car_ready` (the car replay of these S samples).
+int demod_launch(jsdr_demod *d, const void *d_in, bool s16, int S, int64_t chan_stride, int ic, int qc,
+                 float2 *d_out, cudaEvent_t car_ready)
 {
     jsdr_ctx *ctx = d->ctx;
     const int nchan = d->nchan;
-    if (d->dodwn) {
-        JSDR_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
-        JSDR_CUDA(cudaStreamWaitEvent(ctx->side, ctx->ev_fork, 0));
-        k_car_scout<<<(nchan + 127) / 128, 128, 0, ctx->side>>>(d->d_phi, d->d_car, d->d_chunk_car, nchan, S);
-        JSDR_TRY(launched(ctx, "k_car_scout"));
-        JSDR_CUDA(cudaEventRecord(ctx->ev_join, ctx->side));
-    }
-    const float2 *d_in = reinterpret_cast<const float2 *>(iq);
-    float2 *d_out = reinterpret_cast<float2 *>(out);
-    const size_t out_bytes = sizeof(float2) * (size_t)nchan * S;
-    if (mem == JSDR_MEM_HOST) {
-        const size_t total = (chan_stride == 0) ? (size_t)S : (size_t)chan_stride * (nchan - 1) + S;
-        JSDR_TRY(grow(&d->d_in, &d->in_cap, total * sizeof(float2)));
-        JSDR_CUDA(cudaMemcpyAsync(d->d_in, iq, total * sizeof(float2), cudaMemcpyHostToDevice, ctx->stream));
-        d_in = reinterpret_cast<const float2 *>(d->d_in);
-    }
-    if (mem == JSDR_MEM_HOST || !out) {
-        JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_out), &d->out_cap, out_bytes));
-        d_out = reinterpret_cast<float2 *>(d->d_out);
-    }
-    if (d->dodwn) JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
+    if (d->dodwn) JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, car_ready, 0));
     DemodParams p;
     p.in = d_in;
     p.chan_stride = chan_stride;
@@ -500,17 +528,48 @@ int demod_run(jsdr_demod *d, const float *iq, int S, int64_t chan_stride, float 
     p.out = d_out;
     p.dofir = d->dofir;
     p.dodwn = d->dodwn;
+    p.ic = ic;
+    p.qc = qc;
     dim3 grid((S + kTile - 1) / kTile, nchan);
     {
         ProfScope prof(ctx, JSDR_K_DEMOD, ctx->stream);
-        k_demod<<<grid, kThreads, 0, ctx->stream>>>(p);
+        if (s16) k_demod_s16<<<grid, kThreads, 0, ctx->stream>>>(p);
+        else k_demod<<<grid, kThreads, 0, ctx->stream>>>(p);
     }
-    JSDR_TRY(launched(ctx, "k_demod"));
+    JSDR_TRY(launched(ctx, s16 ? "k_demod_s16" : "k_demod"));
     if (d->dofir) {   // the delay line only moves when filter() runs (:415-419)
-        k_demod_tail<<<nchan, 32, 0, ctx->stream>>>(p);
+        if (s16) k_demod_tail<true><<<nchan, 32, 0, ctx->stream>>>(p);
+        else k_demod_tail<false><<<nchan, 32, 0, ctx->stream>>>(p);
         JSDR_TRY(launched(ctx, "k_demod_tail"));
         d->hist_cur ^= 1;
     }
+    return JSDR_OK;
+}
+
+// FIR + NCO of one block for every channel; the result stays on the device in *d_result
+// ([nchan][S] float2: `out` itself for device calls, the staging buffer for host calls).
+// `in` is float IQ, or s16 IQ with its I/Q corrections when s16 is set.
+int demod_run(jsdr_demod *d, const void *in, bool s16, int S, int64_t chan_stride, int ic, int qc, float *out,
+              int mem, float2 **d_result)
+{
+    jsdr_ctx *ctx = d->ctx;
+    const int nchan = d->nchan;
+    if (d->dodwn) JSDR_TRY(demod_car_fork(d, S, ctx->ev_fork, ctx->side, ctx->ev_join));
+    const void *d_in = in;
+    float2 *d_out = reinterpret_cast<float2 *>(out);
+    const size_t out_bytes = sizeof(float2) * (size_t)nchan * S;
+    if (mem == JSDR_MEM_HOST) {
+        const size_t esz = s16 ? 4 : 8;
+        const size_t total = (chan_stride == 0) ? (size_t)S : (size_t)chan_stride * (nchan - 1) + S;
+        JSDR_TRY(grow(&d->d_in, &d->in_cap, total * esz));
+        JSDR_CUDA(cudaMemcpyAsync(d->d_in, in, total * esz, cudaMemcpyHostToDevice, ctx->stream));
+        d_in = d->d_in;
+    }
+    if (mem == JSDR_MEM_HOST || !out) {
+        JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_out), &d->out_cap, out_bytes));
+        d_out = reinterpret_cast<float2 *>(d->d_out);
+    }
+    JSDR_TRY(demod_launch(d, d_in, s16, S, chan_stride, ic, qc, d_out, ctx->ev_join));
     *d_result = d_out;
     return JSDR_OK;
 }
@@ -524,22 +583,34 @@ int demod_check(jsdr_demod *d, const void *iq, const void *out, int S, int64_t c
     return JSDR_OK;
 }
 
-}  // namespace
-
-extern "C" int jsdr_demod_receive_f32(jsdr_demod *d, const float *iq, int S, int64_t chan_stride,
-                                      float *out, int mem)
-try {
-    JSDR_TRY(demod_check(d, iq, out, S, chan_stride, mem));
+int demod_receive(jsdr_demod *d, const void *in, bool s16, int S, int64_t chan_stride, int ic, int qc,
+                  float *out, int mem)
+{
+    JSDR_TRY(demod_check(d, in, out, S, chan_stride, mem));
     if (S == 0) return JSDR_OK;
     jsdr_ctx *ctx = d->ctx;
     JSDR_TRY(ctx->bind());
     float2 *res = nullptr;
-    JSDR_TRY(demod_run(d, iq, S, chan_stride, out, mem, &res));
+    JSDR_TRY(demod_run(d, in, s16, S, chan_stride, ic, qc, out, mem, &res));
     if (mem == JSDR_MEM_HOST) {
         JSDR_CUDA(cudaMemcpyAsync(out, res, sizeof(float2) * (size_t)d->nchan * S, cudaMemcpyDeviceToHost, ctx->stream));
         JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     }
     return JSDR_OK;
+}
+
+}  // namespace
+
+extern "C" int jsdr_demod_receive_f32(jsdr_demod *d, const float *iq, int S, int64_t chan_stride,
+                                      float *out, int mem)
+try {
+    return demod_receive(d, iq, false, S, chan_stride, 0, 0, out, mem);
+} JSDR_CATCH_ALL
+
+extern "C" int jsdr_demod_receive_s16(jsdr_demod *d, const int16_t *raw, int S, int64_t chan_stride,
+                                      int ic, int qc, float *out, int mem)
+try {
+    return demod_receive(d, raw, true, S, chan_stride, ic, qc, out, mem);
 } JSDR_CATCH_ALL
 
 // ------------------------------------------------------------------ detectors, AGC, s16 (:405-481)
@@ -566,14 +637,19 @@ __device__ __noinline__ float running_mean_div(float avg, const float4 *op, int 
     return avg;
 }
 
-// One CTA per channel.  Pass 1: the detector output of every sample (sample parallel; the FM
-// discriminator's previous sample is the neighbour, or the carried li/lq for the first) and the
-// block maximum of |.| (:448-463).  Pass 2 (AM): the running mean avg = ((k)*avg + x)/(k+1) is a
-// sequential float recurrence (:451), replayed by one thread over tiles staged in shared memory.
-// Pass 3: AM subtracts the mean, AGC scales by 1.0f/max, narrow to s16 as Java's (short) does
-// (:469-473).  `det` is scratch [nchan][S].
-__global__ void __launch_bounds__(256, 8) k_detect(const float2 *__restrict__ mixed, int S, int mode, float fmgain, int doagc,
-                                                float2 *__restrict__ lilq, float *__restrict__ det,
+// One CTA per (channel, block): a row of Srow samples per channel is cut into blocks of L
+// samples (the last may be shorter), each one demod.receive call -- so the maximum, the AM running
+// mean (avg restarts at k = 0) and the AGC gain are per block, while li/lq run across blocks.
+// Pass 1: the detector output of every sample (sample parallel; the FM discriminator's previous
+// sample is the neighbour: for the first sample of block j > 0 the last of block j - 1, for the
+// first of the row the carried lilq_in) and the block maximum of |.| (:448-463).  Pass 2 (AM): the
+// running mean avg = ((k)*avg + x)/(k+1) is a sequential float recurrence (:451), replayed by one
+// thread over tiles staged in shared memory.  Pass 3: AM subtracts the mean, AGC scales by
+// 1.0f/max, narrow to s16 as Java's (short) does (:469-473).  The last block of a row leaves its
+// last sample in lilq_out (FM modes); lilq_out may be lilq_in when a row is one block (the CTA
+// reads before it writes).  `det` is scratch [nchan][Srow]; max_avg is [nchan][nblocks][2].
+__global__ void __launch_bounds__(256, 8) k_detect(const float2 *__restrict__ mixed, int Srow, int L, int mode, float fmgain,
+                                                int doagc, const float2 *lilq_in, float2 *lilq_out, float *__restrict__ det,
                                                 int16_t *__restrict__ audio, float *__restrict__ max_avg)
 {
     __shared__ unsigned s_max;
@@ -581,9 +657,12 @@ __global__ void __launch_bounds__(256, 8) k_detect(const float2 *__restrict__ mi
     __shared__ float s_avg;
     __shared__ int s_slow;
     __shared__ __align__(16) float4 s_op[2][512];    // per sample of a tile: (y_hi, y_lo, x, x*y_lo), 1/n = y_hi + y_lo; two tiles
-    const int ch = blockIdx.x, tid = threadIdx.x;
-    const float2 *x = mixed + (size_t)ch * S;
-    float *dv = det + (size_t)ch * S;
+    const int nblk = (Srow + L - 1) / L;
+    const int ch = blockIdx.x / nblk, blk = blockIdx.x - ch * nblk, tid = threadIdx.x;
+    const size_t base = (size_t)ch * Srow + (size_t)blk * L;
+    const int S = min(L, Srow - blk * L);                        // this block's samples
+    const float2 *x = mixed + base;
+    float *dv = det + base;
     if (tid == 0) {
         s_max = 0u;
         s_nan = 0;
@@ -591,7 +670,7 @@ __global__ void __launch_bounds__(256, 8) k_detect(const float2 *__restrict__ mi
         s_avg = 0.0f;
     }
     __syncthreads();
-    const float2 prev0 = lilq[ch];
+    const float2 prev0 = (blk == 0) ? lilq_in[ch] : x[-1];
     unsigned mymax = 0u;
     int mynan = 0;
     for (int k = tid; k < S; k += blockDim.x) {
@@ -615,7 +694,7 @@ __global__ void __launch_bounds__(256, 8) k_detect(const float2 *__restrict__ mi
     atomicMax(&s_max, mymax);
     if (mynan) s_nan = 1;
     __syncthreads();
-    if ((mode == MODE_NFM || mode == MODE_WFM) && tid == 0 && S > 0) lilq[ch] = x[S - 1];
+    if ((mode == MODE_NFM || mode == MODE_WFM) && tid == 0 && S > 0 && blk == nblk - 1) lilq_out[ch] = x[S - 1];
     if (mode == MODE_AM) {
         // avg = ((float)k*avg + x) / (float)(k+1) (:451) is a sequential float recurrence with a
         // division on the chain, walked by one thread.  What does not depend on the chain is filled
@@ -697,11 +776,11 @@ __global__ void __launch_bounds__(256, 8) k_detect(const float2 *__restrict__ mi
         float o = dv[k];
         if (mode == MODE_AM) o = __fsub_rn(o, avg);
         o = __fmul_rn(o, gain);
-        audio[(size_t)ch * S + k] = (int16_t)(java_f2i(__fmul_rn(o, 32767.0f)) & 0xffff);   // (short)(float)
+        audio[base + k] = (int16_t)(java_f2i(__fmul_rn(o, 32767.0f)) & 0xffff);   // (short)(float)
     }
     if (tid == 0 && max_avg) {
-        max_avg[2 * ch] = mx;
-        max_avg[2 * ch + 1] = avg;
+        max_avg[2 * (size_t)blockIdx.x] = mx;
+        max_avg[2 * (size_t)blockIdx.x + 1] = avg;
     }
 }
 
@@ -716,32 +795,56 @@ try {
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
-extern "C" int jsdr_demod_receive_audio_f32(jsdr_demod *d, const float *iq, int S, int64_t chan_stride,
-                                            int16_t *audio, float *max_avg, int mem)
-try {
-    JSDR_TRY(demod_check(d, iq, audio, S, chan_stride, mem));
+namespace {
+
+// k_detect over rows of Srow samples per channel of the FIR + NCO output `res`, cut into blocks
+// of L samples: audio [nchan][Srow], max_avg (nullable) [nchan][ceil(Srow/L)][2].
+int detect_launch(jsdr_demod *d, const float2 *res, int Srow, int L, int16_t *audio, float *max_avg)
+{
+    jsdr_ctx *ctx = d->ctx;
+    const int nchan = d->nchan, nblk = (Srow + L - 1) / L;
+    JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_det), &d->det_cap, (size_t)nchan * Srow * sizeof(float)));
+    // :409 fmgain = ad.rate / (MODE_NFM==mode ? 5000f : 75000f), int / float in float
+    const float fmgain = (float)d->rate / (d->mode == dsp::MODE_NFM ? 5000.0f : 75000.0f);
+    // One block per row: the CTA reads li/lq before it writes them.  Several: block 0 of a row may
+    // still read the carried li/lq while the last block writes its own, so that one goes to the
+    // second half of d_lilq and is copied back behind the kernel.
+    float2 *lilq_out = nblk > 1 ? d->d_lilq + nchan : d->d_lilq;
+    {
+        ProfScope prof(ctx, JSDR_K_DETECT, ctx->stream);
+        dsp::k_detect<<<(unsigned)nchan * nblk, 256, 0, ctx->stream>>>(res, Srow, L, d->mode, fmgain, d->doagc, d->d_lilq,
+                                                                        lilq_out, d->d_det, audio, max_avg);
+    }
+    JSDR_TRY(launched(ctx, "k_detect"));
+    if (nblk > 1 && (d->mode == dsp::MODE_NFM || d->mode == dsp::MODE_WFM))
+        JSDR_CUDA(cudaMemcpyAsync(d->d_lilq, lilq_out, sizeof(float2) * nchan, cudaMemcpyDeviceToDevice, ctx->stream));
+    return JSDR_OK;
+}
+
+// staging of a host call's audio and max/avg pairs (npairs of them) in d->d_audio
+int audio_staging(jsdr_demod *d, size_t nsamp, size_t npairs, int16_t **d_audio, float **d_ma)
+{
+    const size_t ma_off = (nsamp * sizeof(int16_t) + 15) & ~(size_t)15;
+    JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_audio), &d->audio_cap, ma_off + sizeof(float) * 2 * npairs));
+    *d_audio = d->d_audio;
+    *d_ma = reinterpret_cast<float *>(reinterpret_cast<char *>(d->d_audio) + ma_off);
+    return JSDR_OK;
+}
+
+int demod_receive_audio(jsdr_demod *d, const void *in, bool s16, int S, int64_t chan_stride, int ic, int qc,
+                        int16_t *audio, float *max_avg, int mem)
+{
+    JSDR_TRY(demod_check(d, in, audio, S, chan_stride, mem));
     if (S == 0) return JSDR_OK;
     jsdr_ctx *ctx = d->ctx;
     JSDR_TRY(ctx->bind());
     const size_t n = (size_t)d->nchan * S;
     float2 *res = nullptr;
-    JSDR_TRY(demod_run(d, iq, S, chan_stride, nullptr, mem, &res));
-    JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_det), &d->det_cap, n * sizeof(float)));
+    JSDR_TRY(demod_run(d, in, s16, S, chan_stride, ic, qc, nullptr, mem, &res));
     int16_t *d_audio = audio;
     float *d_ma = max_avg;
-    if (mem == JSDR_MEM_HOST) {
-        const size_t ma_off = (n * sizeof(int16_t) + 15) & ~(size_t)15;
-        JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_audio), &d->audio_cap, ma_off + sizeof(float) * 2 * d->nchan));
-        d_audio = d->d_audio;
-        d_ma = reinterpret_cast<float *>(reinterpret_cast<char *>(d->d_audio) + ma_off);
-    }
-    // :409 fmgain = ad.rate / (MODE_NFM==mode ? 5000f : 75000f), int / float in float
-    const float fmgain = (float)d->rate / (d->mode == dsp::MODE_NFM ? 5000.0f : 75000.0f);
-    {
-        ProfScope prof(ctx, JSDR_K_DETECT, ctx->stream);
-        dsp::k_detect<<<d->nchan, 256, 0, ctx->stream>>>(res, S, d->mode, fmgain, d->doagc, d->d_lilq, d->d_det, d_audio, d_ma);
-    }
-    JSDR_TRY(launched(ctx, "k_detect"));
+    if (mem == JSDR_MEM_HOST) JSDR_TRY(audio_staging(d, n, d->nchan, &d_audio, &d_ma));
+    JSDR_TRY(detect_launch(d, res, S, S, d_audio, d_ma));
     if (mem == JSDR_MEM_HOST) {
         JSDR_CUDA(cudaMemcpyAsync(audio, d_audio, n * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
         if (max_avg)
@@ -749,7 +852,53 @@ try {
         JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     }
     return JSDR_OK;
+}
+
+}  // namespace
+
+extern "C" int jsdr_demod_receive_audio_f32(jsdr_demod *d, const float *iq, int S, int64_t chan_stride,
+                                            int16_t *audio, float *max_avg, int mem)
+try {
+    return demod_receive_audio(d, iq, false, S, chan_stride, 0, 0, audio, max_avg, mem);
 } JSDR_CATCH_ALL
+
+extern "C" int jsdr_demod_receive_audio_s16(jsdr_demod *d, const int16_t *raw, int S, int64_t chan_stride,
+                                            int ic, int qc, int16_t *audio, float *max_avg, int mem)
+try {
+    return demod_receive_audio(d, raw, true, S, chan_stride, ic, qc, audio, max_avg, mem);
+} JSDR_CATCH_ALL
+
+// ------------------------------------------------------------------ the pump's demod handler
+// jsdr_pump_demod_s16 (bpsk.cu) runs demod over the pump's resident rows of S samples per channel
+// (chan_stride S) as nblocks successive demod.receive calls of L samples: one FIR + NCO launch over
+// the whole row (the delay line and car carry from call to call anyway), then k_detect per block.
+
+// The car replay of the S samples, on side2 behind whatever the main stream holds now: side2
+// carries only the bank's short VCO / bit-phase replay, while the side stream may still be busy
+// with the bank's tuner-phase replay for this very call (enqueued at the end of the previous one).
+// d->ev_car_ready marks its end; jsdr_pump_demod_run waits on it.
+int jsdr_pump_demod_fork(jsdr_demod *d, int S)
+{
+    if (!d->dodwn) return JSDR_OK;
+    return demod_car_fork(d, S, d->ctx->ev_fork, d->ctx->side2, d->ev_car_ready);
+}
+
+// Staging of the host pump's audio [nchan][S] and max/avg pairs [nchan][nblocks][2].
+int jsdr_pump_demod_staging(jsdr_demod *d, int S, int nblocks, int16_t **d_audio, float **d_max_avg)
+{
+    return audio_staging(d, (size_t)d->nchan * S, (size_t)d->nchan * nblocks, d_audio, d_max_avg);
+}
+
+// FIR + NCO of the s16 rows d_raw [nchan][S] and the detectors per block of L samples, on the main
+// stream: audio [nchan][S] and max_avg (nullable) [nchan][S/L][2] are device pointers.
+int jsdr_pump_demod_run(jsdr_demod *d, const int16_t *d_raw, int S, int L, int ic, int qc, int16_t *audio,
+                        float *max_avg)
+{
+    JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_out), &d->out_cap, sizeof(float2) * (size_t)d->nchan * S));
+    float2 *mixed = reinterpret_cast<float2 *>(d->d_out);
+    JSDR_TRY(demod_launch(d, d_raw, true, S, S, ic, qc, mixed, d->ev_car_ready));
+    return detect_launch(d, mixed, S, L, audio, max_avg);
+}
 
 // =========================================================================== fir.java
 // fir.weights(), fir.java:169-195 (host, one-off)

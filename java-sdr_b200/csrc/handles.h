@@ -152,10 +152,14 @@ struct jsdr_demod {
     size_t in_cap = 0, out_cap = 0;
     // detectors + AGC (demod.java:405-481)
     int mode = 0, doagc = 0;         // MODE_OFF (:87 default)
-    float2 *d_lilq = nullptr;        // [nchan] li, lq of the FM discriminator (:67-68)
+    float2 *d_lilq = nullptr;        // [2][nchan] li, lq of the FM discriminator (:67-68); the second half is
+                                     // k_detect's output when a row holds several blocks
     float *d_det = nullptr;          // [nchan][S] detector output scratch
     int16_t *d_audio = nullptr;      // host-call staging: s16 audio + max/avg
     size_t det_cap = 0, audio_cap = 0;
+    // jsdr_pump_demod_s16: the car replay's end (side2 -> main stream) and the audio's (main
+    // stream -> download stream)
+    cudaEvent_t ev_car_ready = nullptr, ev_audio_ready = nullptr;
 };
 
 struct jsdr_fir {
@@ -167,6 +171,12 @@ struct jsdr_fir {
     int32_t *d_in = nullptr, *d_out = nullptr;
     size_t in_cap = 0, out_cap = 0;
 };
+
+// demod_fir.cu: the demod handler of jsdr_pump_demod_s16 (bpsk.cu)
+int jsdr_pump_demod_fork(jsdr_demod *d, int S);
+int jsdr_pump_demod_staging(jsdr_demod *d, int S, int nblocks, int16_t **d_audio, float **d_max_avg);
+int jsdr_pump_demod_run(jsdr_demod *d, const int16_t *d_raw, int S, int L, int ic, int qc, int16_t *audio,
+                        float *max_avg);
 
 int jsdr_fec_after_bits(jsdr_bpsk *b);   // fec.cu: run the frame stage on the bits of the last receive
 void jsdr_fec_destroy(jsdr_bpsk *b);

@@ -8,7 +8,7 @@ over the same C ABI (include/jsdrcuda.h):
     Publish                  the IPublish bus, jsdr.java:118-147
     fft                      fft.java            receive(float[]) -> "fft-psd"
     FUNcubeBPSKDemod         FUNcubeBPSKDemod.java   (a bank of tuners)
-    demod                    demod.java          FIR + NCO part of receive
+    demod                    demod.java          receive: FIR + NCO, detectors, AGC (float or s16 IQ)
     fir                      fir.java            weights/filter/complex_gen/complex_mod
 
 There is no CPU path: importing works anywhere (so the symbol table can be
@@ -107,6 +107,8 @@ _SIGS = {
     "jsdr_demod_receive_f32": [_vp, _vp, _i, _i64, _vp, _i],
     "jsdr_demod_set_mode": [_vp, _i, _i],
     "jsdr_demod_receive_audio_f32": [_vp, _vp, _i, _i64, _vp, _vp, _i],
+    "jsdr_demod_receive_s16": [_vp, _vp, _i, _i64, _i, _i, _vp, _i],
+    "jsdr_demod_receive_audio_s16": [_vp, _vp, _i, _i64, _i, _i, _vp, _vp, _i],
     "jsdr_waterfall_rows": [_vp, _vp, _i, _i, _i, C.c_uint32, _vp, _i],
     "jsdr_fir_design": [_i, _i, _f, _vp],
     "jsdr_fir_nco_table": [_i, _f, _vp],
@@ -117,6 +119,7 @@ _SIGS = {
     "jsdr_fir_complex_mod_i32": [_vp, _vp, _vp, _vp, _i64, _i],
     "jsdr_pump_receive_s16": [_vp, _vp, _vp, _i, _i, _i, _vp, _vp, _i],
     "jsdr_pump_waterfall_s16": [_vp, _vp, _vp, _i, _i, _i, _i, C.c_uint32, _vp, _vp, _vp, _i],
+    "jsdr_pump_demod_s16": [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _i],
     "jsdr_probe_table": [_i, _vp, _i],
     "jsdr_probe_taps": [_vp, _vp],
     "jsdr_probe_scout_thresholds": [_d, C.POINTER(_d), C.POINTER(_d)],
@@ -585,6 +588,28 @@ class demod:
         _ck(lib().jsdr_demod_receive_audio_f32(self.h, _ptr(a), S, 0 if shared else S, _ptr(audio), _ptr(ma), MEM_HOST))
         return audio, ma
 
+    def _raw(self, raw, shared):
+        a = np.ascontiguousarray(raw).view(np.int16)
+        if shared is None:
+            shared = a.ndim == 1
+        S = a.size // 2 if shared else a.size // (2 * self.nchan)
+        return a, S, 0 if shared else S
+
+    def receive_raw(self, raw: np.ndarray, ic: int = 0, qc: int = 0, shared: bool | None = None) -> np.ndarray:
+        """receive() on s16 IQ (IRawHandler), converted on the device as JavaAudio.java:276-293 does."""
+        a, S, stride = self._raw(raw, shared)
+        out = np.empty((self.nchan, 2 * S), dtype=np.float32)
+        _ck(lib().jsdr_demod_receive_s16(self.h, _ptr(a), S, stride, ic, qc, _ptr(out), MEM_HOST))
+        return out
+
+    def receive_audio_raw(self, raw: np.ndarray, ic: int = 0, qc: int = 0, shared: bool | None = None):
+        """receive_audio() on s16 IQ: returns (s16 audio [nchan, S], max_avg [nchan, 2])."""
+        a, S, stride = self._raw(raw, shared)
+        audio = np.empty((self.nchan, S), dtype=np.int16)
+        ma = np.empty((self.nchan, 2), dtype=np.float32)
+        _ck(lib().jsdr_demod_receive_audio_s16(self.h, _ptr(a), S, stride, ic, qc, _ptr(audio), _ptr(ma), MEM_HOST))
+        return audio, ma
+
 
 def waterfall_rows(ctx: "Context", psd: np.ndarray, width: int, peak_rgb: int = 0x00FFFF) -> np.ndarray:
     """waterfall.paintLine (waterfall.java:90-107) for rows of published "fft-psd" arrays."""
@@ -654,6 +679,14 @@ def pump_waterfall_s16(f: fft, b: FUNcubeBPSKDemod, raw, nblocks: int, width: in
     [nchan*nblocks][width] int32 and peak [nchan*nblocks][2] float32 instead of the PSD."""
     _ck(lib().jsdr_pump_waterfall_s16(f.h, b.h, _ptr(raw), nblocks, ic, qc, width, peak_rgb, _ptr(pixels), _ptr(peak),
                                       _ptr(peak_bin), mem))
+
+
+def pump_demod_s16(f: fft, b: FUNcubeBPSKDemod, d: demod, raw, nblocks: int, psd, audio, max_avg=None, peak_bin=None,
+                   mem: int = MEM_HOST, ic: int = 0, qc: int = 0):
+    """JavaAudio.run's whole fan-out (JavaAudio.java:298-304): the pump plus the demod handler.
+    audio is [nchan][nblocks*N] int16; max_avg (optional) [nchan][nblocks][2] float32, per block."""
+    _ck(lib().jsdr_pump_demod_s16(f.h, b.h, d.h, _ptr(raw), nblocks, ic, qc, _ptr(psd), _ptr(peak_bin), _ptr(audio),
+                                  _ptr(max_avg), mem))
 
 
 # ---------------------------------------------------------------------------- constant tables

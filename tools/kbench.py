@@ -3,6 +3,9 @@
   python tools/kbench.py mix   [nchan] [S]      tuner+decimator: tile / stream f64 / stream f32
   python tools/kbench.py fft   [n ...]          FFT+PSD per length (s16 and f32 input)
   python tools/kbench.py other                  demod.java FIR+NCO, detectors, fir.java int FIR, waterfall rows, frame stage
+  python tools/kbench.py demod [nchan] [S]      demod FIR+NCO and NFM / AM audio, f32 against s16 input, alternated
+  python tools/kbench.py pumpdemod [nchan] [nblk] [n]   the pump with and without the demod handler, alternated
+  python tools/kbench.py duty                   the reference's duty: fft + demod (NFM) + two tuners, per 100 ms block
 Prints achieved GB/s of algorithmic bytes and the fraction of MEASURED_PEAKS.json."""
 import json
 import os
@@ -289,6 +292,176 @@ def detect(S=32768, rate=192000):
     ctx.close()
 
 
+def demod(nchan=1024, S=131072, rate=192000, rounds=4):
+    """demod.java's FIR + NCO (:410-434) and the whole receive (NFM, AM with AGC) on float IQ
+    (8 B per sample in) against s16 IQ (4 B in, converted as JavaAudio.java:276-293 does), same
+    samples, alternated round by round; per-kernel CUDA-event times."""
+    L = J.lib()
+    ctx = J.Context(0)
+    rng = np.random.default_rng(4)
+    adsc = J.AudioDescriptor(rate)
+    raw = rng.integers(-20000, 20000, (16, 2 * S)).astype(np.int16)
+    d_raw, d_iq = ctx.dev_alloc(nchan * S * 4), ctx.dev_alloc(nchan * S * 8)
+    fl = np.stack([r.astype(np.float32) / np.float32(32767.0) for r in raw])
+    for c0 in range(0, nchan, 16):
+        d_raw.upload(raw[: min(16, nchan - c0)], offset=c0 * S * 4)
+        d_iq.upload(fl[: min(16, nchan - c0)], offset=c0 * S * 8)
+    d_out, d_aud, d_ma = ctx.dev_alloc(nchan * S * 8), ctx.dev_alloc(nchan * S * 2), ctx.dev_alloc(nchan * 8)
+    dm = J.demod(ctx, adsc, nchan=nchan, max_block=S)
+    for c in range(nchan):
+        dm.weights(3000, 6000, chan=c)
+    P = J._ptr
+    legs = [("FIR+NCO", None, "demod",
+             lambda: L.jsdr_demod_receive_f32(dm.h, P(d_iq), S, S, P(d_out), J.MEM_DEVICE),
+             lambda: L.jsdr_demod_receive_s16(dm.h, P(d_raw), S, S, 0, 0, P(d_out), J.MEM_DEVICE))]
+    for mode, name in ((3, "NFM"), (2, "AM")):
+        legs.append((f"audio {name}+AGC", mode, None,
+                     lambda: L.jsdr_demod_receive_audio_f32(dm.h, P(d_iq), S, S, P(d_aud), P(d_ma), J.MEM_DEVICE),
+                     lambda: L.jsdr_demod_receive_audio_s16(dm.h, P(d_raw), S, S, 0, 0, P(d_aud), P(d_ma), J.MEM_DEVICE)))
+    res = {}
+    for r in range(rounds):
+        for label, mode, kind, f32, s16 in legs:
+            if mode is not None:
+                dm.set_mode(mode, True)
+            for form, fn in (("f32", f32), ("s16", s16)) if r % 2 == 0 else (("s16", s16), ("f32", f32)):
+                for _ in range(2):
+                    J._ck(fn())
+                ctx.sync()
+                ctx.profile(True)
+                ctx.profile_read()
+                ctx.timer_start()
+                for _ in range(5):
+                    J._ck(fn())
+                ms = ctx.timer_stop_ms() / 5
+                prof = ctx.profile_read()
+                ctx.profile(False)
+                k = {kk: round(v[0] / max(v[1], 1), 4) for kk, v in prof.items() if v[1]}
+                res.setdefault((label, form), []).append((ms, k))
+                print(f"round {r} {label:16s} {form} nchan={nchan} S={S}: {ms:8.4f} ms/call  per-kernel ms {k}", flush=True)
+    print("summary (min .. max over rounds; k_demod = 'demod', k_detect = 'detect'):")
+    for (label, form), v in res.items():
+        calls = [x[0] for x in v]
+        kd = [x[1].get("demod", 0.0) for x in v]
+        kt = [x[1].get("detect", 0.0) for x in v]
+        inb = nchan * S * (4 if form == "s16" else 8)
+        gbs = (inb + nchan * S * 8) / min(kd) / 1e6
+        print(f"  {label:16s} {form}: call {min(calls):.4f} .. {max(calls):.4f} ms   k_demod {min(kd):.4f} .. {max(kd):.4f} ms "
+              f"({gbs:.0f} GB/s in+out, frac {gbs / PEAK:.3f})" + (f"   k_detect {min(kt):.4f} .. {max(kt):.4f} ms" if any(kt) else ""),
+              flush=True)
+    for x in (d_raw, d_iq, d_out, d_aud, d_ma):
+        x.free()
+    dm.close()
+    ctx.close()
+
+
+def pumpdemod(nchan=1024, nblk=32, n=4096, rate=192000, rounds=4, reps=6):
+    """jsdr_pump_receive_s16 (fft + tuner bank, 64-tap decimator, stages 1) against
+    jsdr_pump_demod_s16 (the same plus demod in NFM with AGC) on one resident batch of
+    [nchan][nblk*n] s16, device buffers, alternated round by round."""
+    ctx = J.Context(0)
+    S = nblk * n
+    rng = np.random.default_rng(3)
+    tun = rng.uniform(2000, 90000, nchan)
+    d_raw = ctx.dev_alloc(nchan * S * 4)
+    tile = rng.integers(-20000, 20000, (16, 2 * S)).astype(np.int16)
+    for c0 in range(0, nchan, 16):
+        d_raw.upload(tile[: min(16, nchan - c0)], offset=c0 * S * 4)
+    adsc = J.AudioDescriptor(rate)
+    bank = J.FUNcubeBPSKDemod(ctx, None, adsc, tuning=tun, max_block=S, stages=1)
+    bank.set_ds_filter(J.design_lowpass(64, 4800.0, rate))
+    f = J.fft(ctx, None, adsc, max_batch=nchan * nblk, n=n)
+    dm = J.demod(ctx, adsc, nchan=nchan, max_block=S)
+    for c in range(nchan):
+        dm.weights(3000, 6000, chan=c)
+    dm.set_mode(J.demod.MODE_NFM, True)
+    d_psd, d_pk = ctx.dev_alloc(nchan * nblk * (n + 2) * 4), ctx.dev_alloc(nchan * nblk * 4)
+    d_aud, d_ma = ctx.dev_alloc(nchan * S * 2), ctx.dev_alloc(nchan * nblk * 8)
+    steps = {"fft+bank": lambda: J.pump_receive_s16(f, bank, d_raw, nblk, d_psd, d_pk, mem=J.MEM_DEVICE),
+             "fft+demod+bank": lambda: J.pump_demod_s16(f, bank, dm, d_raw, nblk, d_psd, d_aud, d_ma, d_pk, mem=J.MEM_DEVICE)}
+    res = {}
+    for r in range(rounds):
+        for name in (list(steps) if r % 2 == 0 else list(steps)[::-1]):
+            step = steps[name]
+            for _ in range(3):
+                step()
+            ctx.sync()
+            ctx.profile(True)
+            ctx.profile_read()
+            ctx.profile(False)
+            ctx.timer_start()
+            for _ in range(reps):
+                step()
+            ms = ctx.timer_stop_ms() / reps
+            ctx.profile(True)
+            step()
+            prof = ctx.profile_read()
+            ctx.profile(False)
+            per = {k: round(v[0] / max(v[1], 1), 3) for k, v in prof.items() if v[1]}
+            res.setdefault(name, []).append(ms)
+            print(f"round {r} pump {name:15s} nchan={nchan} nblk={nblk} n={n}: {ms:8.3f} ms/step  "
+                  f"{nchan * S / ms / 1e3:9.1f} Msamples/s  per-kernel ms (profiled step) {per}", flush=True)
+    for name, v in res.items():
+        print(f"summary pump {name:15s}: {min(v):.3f} .. {max(v):.3f} ms/step", flush=True)
+    ctx.close()
+
+
+def duty(rate=192000, calls=230, warm=30):
+    """The reference's own duty (jsdr.java:475-483): ONE stream, one block of rate/10 samples per
+    100 ms, the fft handler, the demod handler (NFM) and two FUNcube tuners to bit decisions, host
+    buffers, per call through the C ABI, in the form of bench.py's latency leg: the three handlers
+    one by one (fft.receive_raw, demod.receive_audio_raw, bank.receive_raw + read_bits) against
+    jsdr_pump_demod_s16 (one call; then read_bits), each timed per block, p50 / p99."""
+    import time
+    ctx = J.Context(0)
+    n = rate // 10
+    adsc = J.AudioDescriptor(rate)
+    rng = np.random.default_rng(5)
+    blk = rng.integers(-8000, 8000, 2 * n).astype(np.int16)
+    f = J.fft(ctx, None, adsc, max_batch=2, n=n)
+    f2 = J.fft(ctx, None, adsc, max_batch=2, n=n)
+    bank = J.FUNcubeBPSKDemod(ctx, None, adsc, tuning=[12000.0, 14000.0], max_block=n, stages=3)
+    bank2 = J.FUNcubeBPSKDemod(ctx, None, adsc, tuning=[12000.0, 14000.0], max_block=n, stages=3)
+    dm = J.demod(ctx, adsc, nchan=1, max_block=n)
+    dm.weights(9000, 15000)
+    dm.set_mode(J.demod.MODE_NFM, True)
+    # the pump's demod needs one channel per tuner: the two rows of the batch are the same stream
+    dm2 = J.demod(ctx, adsc, nchan=2, max_block=n)
+    for c in range(2):
+        dm2.weights(9000, 15000, chan=c)
+    dm2.set_mode(J.demod.MODE_NFM, True)
+    two = np.ascontiguousarray(np.stack([blk, blk]))
+    psd = np.empty((2, n + 2), np.float32)
+    pk = np.empty(2, np.int32)
+    aud = np.empty((2, n), np.int16)
+    ma = np.empty((2, 1, 2), np.float32)
+    t_sep, t_pump = [], []
+    for i in range(calls):
+        t0 = time.perf_counter()
+        f.receive_raw(blk)
+        dm.receive_audio_raw(blk)
+        bank.receive_raw(blk, shared=True)
+        bank.read_bits()
+        t1 = time.perf_counter()
+        J.pump_demod_s16(f2, bank2, dm2, two, 1, psd, aud, ma, pk)
+        bank2.read_bits()
+        t2 = time.perf_counter()
+        if i >= warm:
+            t_sep.append((t1 - t0) * 1e6)
+            t_pump.append((t2 - t1) * 1e6)
+    pct = lambda v, q: round(float(np.percentile(v, q)), 1)
+    out = {"unit": "us", "block": f"N={n} s16 IQ (one 100 ms block at {rate} S/s), MEM_HOST, {calls - warm} calls after {warm} warm-up",
+           "handlers_one_by_one_fft_demodNFM_2tuners_to_bits": {"p50": pct(t_sep, 50), "p99": pct(t_sep, 99)},
+           "pump_demod_s16_then_read_bits": {"p50": pct(t_pump, 50), "p99": pct(t_pump, 99)},
+           "budget_us": 100000,
+           "note": "one by one: jsdr_fft_receive_s16, jsdr_demod_receive_audio_s16 (1 channel), jsdr_bpsk_receive_s16 (shared "
+                   "stream, 2 tuners) + jsdr_bpsk_read_bits; pump: jsdr_pump_demod_s16 with the block as the row of each of "
+                   "the 2 channels (FFT of both rows, demod of both) + jsdr_bpsk_read_bits; includes the ctypes call overhead"}
+    print("duty " + json.dumps(out), flush=True)
+    for h in (f, f2, bank, bank2, dm, dm2):
+        h.close()
+    ctx.close()
+
+
 if __name__ == "__main__":
     what = sys.argv[1] if len(sys.argv) > 1 else "mix"
     if what == "mix":
@@ -302,6 +475,12 @@ if __name__ == "__main__":
         other(*[int(x) for x in sys.argv[2:]])
     elif what == "detect":
         detect(*[int(x) for x in sys.argv[2:]])
+    elif what == "demod":
+        demod(*[int(x) for x in sys.argv[2:]])
+    elif what == "pumpdemod":
+        pumpdemod(*[int(x) for x in sys.argv[2:]])
+    elif what == "duty":
+        duty(*[int(x) for x in sys.argv[2:]])
     else:
         fft([int(x) for x in sys.argv[2:]] or [256, 1024, 4096, 9600, 16384, 19200])
 

@@ -19,6 +19,24 @@ void set_error(const char *fmt, ...)
     va_end(ap);
 }
 
+int upload(jsdr_ctx *ctx, void *dst, const void *src, size_t bytes)
+{
+    JSDR_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
+    return JSDR_OK;
+}
+
+int grow(void **p, size_t *cap, size_t bytes)
+{
+    if (*cap >= bytes) return JSDR_OK;
+    cudaFree(*p);
+    *p = nullptr;
+    *cap = 0;
+    JSDR_CUDA(cudaMalloc(p, bytes));
+    *cap = bytes;
+    return JSDR_OK;
+}
+
 }  // namespace jsdr
 
 using namespace jsdr;

@@ -41,8 +41,6 @@ constexpr double kIdxScaleHi = 40.74366543152521;
 constexpr double kIdxScaleLo = -9.306125250357089e-16;
 constexpr int kDmTile = 128;                             // matched-filter outputs per CTA
 
-enum { FMT_F32 = 0, FMT_S16 = 1 };
-
 // FUNcubeBPSKDemod.java:27-55 — F-suffixed literals inside a double[]: each is
 // rounded to float first, then widened.
 static const float kDsFilterF[27] = {
@@ -135,8 +133,8 @@ __device__ __forceinline__ void raw_to_iq(typename RawT<FMT>::type w, int ic, in
 // Round 1 predicted from approximate thresholds and re-evaluated both comparisons behind the
 // chain (seven more instructions per pair, four of them on the FP64 pipe the chain itself
 // needs): a sub-partition could host one such chain per thread and the bank's replay held 32
-// SMs.  Without them a pair is 3 DADD + 2 DSETP + 6 SEL, so CPT independent chains per
-// thread fit under the latency of one and the same bank needs a third of the SMs.
+// SMs.  Without them a pair is 3 DADD + 2 DSETP + 6 SEL, so two warps of chains share a
+// sub-partition and the same bank needs half the SMs (scout_threads).
 struct ScoutChan {
     double inc, th1, th2, pad;
 };
@@ -152,7 +150,6 @@ __device__ __forceinline__ double phase_step2(double p, double inc, double th1, 
 }
 
 constexpr int kScoutThreads = 512;   // launch bound; the CTA size in use is scout_threads()
-constexpr int kScoutMaxCpt = 4;
 // Dynamic shared memory a scout CTA asks for (and never uses): more than half an SM's 227 KB, so
 // that two scout CTAs can never share an SM (at 90 KB two did when an SM emptied -- a 1024-channel
 // bank ran its replay in 7.4 ms instead of 6.0); what is left still takes three 33.8 KB CTAs of
@@ -167,10 +164,11 @@ static int env_int(const char *name, int lo, int hi, int dflt)
     return (v < lo || v > hi) ? dflt : v;
 }
 
-// CTA size and chains per thread of the phase scout = how many SMs it takes (one CTA each; the
-// streaming data kernel leaves them free when it runs beside it).  profiles/r02_scout_sweep.txt
-// has the sweep behind the defaults.  JSDR_SCOUT_THREADS / JSDR_SCOUT_CPT override (tuning aids).
-static int scout_threads(const jsdr_bpsk *b)
+// CTA size of the phase scout = how many SMs it takes (one CTA each; the streaming data kernel
+// leaves them free when it runs beside it).  profiles/r02_scout_sweep.txt has the sweep behind
+// the defaults.  JSDR_SCOUT_THREADS overrides (tuning aid).  `pump`: the receive is the tuner bank
+// of a pump call (pump.cu).
+static int scout_threads(const jsdr_bpsk *b, bool pump)
 {
     static int forced = -1;
     if (forced < 0) {
@@ -183,90 +181,54 @@ static int scout_threads(const jsdr_bpsk *b)
     // + decimator alone is bound by the replay, BASELINE config 4).  In the pump the data kernels
     // take 8 ms per block, so the replay may take 6.4 ms on half the SMs (two warps per
     // sub-partition): the FFT beside it gets 16 SMs back (4.63 -> 4.28 ms, step 8.29 -> 8.23 ms).
-    return (b->in_pump && b->nchan >= 2048) ? 256 : 128;
-}
-static int scout_cpt(const jsdr_bpsk *b)
-{
-    static int forced = -1;
-    if (forced < 0) forced = env_int("JSDR_SCOUT_CPT", 1, kScoutMaxCpt, 0);
-    if (forced) return forced;
-    // One chain per thread.  Several independent chains per thread would interleave in the FP64 pipe
-    // in principle, but ptxas schedules the unrolled chains one after the other (cuobjdump: 48
-    // dependent DADDs of chain 0, then 48 of chain 1), so CPT = 2..4 measured 2.8-4.5x SLOWER
-    // (profiles/r02_scout_sweep.txt); more warps per CTA is the form that works.
-    (void)b;
-    return 1;
+    return (pump && b->nchan >= 2048) ? 256 : 128;
 }
 
-// Thread t of the grid replays the CPT channels t, t + nthr, t + 2 nthr, ... (consecutive lanes
-// hold consecutive channels, so the checkpoint stores coalesce); the chains of a thread are
-// independent and interleave in the FP64 pipe.
-template <int CPT>
+// Thread t of the grid replays channel t (consecutive lanes hold consecutive channels, so the
+// checkpoint stores coalesce).
 __global__ void __launch_bounds__(kScoutThreads)
 k_tuner_scout(const ScoutChan *__restrict__ par, const double *__restrict__ phase_in,
               double *__restrict__ phase_out, double *__restrict__ ckpt, int nchan, int S)
 {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    const int nthr = gridDim.x * blockDim.x;
+    const int ch = blockIdx.x * blockDim.x + threadIdx.x;
     const int nfull = S >> 5;
-    double p[CPT], inc[CPT], th1[CPT], th2[CPT];
-    bool live[CPT], fast[CPT];
-#pragma unroll
-    for (int k = 0; k < CPT; k++) {
-        const int ch = t + k * nthr;
-        live[k] = ch < nchan;
-        const ScoutChan c = par[live[k] ? ch : 0];
-        p[k] = phase_in[live[k] ? ch : 0];
-        inc[k] = c.inc;
-        th1[k] = c.th1;
-        th2[k] = c.th2;
-        // the pair form covers 0 < inc < 3.1 from a phase inside [0, 2pi]; anything else is replayed
-        // step by step below (a dummy chain keeps this one's slot busy meanwhile)
-        fast[k] = live[k] && inc[k] > 0.0 && inc[k] < 3.1 && p[k] >= 0.0 && p[k] <= kTwoPi;
-    }
-    double q[CPT];
-#pragma unroll
-    for (int k = 0; k < CPT; k++) {
-        q[k] = fast[k] ? p[k] : 0.0;
-        if (!fast[k]) {
-            inc[k] = 1.0;
-            th1[k] = 5.0;
-            th2[k] = 4.0;
-        }
+    const bool live = ch < nchan;
+    const ScoutChan c = par[live ? ch : 0];
+    const double p = phase_in[live ? ch : 0];
+    double inc = c.inc, th1 = c.th1, th2 = c.th2;
+    // the pair form covers 0 < inc < 3.1 from a phase inside [0, 2pi]; anything else runs a dummy
+    // chain in step with the warp and is then replayed step by step below
+    const bool fast = live && inc > 0.0 && inc < 3.1 && p >= 0.0 && p <= kTwoPi;
+    double q = fast ? p : 0.0;
+    if (!fast) {
+        inc = 1.0;
+        th1 = 5.0;
+        th2 = 4.0;
     }
     for (int w = 0; w < nfull; w++) {
+        if (fast) ckpt[(size_t)w * nchan + ch] = q;
 #pragma unroll
-        for (int k = 0; k < CPT; k++)
-            if (fast[k]) ckpt[(size_t)w * nchan + t + k * nthr] = q[k];
-#pragma unroll
-        for (int j = 0; j < 16; j++) {
-#pragma unroll
-            for (int k = 0; k < CPT; k++) q[k] = phase_step2(q[k], inc[k], th1[k], th2[k]);
-        }
+        for (int j = 0; j < 16; j++) q = phase_step2(q, inc, th1, th2);
     }
-#pragma unroll
-    for (int k = 0; k < CPT; k++) {
-        const int ch = t + k * nthr;
-        if (!live[k]) continue;
-        double ph;
-        if (fast[k]) {
-            ph = q[k];
-        } else {                                       // increments the pair form does not cover
-            ph = p[k];
-            const double ic = par[ch].inc;
-            for (int w = 0; w < nfull; w++) {
-                ckpt[(size_t)w * nchan + ch] = ph;
+    if (!live) return;
+    double ph;
+    if (fast) {
+        ph = q;
+    } else {                                           // increments the pair form does not cover
+        ph = p;
+        const double ic = par[ch].inc;
+        for (int w = 0; w < nfull; w++) {
+            ckpt[(size_t)w * nchan + ch] = ph;
 #pragma unroll 4
-                for (int j = 0; j < 32; j++) ph = phase_step(ph, ic);
-            }
+            for (int j = 0; j < 32; j++) ph = phase_step(ph, ic);
         }
-        if (S & 31) {
-            const double ic = par[ch].inc;
-            ckpt[(size_t)nfull * nchan + ch] = ph;
-            for (int j = 0; j < (S & 31); j++) ph = phase_step(ph, ic);
-        }
-        phase_out[ch] = ph;
     }
+    if (S & 31) {
+        const double ic = par[ch].inc;
+        ckpt[(size_t)nfull * nchan + ch] = ph;
+        for (int j = 0; j < (S & 31); j++) ph = phase_step(ph, ic);
+    }
+    phase_out[ch] = ph;
 }
 
 // vcoPhase (:511-516) and dmBitPhase (:581-584) are the same for every channel of
@@ -883,13 +845,6 @@ using namespace jsdr::bpsk;
 
 namespace {
 
-int upload(jsdr_ctx *ctx, void *dst, const void *src, size_t bytes)
-{
-    JSDR_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
-    return JSDR_OK;
-}
-
 // Per-sample advance of x = phase*256/(2*pi) in 2^-48 units, modulo 256, in extended
 // precision (used by k_mixdecim's integer fast path).  0 selects the exact path:
 // non-positive or non-finite increments (mixer bypass, :388).
@@ -950,11 +905,11 @@ static ScoutChan scout_chan(double inc)
 
 // Replay the tuner phase over the next S samples from the committed phase into `P`
 // (side stream).
-int launch_scout(jsdr_bpsk *b, jsdr_bpsk::TunerPlan &P, int S)
+int launch_scout(jsdr_bpsk *b, jsdr_bpsk::TunerPlan &P, int S, bool pump)
 {
     jsdr_ctx *ctx = b->ctx;
     ProfScope prof(ctx, JSDR_K_SCOUT, ctx->side);
-    const int st = scout_threads(b), cpt = scout_cpt(b);
+    const int st = scout_threads(b, pump);
     // The replay is a latency-bound chain that wants its share of a sub-partition's FP64 pipe, and
     // CTAs of a high-priority stream are placed wherever a slot frees up: sixteen of these small
     // CTAs fit in the space one retiring data CTA leaves, and stacked like that they run nine
@@ -964,17 +919,11 @@ int launch_scout(jsdr_bpsk *b, jsdr_bpsk::TunerPlan &P, int S)
     if (!scout_smem) scout_smem = env_int("JSDR_SCOUT_SMEM_KB", 1, 200, kScoutSmem / 1024) * 1024;
     static PerDeviceFlag attr_done;
     JSDR_TRY(attr_done.once(ctx->device, [&]() -> int {
-        JSDR_CUDA(cudaFuncSetAttribute(k_tuner_scout<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, scout_smem));
-        JSDR_CUDA(cudaFuncSetAttribute(k_tuner_scout<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, scout_smem));
-        JSDR_CUDA(cudaFuncSetAttribute(k_tuner_scout<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, scout_smem));
-        JSDR_CUDA(cudaFuncSetAttribute(k_tuner_scout<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, scout_smem));
+        JSDR_CUDA(cudaFuncSetAttribute(k_tuner_scout, cudaFuncAttributeMaxDynamicSharedMemorySize, scout_smem));
         return JSDR_OK;
     }));
-    const int per_cta = st * cpt;
-    const int grid = (b->nchan + per_cta - 1) / per_cta;
-    void (*kern)(const ScoutChan *, const double *, double *, double *, int, int) =
-        cpt == 1 ? k_tuner_scout<1> : cpt == 2 ? k_tuner_scout<2> : cpt == 3 ? k_tuner_scout<3> : k_tuner_scout<4>;
-    kern<<<grid, st, scout_smem, ctx->side>>>(b->d_tu_par, b->d_tu_phase, P.phase_end, P.ckpt, b->nchan, S);
+    const int grid = (b->nchan + st - 1) / st;
+    k_tuner_scout<<<grid, st, scout_smem, ctx->side>>>(b->d_tu_par, b->d_tu_phase, P.phase_end, P.ckpt, b->nchan, S);
     JSDR_TRY(launched(ctx, "k_tuner_scout"));
     JSDR_CUDA(cudaEventRecord(P.ready, ctx->side));
     P.S = S;
@@ -1075,7 +1024,7 @@ int launch_stream_shape(jsdr_bpsk *b, const stream::Params &sp)
 }
 
 template <int FMT>
-int launch_stream(jsdr_bpsk *b, const MixParams &mp, int S)
+int launch_stream(jsdr_bpsk *b, const MixParams &mp, int S, bool pump)
 {
     stream::Params sp;
     sp.in = mp.in;
@@ -1098,11 +1047,11 @@ int launch_stream(jsdr_bpsk *b, const MixParams &mp, int S)
     // about ten per resident warp (round 2; three before): SMs that join late, when the scout
     // lets go of them, and the last wave then balance to within a tenth of a warp's share, for
     // (NQ-1)/R = 2 % of warm-up periods (3.91 -> 3.72 ms in the pump, profiles/r02_stream_segs.txt).
-    const int scout_ctas = (mp.nchan + scout_threads(b) - 1) / scout_threads(b);
+    const int scout_ctas = (mp.nchan + scout_threads(b, pump) - 1) / scout_threads(b, pump);
     // stand-alone, the replay of the next block runs beside this kernel: leave it its SMs.  In the
     // pump it runs beside the FFT that precedes this kernel and is normally done by now, so every SM
     // is taken; work is handed out dynamically, so an SM the scout still holds just joins late.
-    sp.grid = b->in_pump ? b->ctx->sm_count : std::max(b->ctx->sm_count - scout_ctas, b->ctx->sm_count / 2);
+    sp.grid = pump ? b->ctx->sm_count : std::max(b->ctx->sm_count - scout_ctas, b->ctx->sm_count / 2);
     sp.warps_per_cta = (FMT == FMT_S16) ? stream::kWarps : stream::kWarpsF32;
     const int resident = sp.grid * sp.warps_per_cta;
     static int segs_per_warp = 0;
@@ -1174,79 +1123,15 @@ int autotune_block(jsdr_bpsk *b, const void *d_in, int S, long long chan_stride,
     return launched(ctx, "k_at_decim");
 }
 
-// `after_input` (optional) is called once the input is on the device and before
-// the main stream waits for the scouts: the pump enqueues the FFT there, so the
-// data-independent phase replay hides behind it.
-typedef int (*after_input_fn)(void *user, const void *d_in);
-
+// The tuner + decimator of one block behind its phase replay (checkpoints `ckpt`): the streaming
+// kernel or the tile kernel, then the history tail.
 template <int FMT>
-int bpsk_receive(jsdr_bpsk *b, const void *in, int S, long long chan_stride, int ic, int qc, int mem,
-                 after_input_fn after_input = nullptr, void *user = nullptr)
+int mix_decimate(jsdr_bpsk *b, const void *d_in, int S, long long chan_stride, int ic, int qc, int n0, int NO,
+                 const double *ckpt, bool pump)
 {
-    JSDR_REQUIRE(b && in, JSDR_EINVAL, "null argument");
-    JSDR_REQUIRE(S >= 0 && S <= b->max_block, JSDR_EINVAL, "nsamples exceeds max_block_samples");
-    JSDR_REQUIRE(chan_stride == 0 || chan_stride >= S, JSDR_EINVAL, "chan_stride smaller than nsamples");
-    JSDR_REQUIRE(mem == JSDR_MEM_HOST || mem == JSDR_MEM_DEVICE, JSDR_EINVAL, "bad mem");
     jsdr_ctx *ctx = b->ctx;
-    JSDR_TRY(ctx->bind());
-    if (b->ds_read_pending) {      // an asynchronous read of the previous block's output is still draining
-        JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, b->ev_ds_read, 0));
-        b->ds_read_pending = 0;
-    }
-    b->last_nds = 0;
-    if (b->stages >= 2) JSDR_TRY(ensure_stage_buffers(b));   // (before the empty-block return: the reads that follow an
-                                                             //  empty FIRST block answer "nothing", not "stage has not run")
-    if (S == 0) {
-        JSDR_CUDA(cudaMemsetAsync(b->d_nbits, 0, sizeof(int32_t) * b->nchan, ctx->aux));
-        if (b->fec && b->stages >= 3 && b->d_bits) JSDR_TRY(jsdr_fec_after_bits(b));   // no bits: no frames either
-        return JSDR_OK;
-    }
     const int D = b->D;
-    const int NO = (b->ds_cnt + S) / D;
-    const int n0 = D - 1 - b->ds_cnt;
     const int nchan = b->nchan;
-
-    // ---- fork: data-independent work on the side stream.  The tuner plan for this
-    // block was normally computed while the previous block was being processed.
-    jsdr_bpsk::TunerPlan &P = b->plan[b->plan_cur];
-    const bool autotune = b->dofft != 0;               // :358-364 receive(): doBufferFFT instead of doBufferTune
-    if (autotune) JSDR_REQUIRE(S == b->max_block, JSDR_EINVAL, "auto-tune needs whole blocks of max_block_samples");
-    JSDR_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
-    JSDR_CUDA(cudaStreamWaitEvent(ctx->side, ctx->ev_fork, 0));
-    JSDR_CUDA(cudaStreamWaitEvent(ctx->side2, ctx->ev_fork, 0));
-    if (!autotune && !(P.valid && P.S == S)) JSDR_TRY(launch_scout(b, P, S));
-    const int kb = b->bit_cur;                         // buffer of the 9600 S/s stages for this block
-    if (b->stages >= 2 && NO > 0) {
-        // normally replayed already, behind the previous block's tuner scout (look-ahead below)
-        if (!(b->vco_ahead_valid && b->vco_ahead_NO == NO && b->vco_ahead_kb == kb)) JSDR_TRY(launch_vco_scout(b, NO, kb));
-        b->vco_ahead_valid = false;
-    }
-    JSDR_CUDA(cudaEventRecord(ctx->ev_join, ctx->side));
-
-    // ---- input
-    const void *d_in = in;
-    if (mem == JSDR_MEM_HOST) {
-        const size_t esz = (FMT == FMT_S16) ? 4 : 8;
-        const size_t total = (chan_stride == 0) ? (size_t)S : (size_t)chan_stride * (nchan - 1) + S;
-        if (b->in_cap < total * esz) {
-            cudaFree(b->d_in);
-            b->d_in = nullptr;
-            b->in_cap = 0;
-            JSDR_CUDA(cudaMalloc(&b->d_in, total * esz));
-            b->in_cap = total * esz;
-        }
-        JSDR_CUDA(cudaMemcpyAsync(b->d_in, in, total * esz, cudaMemcpyHostToDevice, ctx->stream));
-        d_in = b->d_in;
-    }
-    if (after_input) JSDR_TRY(after_input(user, d_in));
-    if (!autotune) JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, P.ready, 0));
-    // (ev_join — the VCO / bit-phase replay of this block — is only needed by the matched filter:
-    // the tuner + decimator runs beside it)
-    if (autotune) {
-        JSDR_TRY(autotune_block<FMT>(b, d_in, S, chan_stride, ic, qc, n0, NO));
-    } else {
-
-    // ---- tuner + decimator
     MixParams mp;
     mp.in = d_in;
     mp.chan_stride = chan_stride;
@@ -1255,7 +1140,7 @@ int bpsk_receive(jsdr_bpsk *b, const void *in, int S, long long chan_stride, int
     mp.qc = qc;
     mp.tu_inc = b->d_tu_inc;
     mp.tu_dx = b->d_tu_dx;
-    mp.ckpt = P.ckpt;
+    mp.ckpt = ckpt;
     mp.nchan = nchan;
     mp.hist_in = b->d_ds_hist[b->ds_hist_cur];
     mp.hist_out = b->d_ds_hist[b->ds_hist_cur ^ 1];
@@ -1283,7 +1168,7 @@ int bpsk_receive(jsdr_bpsk *b, const void *in, int S, long long chan_stride, int
         const bool want = b->kernel_mode == JSDR_KERNEL_STREAM || (nchan >= 32 && NO >= 64) ||
                           (b->precision == JSDR_PREC_F32 && nchan >= 8);
         if (shape_ok && want) {
-            JSDR_TRY(launch_stream<FMT>(b, mp, P.S));
+            JSDR_TRY(launch_stream<FMT>(b, mp, S, pump));
             streamed = true;
         }
     }
@@ -1307,20 +1192,102 @@ int bpsk_receive(jsdr_bpsk *b, const void *in, int S, long long chan_stride, int
         k_tuner_tail<FMT><<<nchan, 128, 0, ctx->stream>>>(mp);
         JSDR_TRY(launched(ctx, "k_tuner_tail"));
     }
-    // this plan is consumed: its end phase becomes the committed phase, and the
-    // scout starts on the next block (same length assumed) while the rest of this
-    // one is still in flight
-    JSDR_CUDA(cudaEventRecord(P.consumed, ctx->stream));
-    P.used = true;
-    P.valid = false;
-    b->d_tu_phase = P.phase_end;
-    b->plan_cur ^= 1;
-    {
+    return JSDR_OK;
+}
+
+}  // namespace
+
+// jsdr_bpsk_receive_* in two halves, so that the pump (pump.cu) can enqueue its own kernels between
+// them, beside the phase replay on the side stream.  The first half checks, forks this block's
+// data-independent replays onto the side streams and puts the input on the device: *d_in is what
+// the second half reads, or nullptr after an empty block, which is then complete.
+int jsdr::bpsk::receive_begin(jsdr_bpsk *b, const void *in, int fmt, int S, long long chan_stride, int mem,
+                              bool pump, const void **d_in)
+{
+    *d_in = nullptr;
+    JSDR_REQUIRE(b && in, JSDR_EINVAL, "null argument");
+    JSDR_REQUIRE(S >= 0 && S <= b->max_block, JSDR_EINVAL, "nsamples exceeds max_block_samples");
+    JSDR_REQUIRE(chan_stride == 0 || chan_stride >= S, JSDR_EINVAL, "chan_stride smaller than nsamples");
+    JSDR_REQUIRE(mem == JSDR_MEM_HOST || mem == JSDR_MEM_DEVICE, JSDR_EINVAL, "bad mem");
+    jsdr_ctx *ctx = b->ctx;
+    JSDR_TRY(ctx->bind());
+    if (b->ds_read_pending) {      // an asynchronous read of the previous block's output is still draining
+        JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, b->ev_ds_read, 0));
+        b->ds_read_pending = 0;
+    }
+    b->last_nds = 0;
+    if (b->stages >= 2) JSDR_TRY(ensure_stage_buffers(b));   // (before the empty-block return: the reads that follow an
+                                                             //  empty FIRST block answer "nothing", not "stage has not run")
+    if (S == 0) {
+        JSDR_CUDA(cudaMemsetAsync(b->d_nbits, 0, sizeof(int32_t) * b->nchan, ctx->aux));
+        if (b->fec && b->stages >= 3 && b->d_bits) JSDR_TRY(jsdr_fec_after_bits(b));   // no bits: no frames either
+        return JSDR_OK;
+    }
+    const int NO = (b->ds_cnt + S) / b->D;
+
+    // ---- fork: data-independent work on the side stream.  The tuner plan for this
+    // block was normally computed while the previous block was being processed.
+    jsdr_bpsk::TunerPlan &P = b->plan[b->plan_cur];
+    const bool autotune = b->dofft != 0;               // :358-364 receive(): doBufferFFT instead of doBufferTune
+    if (autotune) JSDR_REQUIRE(S == b->max_block, JSDR_EINVAL, "auto-tune needs whole blocks of max_block_samples");
+    JSDR_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));
+    JSDR_CUDA(cudaStreamWaitEvent(ctx->side, ctx->ev_fork, 0));
+    JSDR_CUDA(cudaStreamWaitEvent(ctx->side2, ctx->ev_fork, 0));
+    if (!autotune && !(P.valid && P.S == S)) JSDR_TRY(launch_scout(b, P, S, pump));
+    const int kb = b->bit_cur;                         // buffer of the 9600 S/s stages for this block
+    if (b->stages >= 2 && NO > 0) {
+        // normally replayed already, behind the previous block's tuner scout (look-ahead below)
+        if (!(b->vco_ahead_valid && b->vco_ahead_NO == NO && b->vco_ahead_kb == kb)) JSDR_TRY(launch_vco_scout(b, NO, kb));
+        b->vco_ahead_valid = false;
+    }
+    JSDR_CUDA(cudaEventRecord(ctx->ev_join, ctx->side));
+
+    // ---- input
+    if (mem == JSDR_MEM_HOST) {
+        const size_t esz = (fmt == FMT_S16) ? 4 : 8;
+        const size_t bytes = esz * ((chan_stride == 0) ? (size_t)S : (size_t)chan_stride * (b->nchan - 1) + S);
+        JSDR_TRY(grow(&b->d_in, &b->in_cap, bytes));
+        JSDR_CUDA(cudaMemcpyAsync(b->d_in, in, bytes, cudaMemcpyHostToDevice, ctx->stream));
+        in = b->d_in;
+    }
+    *d_in = in;
+    return JSDR_OK;
+}
+
+// The second half: the tuner + decimator behind this block's phase replay, the next block's
+// replay, the 9600 S/s stages.
+int jsdr::bpsk::receive_end(jsdr_bpsk *b, const void *d_in, int fmt, int S, long long chan_stride, int ic, int qc,
+                            int mem, bool pump)
+{
+    jsdr_ctx *ctx = b->ctx;
+    const int D = b->D;
+    const int NO = (b->ds_cnt + S) / D;
+    const int n0 = D - 1 - b->ds_cnt;
+    const int nchan = b->nchan;
+    const int kb = b->bit_cur;
+    const bool s16 = fmt == FMT_S16;
+    if (b->dofft) {
+        JSDR_TRY(s16 ? autotune_block<FMT_S16>(b, d_in, S, chan_stride, ic, qc, n0, NO)
+                     : autotune_block<FMT_F32>(b, d_in, S, chan_stride, ic, qc, n0, NO));
+    } else {
+        jsdr_bpsk::TunerPlan &P = b->plan[b->plan_cur];
+        JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, P.ready, 0));
+        // (ev_join — the VCO / bit-phase replay of this block — is only needed by the matched filter:
+        // the tuner + decimator runs beside it)
+        JSDR_TRY(s16 ? mix_decimate<FMT_S16>(b, d_in, S, chan_stride, ic, qc, n0, NO, P.ckpt, pump)
+                     : mix_decimate<FMT_F32>(b, d_in, S, chan_stride, ic, qc, n0, NO, P.ckpt, pump));
+        // this plan is consumed: its end phase becomes the committed phase, and the
+        // scout starts on the next block (same length assumed) while the rest of this
+        // one is still in flight
+        JSDR_CUDA(cudaEventRecord(P.consumed, ctx->stream));
+        P.used = true;
+        P.valid = false;
+        b->d_tu_phase = P.phase_end;
+        b->plan_cur ^= 1;
         jsdr_bpsk::TunerPlan &Pn = b->plan[b->plan_cur];
         if (Pn.used) JSDR_CUDA(cudaStreamWaitEvent(ctx->side, Pn.consumed, 0));
-        JSDR_TRY(launch_scout(b, Pn, S));
+        JSDR_TRY(launch_scout(b, Pn, S, pump));
     }
-    }   // !autotune
     b->ds_hist_cur ^= 1;
     b->ds_cnt = (b->ds_cnt + S) % D;
     b->cnt_raw += S;
@@ -1406,7 +1373,13 @@ int bpsk_receive(jsdr_bpsk *b, const void *in, int S, long long chan_stride, int
     return JSDR_OK;
 }
 
-}  // namespace
+int jsdr::bpsk::receive(jsdr_bpsk *b, const void *in, int fmt, int S, long long chan_stride, int ic, int qc, int mem,
+                        bool pump)
+{
+    const void *d_in;
+    JSDR_TRY(receive_begin(b, in, fmt, S, chan_stride, mem, pump, &d_in));
+    return d_in ? receive_end(b, d_in, fmt, S, chan_stride, ic, qc, mem, pump) : JSDR_OK;
+}
 
 extern "C" int jsdr_bpsk_create(jsdr_ctx *ctx, int rate, int nchan, const double *tuning_hz,
                                 int max_block_samples, jsdr_bpsk **out)
@@ -1622,13 +1595,13 @@ try {
 
 extern "C" int jsdr_bpsk_receive_f32(jsdr_bpsk *b, const float *iq, int nsamples, int64_t chan_stride, int mem)
 try {
-    return bpsk_receive<FMT_F32>(b, iq, nsamples, chan_stride, 0, 0, mem);
+    return bpsk::receive(b, iq, FMT_F32, nsamples, chan_stride, 0, 0, mem, false);
 } JSDR_CATCH_ALL
 
 extern "C" int jsdr_bpsk_receive_s16(jsdr_bpsk *b, const int16_t *raw, int nsamples, int64_t chan_stride,
                                      int ic, int qc, int mem)
 try {
-    return bpsk_receive<FMT_S16>(b, raw, nsamples, chan_stride, ic, qc, mem);
+    return bpsk::receive(b, raw, FMT_S16, nsamples, chan_stride, ic, qc, mem, false);
 } JSDR_CATCH_ALL
 
 extern "C" int jsdr_bpsk_last_counts(jsdr_bpsk *b, int32_t *n_ds)
@@ -1733,223 +1706,6 @@ try {
     *dev_ptr = reinterpret_cast<double *>(b->d_ds_out);
     return JSDR_OK;
 } JSDR_CATCH_ALL
-
-// ------------------------------------------------------------------ the pump
-namespace {
-struct PumpPixels {          // jsdr_pump_waterfall_s16: pixel rows and the two trailing floats instead of the PSD
-    int width;
-    uint32_t rgb;
-    int32_t *pixels;         // [batch][width]
-    float *peak;             // [batch][2]: psd[N] (peak Hz), psd[N+1] (peak dB)
-};
-struct PumpDemod {           // jsdr_pump_demod_s16: the demod handler beside the other two
-    jsdr_demod *d;
-    int16_t *audio;          // [nchan][nblocks*n]
-    float *max_avg;          // nullable: [nchan][nblocks][2]
-};
-struct PumpJob {
-    jsdr_fft *f;
-    int batch, ic, qc, S;
-    float *d_psd;
-    int32_t *d_peak;
-    const PumpPixels *px;    // device-resident pixel path: paintLine and the maxima behind the FFT
-    const PumpDemod *dm;     // device-resident demod path: FIR + NCO and detectors behind the FFT
-};
-// runs inside bpsk_receive after its fork, so that the next block's phase replay (side stream)
-// starts beside this FFT and not behind it; the demod kernels follow the FFT there, ahead of
-// the bank's wait for this block's tuner-phase replay
-int pump_fft(void *user, const void *d_in)
-{
-    PumpJob *j = static_cast<PumpJob *>(user);
-    jsdr_fft *f = j->f;
-    jsdr_ctx *ctx = f->ctx;
-    JSDR_TRY(fft::launch(f, d_in, fft::IN_S16, j->batch, j->d_psd, j->d_peak, fft::OUT_PSD, j->ic, j->qc, ctx->stream));
-    if (j->px) {
-        JSDR_TRY(jsdr_launch_waterfall(ctx, j->d_psd, f->n, j->batch, j->px->width, j->px->rgb, j->px->pixels, ctx->stream));
-        JSDR_CUDA(cudaMemcpy2DAsync(j->px->peak, 2 * sizeof(float), j->d_psd + f->n, (f->n + 2) * sizeof(float),
-                                    2 * sizeof(float), (size_t)j->batch, cudaMemcpyDeviceToDevice, ctx->stream));
-    }
-    if (j->dm)
-        JSDR_TRY(jsdr_pump_demod_run(j->dm->d, static_cast<const int16_t *>(d_in), j->S, f->n, j->ic, j->qc,
-                                     j->dm->audio, j->dm->max_avg));
-    return JSDR_OK;
-}
-}  // namespace
-
-// JavaAudio.run's fan-out (JavaAudio.java:262-304) for a batch: each channel's
-// blocks go to the fft handler and to the tuner bank.
-namespace {
-int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int ic, int qc, float *psd,
-                 int32_t *peak_bin, int mem, const PumpPixels *px, const PumpDemod *dm = nullptr);
-}  // namespace
-
-extern "C" int jsdr_pump_receive_s16(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks,
-                                     int ic, int qc, float *psd, int32_t *peak_bin, int mem)
-try {
-    JSDR_REQUIRE(psd, JSDR_EINVAL, "null argument");
-    return pump_receive(f, b, raw, nblocks, ic, qc, psd, peak_bin, mem, nullptr);
-} JSDR_CATCH_ALL
-
-// JavaAudio.run's whole fan-out (JavaAudio.java:298-304): the fft handler, the demod handler and
-// the tuner bank over one resident batch.  The demod part equals nblocks successive demod.receive
-// calls of n samples per channel.
-extern "C" int jsdr_pump_demod_s16(jsdr_fft *f, jsdr_bpsk *b, jsdr_demod *d, const int16_t *raw, int nblocks,
-                                   int ic, int qc, float *psd, int32_t *peak_bin, int16_t *audio, float *max_avg,
-                                   int mem)
-try {
-    JSDR_REQUIRE(f && b && d && raw && psd && audio, JSDR_EINVAL, "null argument");
-    JSDR_REQUIRE(mem == JSDR_MEM_HOST || mem == JSDR_MEM_DEVICE, JSDR_EINVAL, "bad mem");
-    JSDR_REQUIRE(d->ctx == f->ctx && d->ctx == b->ctx, JSDR_EINVAL, "handlers belong to different contexts");
-    JSDR_REQUIRE(d->nchan == b->nchan, JSDR_EINVAL, "the demod and the bank need the same channel count");
-    JSDR_REQUIRE(nblocks > 0, JSDR_EINVAL, "nblocks must be positive");
-    JSDR_REQUIRE((long long)nblocks * f->n <= d->max_block, JSDR_EINVAL, "nblocks*n exceeds the demod's max_block_samples");
-    // (bpsk_receive's own refusal would come after the demod had consumed the block)
-    JSDR_REQUIRE(!b->dofft || (long long)nblocks * f->n == b->max_block, JSDR_EINVAL,
-                 "auto-tune needs whole blocks of max_block_samples");
-    const PumpDemod dm = {d, audio, max_avg};
-    return pump_receive(f, b, raw, nblocks, ic, qc, psd, peak_bin, mem, nullptr, &dm);
-} JSDR_CATCH_ALL
-
-// The same fan-out with waterfall.java's paintLine (:90-107) chained behind every block's PSD on
-// the device: what returns is the pixel row a waterfall draws and the two published maxima
-// (fft.java:223-224), 4*width + 8 bytes per block instead of 4*(N+2).
-extern "C" int jsdr_pump_waterfall_s16(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int ic, int qc,
-                                       int width, uint32_t peak_rgb, int32_t *pixels, float *peak, int32_t *peak_bin,
-                                       int mem)
-try {
-    JSDR_REQUIRE(f && pixels && peak, JSDR_EINVAL, "null argument");
-    JSDR_REQUIRE(width > 0 && width <= f->n, JSDR_EINVAL, "need 0 < width <= n");
-    PumpPixels px = {width, peak_rgb, pixels, peak};
-    return pump_receive(f, b, raw, nblocks, ic, qc, nullptr, peak_bin, mem, &px);
-} JSDR_CATCH_ALL
-
-namespace {
-int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int ic, int qc, float *psd,
-                 int32_t *peak_bin, int mem, const PumpPixels *px, const PumpDemod *dm)
-{
-    JSDR_REQUIRE(f && b && raw, JSDR_EINVAL, "null argument");
-    JSDR_REQUIRE(f->ctx == b->ctx, JSDR_EINVAL, "handlers belong to different contexts");
-    JSDR_REQUIRE(nblocks > 0, JSDR_EINVAL, "nblocks must be positive");
-    const long long S = (long long)nblocks * f->n;
-    const long long batch = (long long)nblocks * b->nchan;
-    JSDR_REQUIRE(S <= b->max_block, JSDR_EINVAL, "nblocks*n exceeds the bank's max_block_samples");
-    JSDR_REQUIRE(batch <= f->max_batch, JSDR_EINVAL, "nchan*nblocks exceeds the fft's max_batch");
-    jsdr_ctx *ctx = f->ctx;
-    JSDR_TRY(ctx->bind());
-    PumpJob job;
-    job.f = f;
-    job.batch = (int)batch;
-    job.ic = ic;                                   // JavaAudio.java:281-288: both handlers see the corrected samples
-    job.qc = qc;
-    job.S = (int)S;
-    job.px = nullptr;
-    job.dm = nullptr;
-    const size_t psd_elems = (size_t)batch * (f->n + 2);
-    if (dm) JSDR_TRY(jsdr_pump_demod_fork(dm->d, (int)S));   // the car replay starts beside everything below
-    if (mem == JSDR_MEM_DEVICE && !px) {
-        job.d_psd = psd;
-        job.d_peak = peak_bin;
-        job.dm = dm;
-        b->in_pump = 1;
-        const int rc = bpsk_receive<FMT_S16>(b, raw, (int)S, S, ic, qc, mem, pump_fft, &job);
-        b->in_pump = 0;
-        return rc;
-    }
-    if (f->out_cap < psd_elems * sizeof(float)) {
-        cudaFree(f->d_out);
-        f->d_out = nullptr;
-        f->out_cap = 0;
-        JSDR_CUDA(cudaMalloc(&f->d_out, psd_elems * sizeof(float)));
-        f->out_cap = psd_elems * sizeof(float);
-    }
-    if (!f->d_peak) JSDR_CUDA(cudaMalloc(&f->d_peak, sizeof(int32_t) * (size_t)f->max_batch));
-    const int N2 = f->n + 2;
-    if (mem == JSDR_MEM_DEVICE) {                      // pixel rows from a resident batch: FFT, paintLine, tuner bank
-        job.d_psd = f->d_out;
-        job.d_peak = peak_bin ? peak_bin : f->d_peak;
-        job.px = px;
-        b->in_pump = 1;
-        const int rc = bpsk_receive<FMT_S16>(b, raw, (int)S, S, ic, qc, mem, pump_fft, &job);
-        b->in_pump = 0;
-        return rc;
-    }
-    const size_t in_bytes = (size_t)b->nchan * (size_t)S * 4;
-    if (b->in_cap < in_bytes) {
-        cudaFree(b->d_in);
-        b->d_in = nullptr;
-        b->in_cap = 0;
-        JSDR_CUDA(cudaMalloc(&b->d_in, in_bytes));
-        b->in_cap = in_bytes;
-    }
-    if (px) {
-        const size_t pix_bytes = (size_t)batch * px->width * sizeof(int32_t);
-        if (f->pix_cap < pix_bytes) {
-            cudaFree(f->d_pix);
-            f->d_pix = nullptr;
-            f->pix_cap = 0;
-            JSDR_CUDA(cudaMalloc(&f->d_pix, pix_bytes));
-            f->pix_cap = pix_bytes;
-        }
-    }
-    // Host path, pipelined over channel chunks: PCIe is full duplex, so the upload of chunk
-    // c+1 (copy_in stream) runs beside the FFT of chunk c (main stream) and the download of
-    // the results of chunk c-1 (copy_out stream).  The tuner bank runs once the whole batch is in.
-    const int nchunk = std::min(16, std::max(1, b->nchan / 8));
-    JSDR_CUDA(cudaEventRecord(ctx->ev_fork, ctx->stream));            // staging buffers are free again
-    JSDR_CUDA(cudaStreamWaitEvent(ctx->copy_in, ctx->ev_fork, 0));
-    for (int c = 0; c < nchunk; c++) {
-        const int c0 = (int)((long long)b->nchan * c / nchunk), c1 = (int)((long long)b->nchan * (c + 1) / nchunk);
-        if (c1 == c0) continue;
-        const size_t in_off = (size_t)c0 * (size_t)S * 4, in_len = (size_t)(c1 - c0) * (size_t)S * 4;
-        const size_t blk0 = (size_t)c0 * nblocks, nblk = (size_t)(c1 - c0) * nblocks;
-        JSDR_CUDA(cudaMemcpyAsync((char *)b->d_in + in_off, (const char *)raw + in_off, in_len,
-                                  cudaMemcpyHostToDevice, ctx->copy_in));
-        JSDR_CUDA(cudaEventRecord(ctx->ev_chunk_in[c], ctx->copy_in));
-        JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk_in[c], 0));
-        JSDR_TRY(fft::launch(f, (const char *)b->d_in + in_off, fft::IN_S16, (int)nblk, f->d_out + blk0 * N2,
-                             f->d_peak + blk0, fft::OUT_PSD, ic, qc, ctx->stream));
-        if (px)
-            JSDR_TRY(jsdr_launch_waterfall(ctx, f->d_out + blk0 * N2, f->n, (int)nblk, px->width, px->rgb,
-                                           f->d_pix + blk0 * px->width, ctx->stream));
-        JSDR_CUDA(cudaEventRecord(ctx->ev_chunk_done[c], ctx->stream));
-        JSDR_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_chunk_done[c], 0));
-        if (px) {
-            JSDR_CUDA(cudaMemcpyAsync(px->pixels + blk0 * px->width, f->d_pix + blk0 * px->width,
-                                      nblk * px->width * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->copy_out));
-            JSDR_CUDA(cudaMemcpy2DAsync(px->peak + blk0 * 2, 2 * sizeof(float), f->d_out + blk0 * N2 + f->n, N2 * sizeof(float),
-                                        2 * sizeof(float), nblk, cudaMemcpyDeviceToHost, ctx->copy_out));
-        } else {
-            JSDR_CUDA(cudaMemcpyAsync(psd + blk0 * N2, f->d_out + blk0 * N2, nblk * N2 * sizeof(float),
-                                      cudaMemcpyDeviceToHost, ctx->copy_out));
-        }
-        if (peak_bin)
-            JSDR_CUDA(cudaMemcpyAsync(peak_bin + blk0, f->d_peak + blk0, sizeof(int32_t) * nblk,
-                                      cudaMemcpyDeviceToHost, ctx->copy_out));
-    }
-    if (dm) {   // the whole batch is in (the main stream waited for every chunk): demod, audio down beside the bank
-        jsdr_demod *d = dm->d;
-        int16_t *d_audio = nullptr;
-        float *d_ma = nullptr;
-        JSDR_TRY(jsdr_pump_demod_staging(d, (int)S, nblocks, &d_audio, &d_ma));
-        JSDR_TRY(jsdr_pump_demod_run(d, static_cast<const int16_t *>(b->d_in), (int)S, f->n, ic, qc, d_audio,
-                                     dm->max_avg ? d_ma : nullptr));
-        JSDR_CUDA(cudaEventRecord(d->ev_audio_ready, ctx->stream));
-        JSDR_CUDA(cudaStreamWaitEvent(ctx->copy_out, d->ev_audio_ready, 0));
-        JSDR_CUDA(cudaMemcpyAsync(dm->audio, d_audio, sizeof(int16_t) * (size_t)b->nchan * S, cudaMemcpyDeviceToHost,
-                                  ctx->copy_out));
-        if (dm->max_avg)
-            JSDR_CUDA(cudaMemcpyAsync(dm->max_avg, d_ma, sizeof(float) * 2 * (size_t)b->nchan * nblocks,
-                                      cudaMemcpyDeviceToHost, ctx->copy_out));
-    }
-    b->in_pump = 1;
-    const int rc_bank = bpsk_receive<FMT_S16>(b, b->d_in, (int)S, S, ic, qc, JSDR_MEM_DEVICE);
-    b->in_pump = 0;
-    JSDR_TRY(rc_bank);
-    JSDR_CUDA(cudaStreamSynchronize(ctx->copy_out));
-    JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
-    return JSDR_OK;
-}
-}  // namespace
 
 // The decimator and matched-filter taps as the kernels use them ((double)(float) of the
 // F-suffixed literals, FUNcubeBPSKDemod.java:27-77), for the reference-pinning tests

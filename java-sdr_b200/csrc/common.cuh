@@ -122,6 +122,12 @@ struct PerDeviceFlag {
     }
 };
 
+// api.cu.  Copy host -> device on the context's main stream and wait for it.
+int upload(jsdr_ctx *ctx, void *dst, const void *src, size_t bytes);
+// Grow-on-demand device buffer: *p holds *cap bytes; if fewer than `bytes`, it is freed and
+// reallocated (contents lost).
+int grow(void **p, size_t *cap, size_t bytes);
+
 // Check the launch that was just made and count it.
 static inline int launched(jsdr_ctx *ctx, const char *what)
 {

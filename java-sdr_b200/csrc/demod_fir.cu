@@ -360,25 +360,6 @@ static int java_d2i(double d)
 using namespace jsdr;
 using namespace jsdr::dsp;
 
-namespace {
-int upload(jsdr_ctx *ctx, void *dst, const void *src, size_t bytes)
-{
-    JSDR_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
-    return JSDR_OK;
-}
-int grow(void **p, size_t *cap, size_t bytes)
-{
-    if (*cap >= bytes) return JSDR_OK;
-    cudaFree(*p);
-    *p = nullptr;
-    *cap = 0;
-    JSDR_CUDA(cudaMalloc(p, bytes));
-    *cap = bytes;
-    return JSDR_OK;
-}
-}  // namespace
-
 // =========================================================================== demod
 extern "C" int jsdr_demod_create(jsdr_ctx *ctx, int rate, int nchan, int max_block_samples, jsdr_demod **out)
 try {
@@ -869,7 +850,7 @@ try {
 } JSDR_CATCH_ALL
 
 // ------------------------------------------------------------------ the pump's demod handler
-// jsdr_pump_demod_s16 (bpsk.cu) runs demod over the pump's resident rows of S samples per channel
+// jsdr_pump_demod_s16 (pump.cu) runs demod over the pump's resident rows of S samples per channel
 // (chan_stride S) as nblocks successive demod.receive calls of L samples: one FIR + NCO launch over
 // the whole row (the delay line and car carry from call to call anyway), then k_detect per block.
 

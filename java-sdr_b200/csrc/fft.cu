@@ -349,27 +349,15 @@ try {
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
-namespace {
-
-int ensure_staging(jsdr_fft *f, size_t in_bytes, size_t out_bytes)
+int jsdr::fft::ensure_staging(jsdr_fft *f, size_t in_bytes, size_t out_bytes)
 {
-    if (f->in_cap < in_bytes) {
-        cudaFree(f->d_in);
-        f->d_in = nullptr;
-        f->in_cap = 0;
-        JSDR_CUDA(cudaMalloc(&f->d_in, in_bytes));
-        f->in_cap = in_bytes;
-    }
-    if (f->out_cap < out_bytes) {
-        cudaFree(f->d_out);
-        f->d_out = nullptr;
-        f->out_cap = 0;
-        JSDR_CUDA(cudaMalloc(&f->d_out, out_bytes));
-        f->out_cap = out_bytes;
-    }
+    JSDR_TRY(grow(&f->d_in, &f->in_cap, in_bytes));
+    JSDR_TRY(grow(reinterpret_cast<void **>(&f->d_out), &f->out_cap, out_bytes));
     if (!f->d_peak) JSDR_CUDA(cudaMalloc(&f->d_peak, sizeof(int32_t) * (size_t)f->max_batch));
     return JSDR_OK;
 }
+
+namespace {
 
 // shared body of the three receive flavours
 int fft_run(jsdr_fft *f, const void *in, int in_fmt, int batch, int ic, int qc, float *out,
@@ -387,7 +375,7 @@ int fft_run(jsdr_fft *f, const void *in, int in_fmt, int batch, int ic, int qc, 
     if (mem == JSDR_MEM_DEVICE) {
         return fft::launch(f, in, in_fmt, batch, out, peak_bin, out_mode, ic, qc, ctx->stream);
     }
-    JSDR_TRY(ensure_staging(f, in_bytes, out_elems * sizeof(float)));
+    JSDR_TRY(fft::ensure_staging(f, in_bytes, out_elems * sizeof(float)));
     JSDR_CUDA(cudaMemcpyAsync(f->d_in, in, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
     JSDR_TRY(fft::launch(f, f->d_in, in_fmt, batch, f->d_out, f->d_peak, out_mode, ic, qc, ctx->stream));
     JSDR_CUDA(cudaMemcpyAsync(out, f->d_out, out_elems * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));

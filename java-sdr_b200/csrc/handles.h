@@ -46,6 +46,7 @@ struct AutoTuneState {
     int centreBin, pad;
 };
 
+enum { FMT_F32 = 0, FMT_S16 = 1 };   // input: (float I, float Q) or s16le (I, Q) pairs
 struct ScoutChan;                    // bpsk.cu
 constexpr int kMaxDsTaps = 128;
 constexpr int kDmTaps = 65;          // MATCHED_FILTER_SIZE
@@ -76,7 +77,6 @@ struct jsdr_bpsk {
     unsigned long long *d_tu_dx56 = nullptr; // [nchan] the same in 8.56 fixed point (streaming kernel)
     int precision = 0;               // JSDR_PREC_F64 (exact) or JSDR_PREC_F32 (decimator in binary32)
     int kernel_mode = 0;             // JSDR_KERNEL_AUTO / _TILE / _STREAM
-    int in_pump = 0;                 // set by jsdr_pump_receive_s16 around the bank's receive
     double *d_tu_phase0 = nullptr;   // [nchan] initial tuPhase (zeros)
     const double *d_tu_phase = nullptr;   // committed tuPhase: phase0 or the phase_end of the last plan used
     // Scout output ("plan") for one block.  Two of them: while the data kernels work
@@ -172,7 +172,7 @@ struct jsdr_fir {
     size_t in_cap = 0, out_cap = 0;
 };
 
-// demod_fir.cu: the demod handler of jsdr_pump_demod_s16 (bpsk.cu)
+// demod_fir.cu: the demod handler of jsdr_pump_demod_s16 (pump.cu)
 int jsdr_pump_demod_fork(jsdr_demod *d, int S);
 int jsdr_pump_demod_staging(jsdr_demod *d, int S, int nblocks, int16_t **d_audio, float **d_max_avg);
 int jsdr_pump_demod_run(jsdr_demod *d, const int16_t *d_raw, int S, int L, int ic, int qc, int16_t *audio,
@@ -188,5 +188,19 @@ enum { OUT_PSD = 0, OUT_SPECTRUM = 1 };
 // enqueue one batched transform on `st` (all pointers are device memory)
 int launch(jsdr_fft *f, const void *d_in, int in_fmt, int batch, float *d_out, int32_t *d_peak,
            int out_mode, int ic, int qc, cudaStream_t st);
+// grow the host-call staging d_in / d_out to at least these sizes; d_peak holds max_batch bins
+int ensure_staging(jsdr_fft *f, size_t in_bytes, size_t out_bytes);
 }  // namespace fft
+
+namespace bpsk {
+// bpsk.cu: jsdr_bpsk_receive_* (`fmt` FMT_F32 / FMT_S16), and the same in two halves for the pump
+// (pump.cu), which enqueues its own kernels between them.  `pump` sizes the phase replay and the
+// decimator's grid for a pump step (scout_threads, launch_stream).
+int receive(jsdr_bpsk *b, const void *in, int fmt, int S, long long chan_stride, int ic, int qc, int mem,
+            bool pump);
+int receive_begin(jsdr_bpsk *b, const void *in, int fmt, int S, long long chan_stride, int mem, bool pump,
+                  const void **d_in);
+int receive_end(jsdr_bpsk *b, const void *d_in, int fmt, int S, long long chan_stride, int ic, int qc, int mem,
+                bool pump);
+}  // namespace bpsk
 }  // namespace jsdr

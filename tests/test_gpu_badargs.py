@@ -133,6 +133,13 @@ def test_bad_arguments_on_live_handles(ctx):
     refused(L.jsdr_pump_receive_s16, f.h, b.h, p(raw), 2, 0, 0, p(big), None, 0)      # 3 ch x 2 blocks > max_batch 4
     refused(L.jsdr_pump_receive_s16, f.h, b.h, None, 1, 0, 0, p(big), None, 0)
     refused(L.jsdr_pump_waterfall_s16, f.h, b.h, p(raw), 1, 0, 0, 0, 0xffff, p(pix), p(psd), None, 0)
+    d3 = J.demod(ctx, adsc, nchan=3, max_block=2 * n)
+    audio = np.zeros((3, n), np.int16)
+    for mem in (-1, 2):                  # every other argument is valid: only mem is refused
+        refused(L.jsdr_pump_receive_s16, f.h, b.h, p(raw), 1, 0, 0, p(big), None, mem)
+        refused(L.jsdr_pump_waterfall_s16, f.h, b.h, p(raw), 1, 0, 0, 16, 0xffff, p(pix), p(psd), None, mem)
+        refused(L.jsdr_pump_demod_s16, f.h, b.h, d3.h, p(raw), 1, 0, 0, p(big), None, p(audio), None, mem)
+    d3.close()
     # ---- memory and context
     q = C.c_void_p()
     refused(L.jsdr_dev_alloc, ctx.h, 1 << 50, C.byref(q))

@@ -11,7 +11,7 @@ BUILD = os.path.join(ROOT, "java-sdr_b200", "csrc", "build")
 KERNELS = [
     ("fft_n4096.o", r"fft_kernelINS0_4PlanILi4096.*Li1ELi0E", "fft_kernel<Plan<4096,64,1,64,64>, IN_S16, OUT_PSD>"),
     ("bpsk.o", r"k_mixdecim_streamILi1ELi0ELi64ELi20ELi16E", "k_mixdecim_stream<S16, F64, 64 taps, D=20, 16 warps>"),
-    ("bpsk.o", r"k_tuner_scoutILi1E", "k_tuner_scout<1>"),
+    ("bpsk.o", r"k_tuner_scoutEPK", "k_tuner_scout"),
     ("fec.o", r"k_fec_decode", "k_fec_decode"),
 ]
 INS = re.compile(r"^\s+/\*([0-9a-f]{4,})\*/\s+(.*?);")

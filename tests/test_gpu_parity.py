@@ -418,28 +418,6 @@ def test_pump_equals_separate_handlers(ctx):
         h.close()
 
 
-@pytest.mark.parametrize("n", [9600, 16384, 19200])
-def test_fft_persistent_plans_many_blocks_per_cta(ctx, n):
-    """Plans whose block fills an SM's shared memory run persistent CTAs that loop over the
-    batch and prefetch the next block's samples; a batch several times the number of resident
-    CTAs must give every block its own spectrum (s16 and float input)."""
-    batch = 700
-    rng = np.random.default_rng(n)
-    raw = rng.integers(-32768, 32768, (batch, 2 * n)).astype(np.int16)
-    for b in range(batch):
-        raw[b, 0] = (b * 37) % 30000                       # make neighbours differ at DC
-    f = J.fft(ctx, None, J.AudioDescriptor(192000), max_batch=batch, n=n)
-    psd, pk = f.receive_batch(raw, s16=True)
-    psd_f, pk_f = f.receive_batch(O.s16_to_float(raw.ravel()).reshape(batch, 2 * n))
-    for b in (0, 1, 147, 148, 149, 295, 296, 443, 444, 698, 699):
-        pw = O.fft_power_f64(O.s16_to_float(raw[b]))
-        for got in (psd, psd_f):
-            amp = np.power(10.0, got[b, :n].astype(np.float64) / 20.0)
-            assert np.max(np.abs(amp - np.sqrt(pw))) <= 2e-4, b
-        assert pk[b] == int(np.argmax(psd[b, :n])) and psd[b, n + 1] == psd[b, pk[b]]
-    f.close()
-
-
 def test_error_paths_return_codes_not_crashes(ctx):
     """Nothing may throw through IAudioHandler.receive (JavaAudio.java:321-323): bad calls come
     back as status codes with a message, and the handles stay usable."""

@@ -1,6 +1,7 @@
 // api.cu — context, memory and timing entry points of libjsdrcuda.so.
 #include <algorithm>
 #include <cstdlib>
+#include <memory>
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
@@ -26,15 +27,11 @@ int upload(jsdr_ctx *ctx, void *dst, const void *src, size_t bytes)
     return JSDR_OK;
 }
 
-int grow(void **p, size_t *cap, size_t bytes)
+int cuda_failed(cudaError_t e, const char *what, const char *call)
 {
-    if (*cap >= bytes) return JSDR_OK;
-    cudaFree(*p);
-    *p = nullptr;
-    *cap = 0;
-    JSDR_CUDA(cudaMalloc(p, bytes));
-    *cap = bytes;
-    return JSDR_OK;
+    set_error("%s: %s: %s", what, call, cudaGetErrorString(e));
+    cudaGetLastError();   // reported: the next launch check must not see it
+    return e == cudaErrorMemoryAllocation ? JSDR_ENOMEM : JSDR_ECUDA;
 }
 
 }  // namespace jsdr
@@ -75,20 +72,17 @@ try {
                   device, prop.major, prop.minor);
         return JSDR_EUNSUPPORTED;
     }
-    jsdr_ctx *ctx = new jsdr_ctx();
+    std::unique_ptr<jsdr_ctx> ctx(new jsdr_ctx());
     ctx->device = device;
     ctx->sm_count = prop.multiProcessorCount;
-    const int rc = ctx_init(ctx);
-    if (rc != JSDR_OK) {                              // half-built: release what exists (destroy skips null handles)
-        jsdr_ctx_destroy(ctx);
-        return rc;
-    }
-    *out = ctx;
+    JSDR_TRY(ctx_init(ctx.get()));
+    *out = ctx.release();
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
 static int ctx_init(jsdr_ctx *ctx)
 {
+    const char *what = "jsdr_ctx_create";
     if (const char *e = getenv("JSDR_L2_PREFETCH")) ctx->l2_prefetch = std::max(0, std::min(atoi(e), 8));   // 0: off, n: n x resident CTAs ahead
     {   // three priorities: the side stream carries the serial, data-independent phase replay and
         // goes first, so that its few CTAs are placed as soon as a slot frees up instead of queueing
@@ -97,49 +91,31 @@ static int ctx_init(jsdr_ctx *ctx)
         int lo = 0, hi = 0;
         JSDR_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
         const int mid = (hi < lo) ? lo - 1 : lo;
-        JSDR_CUDA(cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, mid));
-        JSDR_CUDA(cudaStreamCreateWithPriority(&ctx->side, cudaStreamNonBlocking, hi));
-        JSDR_CUDA(cudaStreamCreateWithPriority(&ctx->side2, cudaStreamNonBlocking, hi));
-        JSDR_CUDA(cudaStreamCreateWithPriority(&ctx->aux, cudaStreamNonBlocking, lo));
+        JSDR_TRY(ctx->stream.create(mid, what));
+        JSDR_TRY(ctx->side.create(hi, what));
+        JSDR_TRY(ctx->side2.create(hi, what));
+        JSDR_TRY(ctx->aux.create(lo, what));
     }
-    JSDR_CUDA(cudaStreamCreateWithFlags(&ctx->copy_in, cudaStreamNonBlocking));
-    JSDR_CUDA(cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking));
+    JSDR_TRY(ctx->copy_in.create(0, what));
+    JSDR_TRY(ctx->copy_out.create(0, what));
     for (int i = 0; i < 16; i++) {
-        JSDR_CUDA(cudaEventCreateWithFlags(&ctx->ev_chunk_in[i], cudaEventDisableTiming));
-        JSDR_CUDA(cudaEventCreateWithFlags(&ctx->ev_chunk_done[i], cudaEventDisableTiming));
+        JSDR_TRY(ctx->ev_chunk_in[i].create(what));
+        JSDR_TRY(ctx->ev_chunk_done[i].create(what));
     }
-    JSDR_CUDA(cudaEventCreate(&ctx->ev_t0));
-    JSDR_CUDA(cudaEventCreate(&ctx->ev_t1));
-    JSDR_CUDA(cudaEventCreateWithFlags(&ctx->ev_aux_fork, cudaEventDisableTiming));
-    JSDR_CUDA(cudaEventCreateWithFlags(&ctx->ev_aux_join, cudaEventDisableTiming));
-    JSDR_CUDA(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
-    JSDR_CUDA(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
+    JSDR_TRY(ctx->ev_t0.create(what, cudaEventDefault));
+    JSDR_TRY(ctx->ev_t1.create(what, cudaEventDefault));
+    JSDR_TRY(ctx->ev_aux_fork.create(what));
+    JSDR_TRY(ctx->ev_aux_join.create(what));
+    JSDR_TRY(ctx->ev_fork.create(what));
+    JSDR_TRY(ctx->ev_join.create(what));
     return JSDR_OK;
 }
 
 extern "C" int jsdr_ctx_destroy(jsdr_ctx *ctx)
 try {
     if (!ctx) return JSDR_OK;
-    ctx->bind();
-    cudaStream_t *streams[] = {&ctx->stream, &ctx->side, &ctx->side2, &ctx->aux, &ctx->copy_in, &ctx->copy_out};
-    for (cudaStream_t *s : streams)
-        if (*s) cudaStreamSynchronize(*s);            // events below may still be pending on any of them
-    cudaEvent_t evs[] = {ctx->ev_t0, ctx->ev_t1, ctx->ev_aux_fork, ctx->ev_aux_join, ctx->ev_fork, ctx->ev_join};
-    for (cudaEvent_t e : evs)
-        if (e) cudaEventDestroy(e);
-    for (auto *v : {&ctx->spans, &ctx->free_spans})
-        for (jsdr_prof_span &sp : *v) {
-            cudaEventDestroy(sp.a);
-            cudaEventDestroy(sp.b);
-        }
-    for (int i = 0; i < 16; i++) {
-        if (ctx->ev_chunk_in[i]) cudaEventDestroy(ctx->ev_chunk_in[i]);
-        if (ctx->ev_chunk_done[i]) cudaEventDestroy(ctx->ev_chunk_done[i]);
-    }
-    for (cudaStream_t *s : streams)
-        if (*s) cudaStreamDestroy(*s);
-    cudaGetLastError();
     delete ctx;
+    cudaGetLastError();
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
@@ -195,7 +171,7 @@ try {
             cudaGetLastError();
             rc = JSDR_ECUDA;
         }
-        ctx->free_spans.push_back(sp);                // every span moves exactly once, error or not
+        ctx->free_spans.push_back(std::move(sp));     // every span moves exactly once, error or not
     }
     ctx->spans.clear();
     return rc;

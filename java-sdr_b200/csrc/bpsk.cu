@@ -923,7 +923,7 @@ int launch_scout(jsdr_bpsk *b, jsdr_bpsk::TunerPlan &P, int S, bool pump)
         return JSDR_OK;
     }));
     const int grid = (b->nchan + st - 1) / st;
-    k_tuner_scout<<<grid, st, scout_smem, ctx->side>>>(b->d_tu_par, b->d_tu_phase, P.phase_end, P.ckpt, b->nchan, S);
+    k_tuner_scout<<<grid, st, scout_smem, ctx->side>>>(b->d_tu_par.get(), b->d_tu_phase, P.phase_end.get(), P.ckpt.get(), b->nchan, S);
     JSDR_TRY(launched(ctx, "k_tuner_scout"));
     JSDR_CUDA(cudaEventRecord(P.ready, ctx->side));
     P.S = S;
@@ -942,15 +942,15 @@ int launch_vco_scout(jsdr_bpsk *b, int NO, int kb)
     // (the bit-timing kernel of two blocks ago may still be reading this buffer)
     // Own stream: a one-CTA serial chain of about a third of the tuner scout's length; behind that
     // scout on the same stream it made the side stream the critical path of the whole chain.
-    if (b->bits_used[kb]) JSDR_CUDA(cudaStreamWaitEvent(ctx->side2, b->ev_bits_done[kb], 0));
+    if (b->bits_used[kb]) JSDR_CUDA(cudaStreamWaitEvent(ctx->side2, b->stage.ev_bits_done[kb], 0));
     // (and the matched filter that last read this buffer, two blocks ago, is done: the event is the
     // newer one of the previous block)
-    if (b->ev_dm_ready) JSDR_CUDA(cudaStreamWaitEvent(ctx->side2, b->ev_dm_ready, 0));
+    if (b->stage.ev_dm_ready) JSDR_CUDA(cudaStreamWaitEvent(ctx->side2, b->stage.ev_dm_ready, 0));
     const int c = b->vco_state_cur;
-    k_vco_scout<<<1, 64, 0, ctx->side2>>>(b->d_vco_state + 2 * c, b->d_vco_state + 2 * (c ^ 1), b->d_vco_ix[kb],
-                                         b->d_bit_roll[kb], NO, vco_inc, bit_inc, bit_time);
+    k_vco_scout<<<1, 64, 0, ctx->side2>>>(b->d_vco_state.get() + 2 * c, b->d_vco_state.get() + 2 * (c ^ 1), b->stage.d_vco_ix[kb].get(),
+                                         b->stage.d_bit_roll[kb].get(), NO, vco_inc, bit_inc, bit_time);
     JSDR_TRY(launched(ctx, "k_vco_scout"));
-    JSDR_CUDA(cudaEventRecord(b->ev_vco_ready, ctx->side2));
+    JSDR_CUDA(cudaEventRecord(b->stage.ev_vco_ready, ctx->side2));
     return JSDR_OK;
 }
 
@@ -958,37 +958,25 @@ int launch_vco_scout(jsdr_bpsk *b, int NO, int kb)
 // stages==1 bank, e.g. the mix+FIR benchmark, never pays for them).
 int ensure_stage_buffers(jsdr_bpsk *b)
 {
-    if (b->d_dm_buf[1]) return JSDR_OK;
+    if (b->stage.d_bits) return JSDR_OK;
     jsdr_ctx *ctx = b->ctx;
+    const char *what = "stage buffers";
     const size_t nc = (size_t)b->nchan;
-    struct { void **p; size_t bytes; } req[] = {
-        {(void **)&b->d_vco_ix[0], (size_t)b->max_ds},
-        {(void **)&b->d_vco_ix[1], (size_t)b->max_ds},
-        {(void **)&b->d_bit_roll[0], (size_t)b->max_ds},
-        {(void **)&b->d_bit_roll[1], (size_t)b->max_ds},
-        {(void **)&b->d_dm_hist[0], sizeof(double2) * 64 * nc},
-        {(void **)&b->d_dm_hist[1], sizeof(double2) * 64 * nc},
-        {(void **)&b->d_bits, nc * b->max_bits},
-        {(void **)&b->d_bit_at, sizeof(long long) * nc * b->max_bits},
-        {(void **)&b->d_dm_buf[0], sizeof(double2) * nc * b->max_ds},
-        {(void **)&b->d_dm_buf[1], sizeof(double2) * nc * b->max_ds},
-    };
-    for (auto &r : req) {
-        cudaError_t e = cudaMalloc(r.p, r.bytes);
-        if (e != cudaSuccess) {
-            set_error("stage buffers: cudaMalloc(%zu): %s", r.bytes, cudaGetErrorString(e));
-            cudaGetLastError();
-            return JSDR_ENOMEM;
-        }
-        JSDR_CUDA(cudaMemsetAsync(*r.p, 0, r.bytes, ctx->stream));
-    }
-    b->d_dm_out = b->d_dm_buf[0];
-    JSDR_CUDA(cudaEventCreateWithFlags(&b->ev_dm_ready, cudaEventDisableTiming));
-    JSDR_CUDA(cudaEventCreateWithFlags(&b->ev_vco_ready, cudaEventDisableTiming));
-    for (int i = 0; i < 2; i++) JSDR_CUDA(cudaEventCreateWithFlags(&b->ev_bits_done[i], cudaEventDisableTiming));
+    jsdr_bpsk::Stages g;
+    for (int i = 0; i < 2; i++) JSDR_TRY(g.d_vco_ix[i].alloc_zeroed((size_t)b->max_ds, ctx->stream, what));
+    for (int i = 0; i < 2; i++) JSDR_TRY(g.d_bit_roll[i].alloc_zeroed((size_t)b->max_ds, ctx->stream, what));
+    for (int i = 0; i < 2; i++) JSDR_TRY(g.d_dm_hist[i].alloc_zeroed(sizeof(double2) * 64 * nc, ctx->stream, what));
+    JSDR_TRY(g.d_bits.alloc_zeroed(nc * b->max_bits, ctx->stream, what));
+    JSDR_TRY(g.d_bit_at.alloc_zeroed(sizeof(long long) * nc * b->max_bits, ctx->stream, what));
+    for (int i = 0; i < 2; i++) JSDR_TRY(g.d_dm_buf[i].alloc_zeroed(sizeof(double2) * nc * b->max_ds, ctx->stream, what));
+    JSDR_TRY(g.ev_dm_ready.create(what));
+    JSDR_TRY(g.ev_vco_ready.create(what));
+    for (int i = 0; i < 2; i++) JSDR_TRY(g.ev_bits_done[i].create(what));
     // the bit stage starts on the auxiliary stream: order it behind the clears above
-    JSDR_CUDA(cudaEventRecord(b->ev_dm_ready, ctx->stream));
-    JSDR_CUDA(cudaStreamWaitEvent(ctx->aux, b->ev_dm_ready, 0));
+    JSDR_CUDA(cudaEventRecord(g.ev_dm_ready, ctx->stream));
+    JSDR_CUDA(cudaStreamWaitEvent(ctx->aux, g.ev_dm_ready, 0));
+    b->stage = std::move(g);
+    b->d_dm_out = b->stage.d_dm_buf[0].get();
     return JSDR_OK;
 }
 
@@ -996,7 +984,7 @@ int bpsk_reset_ds(jsdr_bpsk *b)
 {
     jsdr_ctx *ctx = b->ctx;
     for (int i = 0; i < 2; i++)
-        JSDR_CUDA(cudaMemsetAsync(b->d_ds_hist[i], 0, sizeof(double2) * kMaxDsTaps * (size_t)b->nchan, ctx->stream));
+        JSDR_CUDA(cudaMemsetAsync(b->d_ds_hist[i].get(), 0, sizeof(double2) * kMaxDsTaps * (size_t)b->nchan, ctx->stream));
     b->ds_cnt = 0;
     b->ds_hist_cur = 0;
     return JSDR_OK;
@@ -1032,7 +1020,7 @@ int launch_stream(jsdr_bpsk *b, const MixParams &mp, int S, bool pump)
     sp.S = S;
     sp.ic = mp.ic;
     sp.qc = mp.qc;
-    sp.tu_dx56 = b->d_tu_dx56;
+    sp.tu_dx56 = b->d_tu_dx56.get();
     sp.tu_inc = mp.tu_inc;
     sp.ckpt = mp.ckpt;
     sp.nchan = mp.nchan;
@@ -1063,7 +1051,7 @@ int launch_stream(jsdr_bpsk *b, const MixParams &mp, int S, bool pump)
     sp.nseg = (mp.NO + R - 1) / R;
     sp.ds_out = mp.ds_out;
     sp.max_ds = mp.max_ds;
-    sp.work_counter = reinterpret_cast<unsigned *>(b->d_nbits + b->nchan);   // one spare word behind nbits[]
+    sp.work_counter = reinterpret_cast<unsigned *>(b->d_nbits.get() + b->nchan);   // one spare word behind nbits[]
     for (int k = 0; k < stream::kMaxTaps; k++) {
         sp.taps[k] = (k < b->ntaps) ? b->h_taps[k] : 0.0;
         sp.tapsf[k] = (float)sp.taps[k];
@@ -1088,38 +1076,35 @@ int autotune_block(jsdr_bpsk *b, const void *d_in, int S, long long chan_stride,
     jsdr_ctx *ctx = b->ctx;
     const int nchan = b->nchan, N = S;
     const size_t bytes = sizeof(double2) * (size_t)nchan * (size_t)N;
-    if (!b->d_at_state) {
-        void **bufs[] = {(void **)&b->d_at_work[0], (void **)&b->d_at_work[1], (void **)&b->d_at_rev[0], (void **)&b->d_at_rev[1]};
-        for (void **pp : bufs) {
-            cudaError_t e = cudaMalloc(pp, bytes);
-            if (e != cudaSuccess) {
-                set_error("auto-tune workspace: cudaMalloc(%zu): %s", bytes, cudaGetErrorString(e));
-                cudaGetLastError();
-                return JSDR_ENOMEM;
-            }
-        }
-        JSDR_CUDA(cudaMalloc((void **)&b->d_at_state, sizeof(AutoTuneState) * (size_t)nchan));
-        JSDR_CUDA(cudaMemsetAsync(b->d_at_state, 0, sizeof(AutoTuneState) * (size_t)nchan, ctx->stream));
+    if (!b->at.d_at_state) {
+        const char *what = "auto-tune workspace";
+        jsdr_bpsk::AutoTune g;
+        for (int i = 0; i < 2; i++) JSDR_TRY(g.d_at_work[i].alloc(bytes, what));
+        for (int i = 0; i < 2; i++) JSDR_TRY(g.d_at_rev[i].alloc(bytes, what));
+        JSDR_TRY(g.d_at_state.alloc_zeroed(sizeof(AutoTuneState) * (size_t)nchan, ctx->stream, what));
+        b->at = std::move(g);
     }
+    double2 *work[2] = {b->at.d_at_work[0].get(), b->at.d_at_work[1].get()};
+    double2 *rev[2] = {b->at.d_at_rev[0].get(), b->at.d_at_rev[1].get()};
     JSDR_REQUIRE(fftg::make_plan(N).nstages > 0, JSDR_EUNSUPPORTED, "block length has a prime factor other than 2, 3, 5, 7");
     JSDR_REQUIRE(N >= 1024 && N <= kAutoTuneMaxN, JSDR_EUNSUPPORTED, "auto-tune needs blocks of 1024 to 115712 samples");
     const long long total = (long long)nchan * N;
-    k_at_load<FMT><<<(unsigned)((total + 255) / 256), 256, 0, ctx->stream>>>(d_in, chan_stride, S, nchan, ic, qc, b->d_at_work[0]);
+    k_at_load<FMT><<<(unsigned)((total + 255) / 256), 256, 0, ctx->stream>>>(d_in, chan_stride, S, nchan, ic, qc, work[0]);
     JSDR_TRY(launched(ctx, "k_at_load"));
     int rc = JSDR_OK;
-    double2 *fwd = fftg::run<double>(ctx, ctx->stream, b->d_at_work[0], b->d_at_work[1], N, nchan, -1, &rc);   // :422-423
+    double2 *fwd = fftg::run<double>(ctx, ctx->stream, work[0], work[1], N, nchan, -1, &rc);   // :422-423
     if (rc != JSDR_OK) return rc;
-    JSDR_CUDA(cudaMemsetAsync(b->d_at_rev[0], 0, bytes, ctx->stream));                                         // :419-420
+    JSDR_CUDA(cudaMemsetAsync(rev[0], 0, bytes, ctx->stream));                                         // :419-420
     const size_t smem = sizeof(double) * (size_t)(N / 4 + 64);
     JSDR_CUDA(cudaFuncSetAttribute(k_at_search, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_at_search<<<nchan, 256, smem, ctx->stream>>>(fwd, b->d_at_rev[0], N, b->doUp, b->d_at_state);
+    k_at_search<<<nchan, 256, smem, ctx->stream>>>(fwd, rev[0], N, b->doUp, b->at.d_at_state.get());
     JSDR_TRY(launched(ctx, "k_at_search"));
-    double2 *inv = fftg::run<double>(ctx, ctx->stream, b->d_at_rev[0], b->d_at_rev[1], N, nchan, +1, &rc);     // :459
+    double2 *inv = fftg::run<double>(ctx, ctx->stream, rev[0], rev[1], N, nchan, +1, &rc);     // :459
     if (rc != JSDR_OK) return rc;
     dim3 grid((std::max(NO, 1) + 127) / 128, nchan);
-    k_at_decim<<<grid, 128, 0, ctx->stream>>>(inv, N, 1.0 / (double)N, b->d_ds_hist[b->ds_hist_cur],
-                                              b->d_ds_hist[b->ds_hist_cur ^ 1], b->d_taps, b->ntaps, b->D, n0, NO,
-                                              b->d_ds_out, b->max_ds);
+    k_at_decim<<<grid, 128, 0, ctx->stream>>>(inv, N, 1.0 / (double)N, b->d_ds_hist[b->ds_hist_cur].get(),
+                                              b->d_ds_hist[b->ds_hist_cur ^ 1].get(), b->d_taps.get(), b->ntaps, b->D, n0, NO,
+                                              b->d_ds_out.get(), b->max_ds);
     return launched(ctx, "k_at_decim");
 }
 
@@ -1138,20 +1123,20 @@ int mix_decimate(jsdr_bpsk *b, const void *d_in, int S, long long chan_stride, i
     mp.S = S;
     mp.ic = ic;
     mp.qc = qc;
-    mp.tu_inc = b->d_tu_inc;
-    mp.tu_dx = b->d_tu_dx;
+    mp.tu_inc = b->d_tu_inc.get();
+    mp.tu_dx = b->d_tu_dx.get();
     mp.ckpt = ckpt;
     mp.nchan = nchan;
-    mp.hist_in = b->d_ds_hist[b->ds_hist_cur];
-    mp.hist_out = b->d_ds_hist[b->ds_hist_cur ^ 1];
+    mp.hist_in = b->d_ds_hist[b->ds_hist_cur].get();
+    mp.hist_out = b->d_ds_hist[b->ds_hist_cur ^ 1].get();
     mp.ntaps = b->ntaps;
-    mp.cossin = b->d_cossin2;
+    mp.cossin = b->d_cossin2.get();
     mp.D = D;
     mp.n0 = n0;
     mp.NO = NO;
     mp.magicD = (unsigned)(4294967296ULL / (unsigned)D) + 1u;
     mp.pad = (D & 1) ? 0 : 1;          // even D: one pad slot per D samples makes the lane stride odd
-    mp.ds_out = b->d_ds_out;
+    mp.ds_out = b->d_ds_out.get();
     mp.max_ds = b->max_ds;
     memcpy(mp.taps, b->h_taps, sizeof(mp.taps));
     {
@@ -1219,8 +1204,8 @@ int jsdr::bpsk::receive_begin(jsdr_bpsk *b, const void *in, int fmt, int S, long
     if (b->stages >= 2) JSDR_TRY(ensure_stage_buffers(b));   // (before the empty-block return: the reads that follow an
                                                              //  empty FIRST block answer "nothing", not "stage has not run")
     if (S == 0) {
-        JSDR_CUDA(cudaMemsetAsync(b->d_nbits, 0, sizeof(int32_t) * b->nchan, ctx->aux));
-        if (b->fec && b->stages >= 3 && b->d_bits) JSDR_TRY(jsdr_fec_after_bits(b));   // no bits: no frames either
+        JSDR_CUDA(cudaMemsetAsync(b->d_nbits.get(), 0, sizeof(int32_t) * b->nchan, ctx->aux));
+        if (b->fec && b->stages >= 3 && b->stage.d_bits) JSDR_TRY(jsdr_fec_after_bits(b));   // no bits: no frames either
         return JSDR_OK;
     }
     const int NO = (b->ds_cnt + S) / b->D;
@@ -1246,9 +1231,9 @@ int jsdr::bpsk::receive_begin(jsdr_bpsk *b, const void *in, int fmt, int S, long
     if (mem == JSDR_MEM_HOST) {
         const size_t esz = (fmt == FMT_S16) ? 4 : 8;
         const size_t bytes = esz * ((chan_stride == 0) ? (size_t)S : (size_t)chan_stride * (b->nchan - 1) + S);
-        JSDR_TRY(grow(&b->d_in, &b->in_cap, bytes));
-        JSDR_CUDA(cudaMemcpyAsync(b->d_in, in, bytes, cudaMemcpyHostToDevice, ctx->stream));
-        in = b->d_in;
+        JSDR_TRY(b->d_in.grow(bytes, "tuner bank staging"));
+        JSDR_CUDA(cudaMemcpyAsync(b->d_in.get(), in, bytes, cudaMemcpyHostToDevice, ctx->stream));
+        in = b->d_in.get();
     }
     *d_in = in;
     return JSDR_OK;
@@ -1274,15 +1259,15 @@ int jsdr::bpsk::receive_end(jsdr_bpsk *b, const void *d_in, int fmt, int S, long
         JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, P.ready, 0));
         // (ev_join — the VCO / bit-phase replay of this block — is only needed by the matched filter:
         // the tuner + decimator runs beside it)
-        JSDR_TRY(s16 ? mix_decimate<FMT_S16>(b, d_in, S, chan_stride, ic, qc, n0, NO, P.ckpt, pump)
-                     : mix_decimate<FMT_F32>(b, d_in, S, chan_stride, ic, qc, n0, NO, P.ckpt, pump));
+        JSDR_TRY(s16 ? mix_decimate<FMT_S16>(b, d_in, S, chan_stride, ic, qc, n0, NO, P.ckpt.get(), pump)
+                     : mix_decimate<FMT_F32>(b, d_in, S, chan_stride, ic, qc, n0, NO, P.ckpt.get(), pump));
         // this plan is consumed: its end phase becomes the committed phase, and the
         // scout starts on the next block (same length assumed) while the rest of this
         // one is still in flight
         JSDR_CUDA(cudaEventRecord(P.consumed, ctx->stream));
         P.used = true;
         P.valid = false;
-        b->d_tu_phase = P.phase_end;
+        b->d_tu_phase = P.phase_end.get();
         b->plan_cur ^= 1;
         jsdr_bpsk::TunerPlan &Pn = b->plan[b->plan_cur];
         if (Pn.used) JSDR_CUDA(cudaStreamWaitEvent(ctx->side, Pn.consumed, 0));
@@ -1295,21 +1280,21 @@ int jsdr::bpsk::receive_end(jsdr_bpsk *b, const void *d_in, int fmt, int S, long
 
     // ---- matched filter, bit timing
     if (b->stages >= 2 && NO > 0) {
-        JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, b->ev_vco_ready, 0));
+        JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, b->stage.ev_vco_ready, 0));
         b->vco_state_cur ^= 1;                         // this block's replay is consumed: its end state is committed
         DmParams dp;
-        dp.ds = b->d_ds_out;
+        dp.ds = b->d_ds_out.get();
         dp.max_ds = b->max_ds;
         dp.NO = NO;
-        dp.vco_ix = b->d_vco_ix[kb];
-        dp.hist_in = b->d_dm_hist[b->dm_hist_cur];
-        dp.hist_out = b->d_dm_hist[b->dm_hist_cur ^ 1];
-        dp.dmtaps = b->d_dmtaps;
-        dp.cossin = b->d_cossin;
+        dp.vco_ix = b->stage.d_vco_ix[kb].get();
+        dp.hist_in = b->stage.d_dm_hist[b->dm_hist_cur].get();
+        dp.hist_out = b->stage.d_dm_hist[b->dm_hist_cur ^ 1].get();
+        dp.dmtaps = b->d_dmtaps.get();
+        dp.cossin = b->d_cossin.get();
         dp.base65 = (int)(b->cnt_ds % 65);
-        dp.dm_out = b->d_dm_buf[kb];
-        b->d_dm_out = b->d_dm_buf[kb];
-        if (b->bits_used[kb]) JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, b->ev_bits_done[kb], 0));
+        dp.dm_out = b->stage.d_dm_buf[kb].get();
+        b->d_dm_out = b->stage.d_dm_buf[kb].get();
+        if (b->bits_used[kb]) JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, b->stage.ev_bits_done[kb], 0));
         dim3 grid((NO + kDm2Tile - 1) / kDm2Tile, nchan);
         const size_t dm_smem = sizeof(double2) * (size_t)(kDm2Tile + 64 + 16);
         static PerDeviceFlag dm_attr;
@@ -1327,18 +1312,18 @@ int jsdr::bpsk::receive_end(jsdr_bpsk *b, const void *d_in, int fmt, int S, long
         b->dm_hist_cur ^= 1;
         if (b->stages >= 3) {
             // bit timing on the auxiliary stream: it overlaps the next block's tuner + matched filter
-            JSDR_CUDA(cudaEventRecord(b->ev_dm_ready, ctx->stream));
-            JSDR_CUDA(cudaStreamWaitEvent(ctx->aux, b->ev_dm_ready, 0));
+            JSDR_CUDA(cudaEventRecord(b->stage.ev_dm_ready, ctx->stream));
+            JSDR_CUDA(cudaStreamWaitEvent(ctx->aux, b->stage.ev_dm_ready, 0));
             TimingParams tp;
-            tp.dm = b->d_dm_buf[kb];
+            tp.dm = b->stage.d_dm_buf[kb].get();
             tp.max_ds = b->max_ds;
             tp.NO = NO;
             tp.nchan = nchan;
-            tp.bit_roll = b->d_bit_roll[kb];
-            tp.ts = b->d_ts;
-            tp.bits = b->d_bits;
-            tp.bit_at = b->d_bit_at;
-            tp.nbits = b->d_nbits;
+            tp.bit_roll = b->stage.d_bit_roll[kb].get();
+            tp.ts = b->d_ts.get();
+            tp.bits = b->stage.d_bits.get();
+            tp.bit_at = b->stage.d_bit_at.get();
+            tp.nbits = b->d_nbits.get();
             tp.max_bits = b->max_bits;
             tp.cnt_ds0 = b->cnt_ds;
             {
@@ -1359,10 +1344,10 @@ int jsdr::bpsk::receive_end(jsdr_bpsk *b, const void *d_in, int fmt, int S, long
         }
     }
     if (NO == 0)   // nothing reached the 9600 S/s stage in this call: no bits either
-        JSDR_CUDA(cudaMemsetAsync(b->d_nbits, 0, sizeof(int32_t) * nchan, ctx->aux));
-    if (b->fec && b->stages >= 3 && b->d_bits) JSDR_TRY(jsdr_fec_after_bits(b));   // :553-574, auxiliary stream
+        JSDR_CUDA(cudaMemsetAsync(b->d_nbits.get(), 0, sizeof(int32_t) * nchan, ctx->aux));
+    if (b->fec && b->stages >= 3 && b->stage.d_bits) JSDR_TRY(jsdr_fec_after_bits(b));   // :553-574, auxiliary stream
     if (b->stages >= 3 && NO > 0) {
-        JSDR_CUDA(cudaEventRecord(b->ev_bits_done[kb], ctx->aux));
+        JSDR_CUDA(cudaEventRecord(b->stage.ev_bits_done[kb], ctx->aux));
         b->bits_used[kb] = true;
     }
     b->cnt_ds += NO;
@@ -1390,51 +1375,39 @@ try {
     for (int c = 0; c < nchan; c++)
         JSDR_REQUIRE(std::isfinite(tuning_hz[c]), JSDR_EINVAL, "every tuning must be a finite frequency (the reference's comes from an int config key or the dialog, :175-195)");
     JSDR_TRY(ctx->bind());
-    jsdr_bpsk *b = new jsdr_bpsk();
-    b->ctx = ctx;
+    std::unique_ptr<jsdr_bpsk> b(new jsdr_bpsk(ctx));
     b->rate = rate;
     b->D = rate / 9600;                 // :476 adsc.rate/DOWN_SAMPLE_RATE (integer division)
     b->nchan = nchan;
     b->max_block = max_block_samples;
     b->max_ds = max_block_samples / b->D + 2;
-    b->max_words = (max_block_samples + 31) / 32 + 1;
+    b->max_words = (int)((max_block_samples + 31LL) / 32 + 1);
     b->max_bits = b->max_ds;
     b->h_tuning.assign(tuning_hz, tuning_hz + nchan);
     const size_t nc = (size_t)nchan;
-#define ALLOC(ptr, bytes)                                            \
-    do {                                                             \
-        cudaError_t e_ = cudaMalloc((void **)&(ptr), (bytes));       \
-        if (e_ != cudaSuccess) {                                     \
-            set_error("jsdr_bpsk_create: cudaMalloc(%zu): %s", (size_t)(bytes), cudaGetErrorString(e_)); \
-            jsdr_bpsk_destroy(b);                                    \
-            cudaGetLastError();                                      \
-            return JSDR_ENOMEM;                                      \
-        }                                                            \
-        cudaMemsetAsync((ptr), 0, (bytes), ctx->stream);             \
-    } while (0)
-    ALLOC(b->d_taps, sizeof(double) * kMaxDsTaps);
-    ALLOC(b->d_dmtaps, sizeof(double) * kDmTaps);
-    ALLOC(b->d_cossin, sizeof(double) * 512);
-    ALLOC(b->d_cossin2, sizeof(double2) * 257);
-    ALLOC(b->d_tu_inc, sizeof(double) * nc);
-    ALLOC(b->d_tu_par, sizeof(ScoutChan) * nc);
-    ALLOC(b->d_tu_dx, sizeof(unsigned long long) * nc);
-    ALLOC(b->d_tu_dx56, sizeof(unsigned long long) * nc);
-    ALLOC(b->d_tu_phase0, sizeof(double) * nc);
-    b->d_tu_phase = b->d_tu_phase0;
-    for (int i = 0; i < 2; i++) {
-        ALLOC(b->plan[i].ckpt, sizeof(double) * nc * b->max_words);
-        ALLOC(b->plan[i].phase_end, sizeof(double) * nc);
-        cudaEventCreateWithFlags(&b->plan[i].ready, cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&b->plan[i].consumed, cudaEventDisableTiming);
+    const char *what = "jsdr_bpsk_create";
+    cudaStream_t st = ctx->stream;
+    JSDR_TRY(b->d_taps.alloc_zeroed(sizeof(double) * kMaxDsTaps, st, what));
+    JSDR_TRY(b->d_dmtaps.alloc_zeroed(sizeof(double) * kDmTaps, st, what));
+    JSDR_TRY(b->d_cossin.alloc_zeroed(sizeof(double) * 512, st, what));
+    JSDR_TRY(b->d_cossin2.alloc_zeroed(sizeof(double2) * 257, st, what));
+    JSDR_TRY(b->d_tu_inc.alloc_zeroed(sizeof(double) * nc, st, what));
+    JSDR_TRY(b->d_tu_par.alloc_zeroed(sizeof(ScoutChan) * nc, st, what));
+    JSDR_TRY(b->d_tu_dx.alloc_zeroed(sizeof(unsigned long long) * nc, st, what));
+    JSDR_TRY(b->d_tu_dx56.alloc_zeroed(sizeof(unsigned long long) * nc, st, what));
+    JSDR_TRY(b->d_tu_phase0.alloc_zeroed(sizeof(double) * nc, st, what));
+    b->d_tu_phase = b->d_tu_phase0.get();
+    for (jsdr_bpsk::TunerPlan &P : b->plan) {
+        JSDR_TRY(P.ckpt.alloc_zeroed(sizeof(double) * nc * b->max_words, st, what));
+        JSDR_TRY(P.phase_end.alloc_zeroed(sizeof(double) * nc, st, what));
+        JSDR_TRY(P.ready.create(what));
+        JSDR_TRY(P.consumed.create(what));
     }
-    ALLOC(b->d_ds_hist[0], sizeof(double2) * kMaxDsTaps * nc);
-    ALLOC(b->d_ds_hist[1], sizeof(double2) * kMaxDsTaps * nc);
-    ALLOC(b->d_ds_out, sizeof(double2) * nc * b->max_ds);
-    ALLOC(b->d_vco_state, sizeof(double) * 4);
-    ALLOC(b->d_ts, sizeof(TimingState) * nc);
-    ALLOC(b->d_nbits, sizeof(int32_t) * (nc + 1));   // + the streaming kernel's work counter
-#undef ALLOC
+    for (int i = 0; i < 2; i++) JSDR_TRY(b->d_ds_hist[i].alloc_zeroed(sizeof(double2) * kMaxDsTaps * nc, st, what));
+    JSDR_TRY(b->d_ds_out.alloc_zeroed(sizeof(double2) * nc * b->max_ds, st, what));
+    JSDR_TRY(b->d_vco_state.alloc_zeroed(sizeof(double) * 4, st, what));
+    JSDR_TRY(b->d_ts.alloc_zeroed(sizeof(TimingState) * nc, st, what));
+    JSDR_TRY(b->d_nbits.alloc_zeroed(sizeof(int32_t) * (nc + 1), st, what));   // + the streaming kernel's work counter
     // tables and constants, computed on the host exactly as the reference's setup code does
     std::vector<double> cossin(512);
     for (int n = 0; n < 256; n++) {                       // :159-162
@@ -1461,52 +1434,23 @@ try {
     std::vector<TimingState> ts(nchan);
     memset(ts.data(), 0, sizeof(TimingState) * nc);
     for (int c = 0; c < nchan; c++) ts[c].dmEnergyOut = 1.0;                             // :499
-    int rc = upload(ctx, b->d_cossin, cossin.data(), sizeof(double) * 512);
-    if (rc == JSDR_OK) rc = upload(ctx, b->d_taps, taps.data(), sizeof(double) * kMaxDsTaps);
-    if (rc == JSDR_OK) rc = upload(ctx, b->d_dmtaps, dmt.data(), sizeof(double) * kDmTaps);
-    if (rc == JSDR_OK) rc = upload(ctx, b->d_tu_inc, inc.data(), sizeof(double) * nc);
-    if (rc == JSDR_OK) {
-        std::vector<ScoutChan> par(nchan);
-        for (int c = 0; c < nchan; c++) par[c] = scout_chan(inc[c]);
-        rc = upload(ctx, b->d_tu_par, par.data(), sizeof(ScoutChan) * nc);
-    }
-    if (rc == JSDR_OK) rc = upload(ctx, b->d_tu_dx, dx.data(), sizeof(unsigned long long) * nc);
-    if (rc == JSDR_OK) rc = upload(ctx, b->d_tu_dx56, dx56.data(), sizeof(unsigned long long) * nc);
-    if (rc == JSDR_OK) rc = upload(ctx, b->d_cossin2, cs2.data(), sizeof(double) * 2 * 257);
-    if (rc == JSDR_OK) rc = upload(ctx, b->d_ts, ts.data(), sizeof(TimingState) * nc);
-    if (rc != JSDR_OK) {
-        jsdr_bpsk_destroy(b);
-        return rc;
-    }
-    *out = b;
+    std::vector<ScoutChan> par(nchan);
+    for (int c = 0; c < nchan; c++) par[c] = scout_chan(inc[c]);
+    JSDR_TRY(upload(ctx, b->d_cossin.get(), cossin.data(), sizeof(double) * 512));
+    JSDR_TRY(upload(ctx, b->d_taps.get(), taps.data(), sizeof(double) * kMaxDsTaps));
+    JSDR_TRY(upload(ctx, b->d_dmtaps.get(), dmt.data(), sizeof(double) * kDmTaps));
+    JSDR_TRY(upload(ctx, b->d_tu_inc.get(), inc.data(), sizeof(double) * nc));
+    JSDR_TRY(upload(ctx, b->d_tu_par.get(), par.data(), sizeof(ScoutChan) * nc));
+    JSDR_TRY(upload(ctx, b->d_tu_dx.get(), dx.data(), sizeof(unsigned long long) * nc));
+    JSDR_TRY(upload(ctx, b->d_tu_dx56.get(), dx56.data(), sizeof(unsigned long long) * nc));
+    JSDR_TRY(upload(ctx, b->d_cossin2.get(), cs2.data(), sizeof(double) * 2 * 257));
+    JSDR_TRY(upload(ctx, b->d_ts.get(), ts.data(), sizeof(TimingState) * nc));
+    *out = b.release();
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
 extern "C" int jsdr_bpsk_destroy(jsdr_bpsk *b)
 try {
-    if (!b) return JSDR_OK;
-    b->ctx->bind();
-    cudaStreamSynchronize(b->ctx->side);
-    cudaStreamSynchronize(b->ctx->side2);
-    cudaStreamSynchronize(b->ctx->stream);
-    cudaStreamSynchronize(b->ctx->aux);
-    if (b->ds_read_pending) cudaStreamSynchronize(b->ctx->copy_out);   // an asynchronous read may still be draining
-    if (b->ev_dm_ready) cudaEventDestroy(b->ev_dm_ready);
-    if (b->ev_vco_ready) cudaEventDestroy(b->ev_vco_ready);
-    if (b->ev_ds_ready) cudaEventDestroy(b->ev_ds_ready);
-    if (b->ev_ds_read) cudaEventDestroy(b->ev_ds_read);
-    for (int i = 0; i < 2; i++)
-        if (b->ev_bits_done[i]) cudaEventDestroy(b->ev_bits_done[i]);
-    void *ptrs[] = {b->d_taps, b->d_dmtaps, b->d_cossin, b->d_tu_inc, b->d_tu_par, b->d_tu_phase0, b->d_tu_dx, b->d_tu_dx56, b->d_cossin2, b->plan[0].ckpt, b->plan[0].phase_end, b->plan[1].ckpt, b->plan[1].phase_end,
-                    b->d_ds_hist[0], b->d_ds_hist[1], b->d_ds_out, b->d_vco_state, b->d_vco_ix[0], b->d_vco_ix[1],
-                    b->d_bit_roll[0], b->d_bit_roll[1], b->d_dm_hist[0], b->d_dm_hist[1], b->d_dm_buf[0], b->d_dm_buf[1], b->d_ts, b->d_bits,
-                    b->d_bit_at, b->d_nbits, b->d_in, b->d_at_work[0], b->d_at_work[1], b->d_at_rev[0], b->d_at_rev[1], b->d_at_state};
-    for (void *p : ptrs) cudaFree(p);
-    jsdr_fec_destroy(b);
-    for (int i = 0; i < 2; i++) {
-        if (b->plan[i].ready) cudaEventDestroy(b->plan[i].ready);
-        if (b->plan[i].consumed) cudaEventDestroy(b->plan[i].consumed);
-    }
     delete b;
     return JSDR_OK;
 } JSDR_CATCH_ALL
@@ -1539,9 +1483,9 @@ try {
     jsdr_ctx *ctx = b->ctx;
     JSDR_TRY(ctx->bind());
     for (int c = 0; c < b->nchan; c++) centre_bin[c] = 0;
-    if (!b->d_at_state) return JSDR_OK;                // no auto-tune block yet (centreBin = 0, :405)
+    if (!b->at.d_at_state) return JSDR_OK;                // no auto-tune block yet (centreBin = 0, :405)
     std::vector<AutoTuneState> st(b->nchan);
-    JSDR_CUDA(cudaMemcpyAsync(st.data(), b->d_at_state, sizeof(AutoTuneState) * (size_t)b->nchan, cudaMemcpyDeviceToHost, ctx->stream));
+    JSDR_CUDA(cudaMemcpyAsync(st.data(), b->at.d_at_state.get(), sizeof(AutoTuneState) * (size_t)b->nchan, cudaMemcpyDeviceToHost, ctx->stream));
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     for (int c = 0; c < b->nchan; c++) centre_bin[c] = st[c].centreBin;
     return JSDR_OK;
@@ -1573,12 +1517,12 @@ try {
     b->h_tuning[chan] = hz;
     double inc = 2.0 * M_PI * hz / (double)b->rate;       // :188
     unsigned long long dx = index_step_fixed(inc);
-    JSDR_TRY(upload(b->ctx, b->d_tu_dx + chan, &dx, sizeof(dx)));
+    JSDR_TRY(upload(b->ctx, b->d_tu_dx.get() + chan, &dx, sizeof(dx)));
     unsigned long long dx56 = index_step_fixed56(inc);
-    JSDR_TRY(upload(b->ctx, b->d_tu_dx56 + chan, &dx56, sizeof(dx56)));
+    JSDR_TRY(upload(b->ctx, b->d_tu_dx56.get() + chan, &dx56, sizeof(dx56)));
     const ScoutChan sc = scout_chan(inc);
-    JSDR_TRY(upload(b->ctx, b->d_tu_par + chan, &sc, sizeof(sc)));
-    return upload(b->ctx, b->d_tu_inc + chan, &inc, sizeof(double));
+    JSDR_TRY(upload(b->ctx, b->d_tu_par.get() + chan, &sc, sizeof(sc)));
+    return upload(b->ctx, b->d_tu_inc.get() + chan, &inc, sizeof(double));
 } JSDR_CATCH_ALL
 
 extern "C" int jsdr_bpsk_set_ds_filter(jsdr_bpsk *b, const double *taps, int ntaps)
@@ -1587,7 +1531,7 @@ try {
     JSDR_TRY(b->ctx->bind());
     std::vector<double> t(kMaxDsTaps, 0.0);
     for (int i = 0; i < ntaps; i++) t[i] = taps[i];
-    JSDR_TRY(upload(b->ctx, b->d_taps, t.data(), sizeof(double) * kMaxDsTaps));
+    JSDR_TRY(upload(b->ctx, b->d_taps.get(), t.data(), sizeof(double) * kMaxDsTaps));
     for (int i = 0; i < kMaxDsTaps; i++) b->h_taps[i] = t[i];
     b->ntaps = ntaps;
     return bpsk_reset_ds(b);
@@ -1627,7 +1571,7 @@ int read_rows(jsdr_bpsk *b, const double2 *src, double *out, int mem)
 }
 }  // namespace
 
-extern "C" int jsdr_bpsk_read_ds(jsdr_bpsk *b, double *out, int mem) { return read_rows(b, b ? b->d_ds_out : nullptr, out, mem); }
+extern "C" int jsdr_bpsk_read_ds(jsdr_bpsk *b, double *out, int mem) { return read_rows(b, b ? b->d_ds_out.get() : nullptr, out, mem); }
 
 // The same rows, copied on the download stream behind the decimator and without waiting: the
 // copy overlaps whatever the caller submits next (the upload of the following block, in the
@@ -1638,14 +1582,17 @@ try {
     JSDR_REQUIRE(mem == JSDR_MEM_HOST || mem == JSDR_MEM_DEVICE, JSDR_EINVAL, "bad mem");
     jsdr_ctx *ctx = b->ctx;
     JSDR_TRY(ctx->bind());
-    if (!b->ev_ds_ready) {
-        JSDR_CUDA(cudaEventCreateWithFlags(&b->ev_ds_ready, cudaEventDisableTiming));
-        JSDR_CUDA(cudaEventCreateWithFlags(&b->ev_ds_read, cudaEventDisableTiming));
+    if (!b->ev_ds_read) {
+        Event ready, read;
+        JSDR_TRY(ready.create("jsdr_bpsk_read_ds_async"));
+        JSDR_TRY(read.create("jsdr_bpsk_read_ds_async"));
+        b->ev_ds_ready = std::move(ready);
+        b->ev_ds_read = std::move(read);
     }
     if (b->last_nds == 0) return JSDR_OK;
     JSDR_CUDA(cudaEventRecord(b->ev_ds_ready, ctx->stream));
     JSDR_CUDA(cudaStreamWaitEvent(ctx->copy_out, b->ev_ds_ready, 0));
-    JSDR_CUDA(cudaMemcpy2DAsync(out, sizeof(double2) * b->last_nds, b->d_ds_out, sizeof(double2) * b->max_ds,
+    JSDR_CUDA(cudaMemcpy2DAsync(out, sizeof(double2) * b->last_nds, b->d_ds_out.get(), sizeof(double2) * b->max_ds,
                                 sizeof(double2) * b->last_nds, b->nchan,
                                 mem == JSDR_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice,
                                 ctx->copy_out));
@@ -1664,18 +1611,18 @@ extern "C" int jsdr_bpsk_read_bits(jsdr_bpsk *b, int8_t *bits, int64_t *bit_at, 
                                    int max_bits, int mem)
 try {
     JSDR_REQUIRE(b && nbits, JSDR_EINVAL, "null argument");
-    JSDR_REQUIRE(b->stages >= 3 && b->d_bits, JSDR_ESTATE, "bit decision stage is disabled or has not run");
+    JSDR_REQUIRE(b->stages >= 3 && b->stage.d_bits, JSDR_ESTATE, "bit decision stage is disabled or has not run");
     JSDR_REQUIRE(max_bits >= 0, JSDR_EINVAL, "negative max_bits");
     jsdr_ctx *ctx = b->ctx;
     JSDR_TRY(ctx->bind());
     const cudaMemcpyKind kind = mem == JSDR_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
-    JSDR_CUDA(cudaMemcpyAsync(nbits, b->d_nbits, sizeof(int32_t) * b->nchan, kind, ctx->aux));
+    JSDR_CUDA(cudaMemcpyAsync(nbits, b->d_nbits.get(), sizeof(int32_t) * b->nchan, kind, ctx->aux));
     const int w = max_bits < b->max_bits ? max_bits : b->max_bits;
     if (bits && w > 0)
-        JSDR_CUDA(cudaMemcpy2DAsync(bits, (size_t)max_bits, b->d_bits, (size_t)b->max_bits, (size_t)w,
+        JSDR_CUDA(cudaMemcpy2DAsync(bits, (size_t)max_bits, b->stage.d_bits.get(), (size_t)b->max_bits, (size_t)w,
                                     b->nchan, kind, ctx->aux));
     if (bit_at && w > 0)
-        JSDR_CUDA(cudaMemcpy2DAsync(bit_at, sizeof(int64_t) * max_bits, b->d_bit_at,
+        JSDR_CUDA(cudaMemcpy2DAsync(bit_at, sizeof(int64_t) * max_bits, b->stage.d_bit_at.get(),
                                     sizeof(long long) * b->max_bits, sizeof(int64_t) * w, b->nchan, kind,
                                     ctx->aux));
     if (mem == JSDR_MEM_HOST) JSDR_CUDA(cudaStreamSynchronize(ctx->aux));
@@ -1688,7 +1635,7 @@ try {
     jsdr_ctx *ctx = b->ctx;
     JSDR_TRY(ctx->bind());
     std::vector<TimingState> ts(b->nchan);
-    JSDR_CUDA(cudaMemcpyAsync(ts.data(), b->d_ts, sizeof(TimingState) * (size_t)b->nchan,
+    JSDR_CUDA(cudaMemcpyAsync(ts.data(), b->d_ts.get(), sizeof(TimingState) * (size_t)b->nchan,
                               cudaMemcpyDeviceToHost, ctx->aux));
     JSDR_CUDA(cudaStreamSynchronize(ctx->aux));
     for (int c = 0; c < b->nchan; c++) {
@@ -1703,7 +1650,7 @@ try {
 extern "C" int jsdr_bpsk_ds_device_ptr(jsdr_bpsk *b, double **dev_ptr)
 try {
     JSDR_REQUIRE(b && dev_ptr, JSDR_EINVAL, "null argument");
-    *dev_ptr = reinterpret_cast<double *>(b->d_ds_out);
+    *dev_ptr = reinterpret_cast<double *>(b->d_ds_out.get());
     return JSDR_OK;
 } JSDR_CATCH_ALL
 

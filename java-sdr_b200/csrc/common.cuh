@@ -10,6 +10,7 @@
 #include <mutex>
 #include <new>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/jsdrcuda.h"
@@ -63,26 +64,124 @@ void set_error(const char *fmt, ...);
         return JSDR_EINTERNAL;                                                       \
     }
 
+// api.cu.  Report a failed CUDA call `call` made for `what` and clear it (as JSDR_CUDA does):
+// JSDR_ENOMEM for cudaErrorMemoryAllocation, JSDR_ECUDA for everything else.
+int cuda_failed(cudaError_t e, const char *what, const char *call);
+
+// ---- owners of device memory, events and streams ------------------------------------------
+// Move-only; the destructor releases what the owner holds.  Acquiring returns a JSDR status and
+// reports a failure through cuda_failed, naming `what`.  Every buffer, event and stream a handle
+// keeps is one of these, so that a destroy and a failed create release through the same path.
+
+// Device memory with its capacity.
+template <class T>
+class DevBuf {
+public:
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p_(o.p_), cap_(o.cap_) { o.p_ = nullptr, o.cap_ = 0; }
+    DevBuf &operator=(DevBuf &&o) noexcept   // what this held is released with `o`
+    {
+        std::swap(p_, o.p_);
+        std::swap(cap_, o.cap_);
+        return *this;
+    }
+    ~DevBuf() { reset(); }
+    T *get() const { return p_; }
+    explicit operator bool() const { return p_ != nullptr; }
+    void reset()
+    {
+        if (p_) cudaFree(p_);
+        p_ = nullptr, cap_ = 0;
+    }
+    // `bytes` of new memory; what was held is freed first
+    int alloc(size_t bytes, const char *what)
+    {
+        reset();
+        void *p = nullptr;
+        const cudaError_t e = cudaMalloc(&p, bytes);
+        if (e != cudaSuccess) return cuda_failed(e, what, "cudaMalloc");
+        p_ = static_cast<T *>(p), cap_ = bytes;
+        return JSDR_OK;
+    }
+    // grow on demand: reallocated (contents lost) only when it holds fewer than `bytes`
+    int grow(size_t bytes, const char *what) { return cap_ >= bytes ? JSDR_OK : alloc(bytes, what); }
+    // the same, cleared to zeros on `st`
+    int alloc_zeroed(size_t bytes, cudaStream_t st, const char *what)
+    {
+        JSDR_TRY(alloc(bytes, what));
+        const cudaError_t e = cudaMemsetAsync(p_, 0, bytes, st);
+        return e == cudaSuccess ? JSDR_OK : cuda_failed(e, what, "cudaMemsetAsync");
+    }
+
+private:
+    T *p_ = nullptr;
+    size_t cap_ = 0;
+};
+
+inline void release(cudaEvent_t e) { cudaEventDestroy(e); }
+inline void release(cudaStream_t s) { cudaStreamDestroy(s); }
+
+// An event or a stream: converts to the runtime's handle, which it keeps owning.
+template <class H>
+class Owned {
+public:
+    Owned() = default;
+    Owned(Owned &&o) noexcept : h_(o.h_) { o.h_ = nullptr; }
+    Owned &operator=(Owned &&o) noexcept   // what this held is released with `o`
+    {
+        std::swap(h_, o.h_);
+        return *this;
+    }
+    ~Owned() { reset(); }
+    operator H() const { return h_; }
+    void reset()
+    {
+        if (h_) release(h_);
+        h_ = nullptr;
+    }
+
+protected:
+    H h_ = nullptr;
+};
+
+struct Event : Owned<cudaEvent_t> {
+    int create(const char *what, unsigned flags = cudaEventDisableTiming)
+    {
+        reset();
+        const cudaError_t e = cudaEventCreateWithFlags(&h_, flags);
+        return e == cudaSuccess ? JSDR_OK : (h_ = nullptr, cuda_failed(e, what, "cudaEventCreateWithFlags"));
+    }
+};
+
+struct Stream : Owned<cudaStream_t> {
+    int create(int priority, const char *what)   // non-blocking; priority 0 is the runtime's default
+    {
+        reset();
+        const cudaError_t e = cudaStreamCreateWithPriority(&h_, cudaStreamNonBlocking, priority);
+        return e == cudaSuccess ? JSDR_OK : (h_ = nullptr, cuda_failed(e, what, "cudaStreamCreateWithPriority"));
+    }
+};
+
 }  // namespace jsdr
 
 struct jsdr_prof_span {
     int kind;
-    cudaEvent_t a, b;
+    jsdr::Event a, b;
 };
 
 struct jsdr_ctx {
     int device = 0;
     int sm_count = 0;
     int l2_prefetch = 1;             // FFT: bulk-prefetch the input of the CTA n x (resident CTAs) ahead into L2 (JSDR_L2_PREFETCH=n, 0: off)
-    cudaStream_t stream = nullptr;   // main stream: data kernels
-    cudaStream_t side = nullptr;     // side stream: data-independent phase scouts
-    cudaStream_t side2 = nullptr;    // the VCO / bit-phase replay: one short serial chain, beside the tuner scout
-    cudaStream_t aux = nullptr;      // low priority: work that runs beside the main stream's kernel
-    cudaEvent_t ev_aux_fork = nullptr, ev_aux_join = nullptr;
-    cudaStream_t copy_in = nullptr, copy_out = nullptr;   // host<->device copies of the chunked host path
-    cudaEvent_t ev_chunk_in[16] = {nullptr}, ev_chunk_done[16] = {nullptr};
-    cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+    jsdr::Stream stream;             // main stream: data kernels
+    jsdr::Stream side;               // side stream: data-independent phase scouts
+    jsdr::Stream side2;              // the VCO / bit-phase replay: one short serial chain, beside the tuner scout
+    jsdr::Stream aux;                // low priority: work that runs beside the main stream's kernel
+    jsdr::Stream copy_in, copy_out;  // host<->device copies of the chunked host path
+    jsdr::Event ev_aux_fork, ev_aux_join;
+    jsdr::Event ev_chunk_in[16], ev_chunk_done[16];
+    jsdr::Event ev_t0, ev_t1;
+    jsdr::Event ev_fork, ev_join;
     int64_t launches = 0;
     // per-kernel timing: event pairs recorded around the launches while `profiling` is on
     bool profiling = false;
@@ -90,6 +189,14 @@ struct jsdr_ctx {
     std::vector<jsdr_prof_span> free_spans;  // event pairs ready for reuse
 
     int bind() const { return cudaSetDevice(device) == cudaSuccess ? JSDR_OK : JSDR_ECUDA; }
+    // the events above may still be pending on any stream; the owners release them after this
+    ~jsdr_ctx()
+    {
+        bind();
+        const cudaStream_t all[] = {stream, side, side2, aux, copy_in, copy_out};
+        for (cudaStream_t s : all)
+            if (s) cudaStreamSynchronize(s);
+    }
 };
 
 namespace jsdr {
@@ -124,9 +231,6 @@ struct PerDeviceFlag {
 
 // api.cu.  Copy host -> device on the context's main stream and wait for it.
 int upload(jsdr_ctx *ctx, void *dst, const void *src, size_t bytes);
-// Grow-on-demand device buffer: *p holds *cap bytes; if fewer than `bytes`, it is freed and
-// reallocated (contents lost).
-int grow(void **p, size_t *cap, size_t bytes);
 
 // Check the launch that was just made and count it.
 static inline int launched(jsdr_ctx *ctx, const char *what)
@@ -154,11 +258,11 @@ struct ProfScope {
     {
         if (!on) return;
         if (!c->free_spans.empty()) {
-            sp = c->free_spans.back();
+            sp = std::move(c->free_spans.back());
             c->free_spans.pop_back();
-        } else if (cudaEventCreate(&sp.a) != cudaSuccess || cudaEventCreate(&sp.b) != cudaSuccess) {
-            cudaGetLastError();
-            on = false;
+        } else if (sp.a.create("profiling", cudaEventDefault) != JSDR_OK ||
+                   sp.b.create("profiling", cudaEventDefault) != JSDR_OK) {
+            on = false;   // this launch is not timed
             return;
         }
         sp.kind = kind;
@@ -168,7 +272,7 @@ struct ProfScope {
     {
         if (!on) return;
         cudaEventRecord(sp.b, st);
-        ctx->spans.push_back(sp);
+        ctx->spans.push_back(std::move(sp));
     }
 };
 

@@ -367,55 +367,31 @@ try {
     JSDR_REQUIRE(rate > 0 && nchan > 0 && max_block_samples > 0, JSDR_EINVAL, "sizes must be positive");
     JSDR_REQUIRE(nchan <= 65535, JSDR_EINVAL, "at most 65535 channels per handle (the channel is the grid's y index)");
     JSDR_TRY(ctx->bind());
-    jsdr_demod *d = new jsdr_demod();
-    d->ctx = ctx;
+    std::unique_ptr<jsdr_demod> d(new jsdr_demod(ctx));
     d->rate = rate;
     d->nchan = nchan;
     d->max_block = max_block_samples;
-    d->max_chunks = (max_block_samples + kChunk - 1) / kChunk + 1;
+    d->max_chunks = (int)((max_block_samples + kChunk - 1LL) / kChunk + 1);
     d->h_w.assign((size_t)nchan * kTaps, 0.0f);       // taps are zero until weights() runs (SURVEY Q5)
     d->h_phi.assign(nchan, 0.0f);
     const size_t nc = (size_t)nchan;
-    cudaError_t e = cudaSuccess;
-    if (e == cudaSuccess) e = cudaMalloc(&d->d_w, sizeof(float) * kTaps * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&d->d_phi, sizeof(float) * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&d->d_car, sizeof(float) * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&d->d_chunk_car, sizeof(float) * nc * d->max_chunks);
-    if (e == cudaSuccess) e = cudaMalloc(&d->d_hist[0], sizeof(float2) * kHist * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&d->d_hist[1], sizeof(float2) * kHist * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&d->d_lilq, sizeof(float2) * 2 * nc);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&d->ev_car_ready, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&d->ev_audio_ready, cudaEventDisableTiming);
-    if (e != cudaSuccess) {
-        set_error("jsdr_demod_create: %s", cudaGetErrorString(e));
-        jsdr_demod_destroy(d);
-        cudaGetLastError();
-        return JSDR_ENOMEM;
-    }
-    cudaMemsetAsync(d->d_w, 0, sizeof(float) * kTaps * nc, ctx->stream);
-    cudaMemsetAsync(d->d_phi, 0, sizeof(float) * nc, ctx->stream);
-    cudaMemsetAsync(d->d_car, 0, sizeof(float) * nc, ctx->stream);
-    cudaMemsetAsync(d->d_hist[0], 0, sizeof(float2) * kHist * nc, ctx->stream);
-    cudaMemsetAsync(d->d_hist[1], 0, sizeof(float2) * kHist * nc, ctx->stream);
-    cudaMemsetAsync(d->d_lilq, 0, sizeof(float2) * 2 * nc, ctx->stream);
-    JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
-    *out = d;
+    const char *what = "jsdr_demod_create";
+    cudaStream_t st = ctx->stream;
+    JSDR_TRY(d->d_w.alloc_zeroed(sizeof(float) * kTaps * nc, st, what));
+    JSDR_TRY(d->d_phi.alloc_zeroed(sizeof(float) * nc, st, what));
+    JSDR_TRY(d->d_car.alloc_zeroed(sizeof(float) * nc, st, what));
+    JSDR_TRY(d->d_chunk_car.alloc(sizeof(float) * nc * d->max_chunks, what));
+    for (int i = 0; i < 2; i++) JSDR_TRY(d->d_hist[i].alloc_zeroed(sizeof(float2) * kHist * nc, st, what));
+    JSDR_TRY(d->d_lilq.alloc_zeroed(sizeof(float2) * 2 * nc, st, what));
+    JSDR_TRY(d->ev_car_ready.create(what));
+    JSDR_TRY(d->ev_audio_ready.create(what));
+    JSDR_CUDA(cudaStreamSynchronize(st));
+    *out = d.release();
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
 extern "C" int jsdr_demod_destroy(jsdr_demod *d)
 try {
-    if (!d) return JSDR_OK;
-    d->ctx->bind();
-    cudaStreamSynchronize(d->ctx->side);
-    cudaStreamSynchronize(d->ctx->side2);
-    cudaStreamSynchronize(d->ctx->copy_out);
-    cudaStreamSynchronize(d->ctx->stream);
-    void *ptrs[] = {d->d_w, d->d_phi, d->d_car, d->d_chunk_car, d->d_hist[0], d->d_hist[1], d->d_in, d->d_out,
-                    d->d_lilq, d->d_det, d->d_audio};
-    for (void *p : ptrs) cudaFree(p);
-    if (d->ev_car_ready) cudaEventDestroy(d->ev_car_ready);
-    if (d->ev_audio_ready) cudaEventDestroy(d->ev_audio_ready);
     delete d;
     return JSDR_OK;
 } JSDR_CATCH_ALL
@@ -446,13 +422,13 @@ try {
         }
         d->h_phi[chan] = (float)(2 * M_PI * nlo);       // :368
         const float zero = 0.0f;
-        JSDR_TRY(upload(ctx, d->d_phi + chan, &d->h_phi[chan], sizeof(float)));
-        JSDR_TRY(upload(ctx, d->d_car + chan, &zero, sizeof(float)));   // :369
+        JSDR_TRY(upload(ctx, d->d_phi.get() + chan, &d->h_phi[chan], sizeof(float)));
+        JSDR_TRY(upload(ctx, d->d_car.get() + chan, &zero, sizeof(float)));   // :369
     }
-    JSDR_TRY(upload(ctx, d->d_w + (size_t)chan * kTaps, w, sizeof(float) * kTaps));
+    JSDR_TRY(upload(ctx, d->d_w.get() + (size_t)chan * kTaps, w, sizeof(float) * kTaps));
     // :372-374 clear the delay line
     for (int i = 0; i < 2; i++)
-        JSDR_CUDA(cudaMemsetAsync(d->d_hist[i] + (size_t)chan * kHist, 0, sizeof(float2) * kHist, ctx->stream));
+        JSDR_CUDA(cudaMemsetAsync(d->d_hist[i].get() + (size_t)chan * kHist, 0, sizeof(float2) * kHist, ctx->stream));
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     return JSDR_OK;
 } JSDR_CATCH_ALL
@@ -482,7 +458,7 @@ int demod_car_fork(jsdr_demod *d, int S, cudaEvent_t fork, cudaStream_t side, cu
     jsdr_ctx *ctx = d->ctx;
     JSDR_CUDA(cudaEventRecord(fork, ctx->stream));
     JSDR_CUDA(cudaStreamWaitEvent(side, fork, 0));
-    k_car_scout<<<(d->nchan + 127) / 128, 128, 0, side>>>(d->d_phi, d->d_car, d->d_chunk_car, d->nchan, S);
+    k_car_scout<<<(d->nchan + 127) / 128, 128, 0, side>>>(d->d_phi.get(), d->d_car.get(), d->d_chunk_car.get(), d->nchan, S);
     JSDR_TRY(launched(ctx, "k_car_scout"));
     JSDR_CUDA(cudaEventRecord(join, side));
     return JSDR_OK;
@@ -501,11 +477,11 @@ int demod_launch(jsdr_demod *d, const void *d_in, bool s16, int S, int64_t chan_
     p.chan_stride = chan_stride;
     p.S = S;
     p.nchan = nchan;
-    p.w = d->d_w;
-    p.phi = d->d_phi;
-    p.chunk_car = d->d_chunk_car;
-    p.hist_in = d->d_hist[d->hist_cur];
-    p.hist_out = d->d_hist[d->hist_cur ^ 1];
+    p.w = d->d_w.get();
+    p.phi = d->d_phi.get();
+    p.chunk_car = d->d_chunk_car.get();
+    p.hist_in = d->d_hist[d->hist_cur].get();
+    p.hist_out = d->d_hist[d->hist_cur ^ 1].get();
     p.out = d_out;
     p.dofir = d->dofir;
     p.dodwn = d->dodwn;
@@ -542,13 +518,13 @@ int demod_run(jsdr_demod *d, const void *in, bool s16, int S, int64_t chan_strid
     if (mem == JSDR_MEM_HOST) {
         const size_t esz = s16 ? 4 : 8;
         const size_t total = (chan_stride == 0) ? (size_t)S : (size_t)chan_stride * (nchan - 1) + S;
-        JSDR_TRY(grow(&d->d_in, &d->in_cap, total * esz));
-        JSDR_CUDA(cudaMemcpyAsync(d->d_in, in, total * esz, cudaMemcpyHostToDevice, ctx->stream));
-        d_in = d->d_in;
+        JSDR_TRY(d->d_in.grow(total * esz, "demod staging"));
+        JSDR_CUDA(cudaMemcpyAsync(d->d_in.get(), in, total * esz, cudaMemcpyHostToDevice, ctx->stream));
+        d_in = d->d_in.get();
     }
     if (mem == JSDR_MEM_HOST || !out) {
-        JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_out), &d->out_cap, out_bytes));
-        d_out = reinterpret_cast<float2 *>(d->d_out);
+        JSDR_TRY(d->d_out.grow(out_bytes, "demod staging"));
+        d_out = d->d_out.get();
     }
     JSDR_TRY(demod_launch(d, d_in, s16, S, chan_stride, ic, qc, d_out, ctx->ev_join));
     *d_result = d_out;
@@ -784,21 +760,21 @@ int detect_launch(jsdr_demod *d, const float2 *res, int Srow, int L, int16_t *au
 {
     jsdr_ctx *ctx = d->ctx;
     const int nchan = d->nchan, nblk = (Srow + L - 1) / L;
-    JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_det), &d->det_cap, (size_t)nchan * Srow * sizeof(float)));
+    JSDR_TRY(d->d_det.grow((size_t)nchan * Srow * sizeof(float), "demod detector"));
     // :409 fmgain = ad.rate / (MODE_NFM==mode ? 5000f : 75000f), int / float in float
     const float fmgain = (float)d->rate / (d->mode == dsp::MODE_NFM ? 5000.0f : 75000.0f);
     // One block per row: the CTA reads li/lq before it writes them.  Several: block 0 of a row may
     // still read the carried li/lq while the last block writes its own, so that one goes to the
     // second half of d_lilq and is copied back behind the kernel.
-    float2 *lilq_out = nblk > 1 ? d->d_lilq + nchan : d->d_lilq;
+    float2 *lilq = d->d_lilq.get(), *lilq_out = nblk > 1 ? lilq + nchan : lilq;
     {
         ProfScope prof(ctx, JSDR_K_DETECT, ctx->stream);
-        dsp::k_detect<<<(unsigned)nchan * nblk, 256, 0, ctx->stream>>>(res, Srow, L, d->mode, fmgain, d->doagc, d->d_lilq,
-                                                                        lilq_out, d->d_det, audio, max_avg);
+        dsp::k_detect<<<(unsigned)nchan * nblk, 256, 0, ctx->stream>>>(res, Srow, L, d->mode, fmgain, d->doagc, lilq,
+                                                                        lilq_out, d->d_det.get(), audio, max_avg);
     }
     JSDR_TRY(launched(ctx, "k_detect"));
     if (nblk > 1 && (d->mode == dsp::MODE_NFM || d->mode == dsp::MODE_WFM))
-        JSDR_CUDA(cudaMemcpyAsync(d->d_lilq, lilq_out, sizeof(float2) * nchan, cudaMemcpyDeviceToDevice, ctx->stream));
+        JSDR_CUDA(cudaMemcpyAsync(lilq, lilq_out, sizeof(float2) * nchan, cudaMemcpyDeviceToDevice, ctx->stream));
     return JSDR_OK;
 }
 
@@ -806,9 +782,9 @@ int detect_launch(jsdr_demod *d, const float2 *res, int Srow, int L, int16_t *au
 int audio_staging(jsdr_demod *d, size_t nsamp, size_t npairs, int16_t **d_audio, float **d_ma)
 {
     const size_t ma_off = (nsamp * sizeof(int16_t) + 15) & ~(size_t)15;
-    JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_audio), &d->audio_cap, ma_off + sizeof(float) * 2 * npairs));
-    *d_audio = d->d_audio;
-    *d_ma = reinterpret_cast<float *>(reinterpret_cast<char *>(d->d_audio) + ma_off);
+    JSDR_TRY(d->d_audio.grow(ma_off + sizeof(float) * 2 * npairs, "demod staging"));
+    *d_audio = d->d_audio.get();
+    *d_ma = reinterpret_cast<float *>(reinterpret_cast<char *>(d->d_audio.get()) + ma_off);
     return JSDR_OK;
 }
 
@@ -875,8 +851,8 @@ int jsdr_pump_demod_staging(jsdr_demod *d, int S, int nblocks, int16_t **d_audio
 int jsdr_pump_demod_run(jsdr_demod *d, const int16_t *d_raw, int S, int L, int ic, int qc, int16_t *audio,
                         float *max_avg)
 {
-    JSDR_TRY(grow(reinterpret_cast<void **>(&d->d_out), &d->out_cap, sizeof(float2) * (size_t)d->nchan * S));
-    float2 *mixed = reinterpret_cast<float2 *>(d->d_out);
+    JSDR_TRY(d->d_out.grow(sizeof(float2) * (size_t)d->nchan * S, "demod staging"));
+    float2 *mixed = d->d_out.get();
     JSDR_TRY(demod_launch(d, d_raw, true, S, S, ic, qc, mixed, d->ev_car_ready));
     return detect_launch(d, mixed, S, L, audio, max_avg);
 }
@@ -925,35 +901,19 @@ try {
     JSDR_REQUIRE(nchan > 0 && max_block_samples > 0, JSDR_EINVAL, "sizes must be positive");
     JSDR_REQUIRE(nchan <= 65535, JSDR_EINVAL, "at most 65535 channels per handle (the channel is the grid's y index)");
     JSDR_TRY(ctx->bind());
-    jsdr_fir *f = new jsdr_fir();
-    f->ctx = ctx;
+    std::unique_ptr<jsdr_fir> f(new jsdr_fir(ctx));
     f->nchan = nchan;
     f->max_block = max_block_samples;
     const size_t nc = (size_t)nchan;
-    cudaError_t e = cudaMalloc(&f->d_w, sizeof(double) * kTaps * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_hist[0], sizeof(int32_t) * kHist * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_hist[1], sizeof(int32_t) * kHist * nc);
-    if (e != cudaSuccess) {
-        set_error("jsdr_fir_create: %s", cudaGetErrorString(e));
-        jsdr_fir_destroy(f);
-        cudaGetLastError();
-        return JSDR_ENOMEM;
-    }
-    cudaMemsetAsync(f->d_w, 0, sizeof(double) * kTaps * nc, ctx->stream);
-    cudaMemsetAsync(f->d_hist[0], 0, sizeof(int32_t) * kHist * nc, ctx->stream);
-    cudaMemsetAsync(f->d_hist[1], 0, sizeof(int32_t) * kHist * nc, ctx->stream);
+    JSDR_TRY(f->d_w.alloc_zeroed(sizeof(double) * kTaps * nc, ctx->stream, "jsdr_fir_create"));
+    for (int i = 0; i < 2; i++) JSDR_TRY(f->d_hist[i].alloc_zeroed(sizeof(int32_t) * kHist * nc, ctx->stream, "jsdr_fir_create"));
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
-    *out = f;
+    *out = f.release();
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
 extern "C" int jsdr_fir_destroy(jsdr_fir *f)
 try {
-    if (!f) return JSDR_OK;
-    f->ctx->bind();
-    cudaStreamSynchronize(f->ctx->stream);
-    void *ptrs[] = {f->d_w, f->d_hist[0], f->d_hist[1], f->d_in, f->d_out};
-    for (void *p : ptrs) cudaFree(p);
     delete f;
     return JSDR_OK;
 } JSDR_CATCH_ALL
@@ -963,9 +923,9 @@ try {
     JSDR_REQUIRE(f && w && chan >= 0 && chan < f->nchan, JSDR_EINVAL, "bad channel");
     jsdr_ctx *ctx = f->ctx;
     JSDR_TRY(ctx->bind());
-    JSDR_TRY(upload(ctx, f->d_w + (size_t)chan * kTaps, w, sizeof(double) * kTaps));
+    JSDR_TRY(upload(ctx, f->d_w.get() + (size_t)chan * kTaps, w, sizeof(double) * kTaps));
     for (int i = 0; i < 2; i++)                          // :192-193 clear previous samples
-        JSDR_CUDA(cudaMemsetAsync(f->d_hist[i] + (size_t)chan * kHist, 0, sizeof(int32_t) * kHist, ctx->stream));
+        JSDR_CUDA(cudaMemsetAsync(f->d_hist[i].get() + (size_t)chan * kHist, 0, sizeof(int32_t) * kHist, ctx->stream));
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     return JSDR_OK;
 } JSDR_CATCH_ALL
@@ -986,19 +946,19 @@ try {
     const size_t out_bytes = sizeof(int32_t) * (size_t)nchan * S;
     if (mem == JSDR_MEM_HOST) {
         const size_t total = (chan_stride == 0) ? (size_t)S : (size_t)chan_stride * (nchan - 1) + S;
-        JSDR_TRY(grow(reinterpret_cast<void **>(&f->d_in), &f->in_cap, total * sizeof(int32_t)));
-        JSDR_TRY(grow(reinterpret_cast<void **>(&f->d_out), &f->out_cap, out_bytes));
-        JSDR_CUDA(cudaMemcpyAsync(f->d_in, in, total * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-        d_in = f->d_in;
-        d_out = f->d_out;
+        JSDR_TRY(f->d_in.grow(total * sizeof(int32_t), "fir staging"));
+        JSDR_TRY(f->d_out.grow(out_bytes, "fir staging"));
+        JSDR_CUDA(cudaMemcpyAsync(f->d_in.get(), in, total * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+        d_in = f->d_in.get();
+        d_out = f->d_out.get();
     }
     FirParams p;
     p.in = d_in;
     p.chan_stride = chan_stride;
     p.S = S;
-    p.w = f->d_w;
-    p.hist_in = f->d_hist[f->hist_cur];
-    p.hist_out = f->d_hist[f->hist_cur ^ 1];
+    p.w = f->d_w.get();
+    p.hist_in = f->d_hist[f->hist_cur].get();
+    p.hist_out = f->d_hist[f->hist_cur ^ 1].get();
     p.out = d_out;
     dim3 grid((S + kThreads * kFirOut - 1) / (kThreads * kFirOut), nchan);
     {
@@ -1010,7 +970,7 @@ try {
     JSDR_TRY(launched(ctx, "k_fir_tail"));
     f->hist_cur ^= 1;
     if (mem == JSDR_MEM_HOST) {
-        JSDR_CUDA(cudaMemcpyAsync(out, f->d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        JSDR_CUDA(cudaMemcpyAsync(out, f->d_out.get(), out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
         JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     }
     return JSDR_OK;
@@ -1026,10 +986,10 @@ try {
     const size_t bytes = sizeof(int2) * (size_t)npairs;
     const int2 *da = reinterpret_cast<const int2 *>(a), *db = reinterpret_cast<const int2 *>(b);
     int2 *dout = reinterpret_cast<int2 *>(out);
-    void *tmp = nullptr;
+    DevBuf<int2> tmp;
     if (mem == JSDR_MEM_HOST) {
-        JSDR_CUDA(cudaMalloc(&tmp, 3 * bytes));
-        int2 *t = static_cast<int2 *>(tmp);
+        JSDR_TRY(tmp.alloc(3 * bytes, "jsdr_fir_complex_mod_i32"));
+        int2 *t = tmp.get();
         JSDR_CUDA(cudaMemcpyAsync(t, a, bytes, cudaMemcpyHostToDevice, ctx->stream));
         JSDR_CUDA(cudaMemcpyAsync(t + npairs, b, bytes, cudaMemcpyHostToDevice, ctx->stream));
         da = t;
@@ -1043,7 +1003,6 @@ try {
     if (mem == JSDR_MEM_HOST) {
         JSDR_CUDA(cudaMemcpyAsync(out, dout, bytes, cudaMemcpyDeviceToHost, ctx->stream));
         JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
-        cudaFree(tmp);
     }
     return JSDR_OK;
 } JSDR_CATCH_ALL
@@ -1098,30 +1057,20 @@ try {
     JSDR_TRY(ctx->bind());
     const float *d_psd = psd;
     int32_t *d_pix = pixels;
-    void *tmp_in = nullptr, *tmp_out = nullptr;
+    DevBuf<float> tmp_in;
+    DevBuf<int32_t> tmp_out;
     const size_t in_bytes = sizeof(float) * (size_t)rows * (n + 2), out_bytes = sizeof(int32_t) * (size_t)rows * width;
     if (mem == JSDR_MEM_HOST) {
-        JSDR_CUDA(cudaMalloc(&tmp_in, in_bytes));
-        cudaError_t e = cudaMalloc(&tmp_out, out_bytes);
-        if (e != cudaSuccess) {
-            cudaFree(tmp_in);
-            set_error("jsdr_waterfall_rows: cudaMalloc: %s", cudaGetErrorString(e));
-            return JSDR_ENOMEM;
-        }
-        cudaMemcpyAsync(tmp_in, psd, in_bytes, cudaMemcpyHostToDevice, ctx->stream);
-        d_psd = static_cast<const float *>(tmp_in);
-        d_pix = static_cast<int32_t *>(tmp_out);
+        JSDR_TRY(tmp_in.alloc(in_bytes, "jsdr_waterfall_rows"));
+        JSDR_TRY(tmp_out.alloc(out_bytes, "jsdr_waterfall_rows"));
+        JSDR_CUDA(cudaMemcpyAsync(tmp_in.get(), psd, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        d_psd = tmp_in.get();
+        d_pix = tmp_out.get();
     }
-    int rc = jsdr_launch_waterfall(ctx, d_psd, n, rows, width, peak_rgb, d_pix, ctx->stream);
+    JSDR_TRY(jsdr_launch_waterfall(ctx, d_psd, n, rows, width, peak_rgb, d_pix, ctx->stream));
     if (mem == JSDR_MEM_HOST) {
-        if (rc == JSDR_OK) cudaMemcpyAsync(pixels, d_pix, out_bytes, cudaMemcpyDeviceToHost, ctx->stream);
-        cudaError_t e = cudaStreamSynchronize(ctx->stream);
-        cudaFree(tmp_in);
-        cudaFree(tmp_out);
-        if (rc == JSDR_OK && e != cudaSuccess) {
-            set_error("jsdr_waterfall_rows: %s", cudaGetErrorString(e));
-            rc = JSDR_ECUDA;
-        }
+        JSDR_CUDA(cudaMemcpyAsync(pixels, d_pix, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     }
-    return rc;
+    return JSDR_OK;
 } JSDR_CATCH_ALL

@@ -464,15 +464,17 @@ using namespace jsdr;
 
 struct jsdr_fec_state {
     int max_frames = 0;                       // frame slots on the device (>= what the caller asked for)
-    int16_t *d_mettab = nullptr;              // [2][256], this bank's copy of the caller's metric table
-    int8_t *d_hist[2] = {nullptr, nullptr};   // [nchan][5199]
+    DevBuf<int16_t> d_mettab;                 // [2][256], this bank's copy of the caller's metric table
+    DevBuf<int8_t> d_hist[2];                 // [nchan][5199]
     int cur = 0;
-    fec::FrameMeta *d_frames = nullptr;
-    int *d_nframes = nullptr;
+    DevBuf<fec::FrameMeta> d_frames;
+    DevBuf<int> d_nframes;
     const uint8_t *d_rs_par = nullptr;        // [128][32] parity map (per device, shared)
-    uint8_t *d_data = nullptr;                // [max_frames][256]
-    long long *d_cnt = nullptr;               // [2][nchan] cntFEC, cntDec (:567,571)
+    DevBuf<uint8_t> d_data;                   // [max_frames][256]
+    DevBuf<long long> d_cnt;                  // [2][nchan] cntFEC, cntDec (:567,571)
 };
+
+void jsdr_fec_delete::operator()(jsdr_fec_state *f) const { delete f; }
 
 extern "C" int jsdr_bpsk_enable_fec(jsdr_bpsk *b, const int16_t *mettab, int max_frames)
 try {
@@ -494,11 +496,12 @@ try {
         return JSDR_OK;
     }));
     if (b->fec) {                                               // metric table refreshed, state kept: behind this bank's own work
-        JSDR_CUDA(cudaMemcpyAsync(b->fec->d_mettab, mettab, 512 * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->aux));
+        JSDR_CUDA(cudaMemcpyAsync(b->fec->d_mettab.get(), mettab, 512 * sizeof(int16_t), cudaMemcpyHostToDevice, ctx->aux));
         JSDR_CUDA(cudaStreamSynchronize(ctx->aux));
         return JSDR_OK;
     }
-    jsdr_fec_state *f = new jsdr_fec_state();
+    const char *what = "jsdr_bpsk_enable_fec";
+    std::unique_ptr<jsdr_fec_state, jsdr_fec_delete> f(new jsdr_fec_state());
     // Every detection of a call is decoded (cntDec must follow cntFEC as in :563-571): a channel
     // can complete at most one frame per 5200 bits of signal, so nchan * (max_bits/5200 + 2)
     // slots cover everything but a correlator firing on noise more than twice per frame time.
@@ -506,43 +509,38 @@ try {
     f->d_rs_par = d_rs_par[ctx->device & 63];
     max_frames = f->max_frames;
     const size_t nc = (size_t)b->nchan;
-    cudaError_t e = cudaMalloc(&f->d_hist[0], nc * fec::HIST);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_hist[1], nc * fec::HIST);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_frames, sizeof(fec::FrameMeta) * (size_t)max_frames);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_nframes, sizeof(int));
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_data, (size_t)max_frames * 256);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_cnt, sizeof(long long) * 2 * nc);
-    if (e == cudaSuccess) e = cudaMalloc(&f->d_mettab, 512 * sizeof(int16_t));
-    if (e == cudaSuccess) e = cudaMemcpy(f->d_mettab, mettab, 512 * sizeof(int16_t), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-        set_error("jsdr_bpsk_enable_fec: cudaMalloc: %s", cudaGetErrorString(e));
-        cudaGetLastError();
-        return JSDR_ENOMEM;
-    }
-    JSDR_CUDA(cudaMemsetAsync(f->d_hist[0], 0, nc * fec::HIST, ctx->stream));     // dmFECCorr starts as zeros (:503)
-    JSDR_CUDA(cudaMemsetAsync(f->d_nframes, 0, sizeof(int), ctx->stream));
-    JSDR_CUDA(cudaMemsetAsync(f->d_cnt, 0, sizeof(long long) * 2 * nc, ctx->stream));
+    JSDR_TRY(f->d_hist[0].alloc_zeroed(nc * fec::HIST, ctx->stream, what));      // dmFECCorr starts as zeros (:503)
+    JSDR_TRY(f->d_hist[1].alloc(nc * fec::HIST, what));
+    JSDR_TRY(f->d_frames.alloc(sizeof(fec::FrameMeta) * (size_t)max_frames, what));
+    JSDR_TRY(f->d_nframes.alloc_zeroed(sizeof(int), ctx->stream, what));
+    JSDR_TRY(f->d_data.alloc((size_t)max_frames * 256, what));
+    JSDR_TRY(f->d_cnt.alloc_zeroed(sizeof(long long) * 2 * nc, ctx->stream, what));
+    JSDR_TRY(f->d_mettab.alloc(512 * sizeof(int16_t), what));
+    JSDR_CUDA(cudaMemcpy(f->d_mettab.get(), mettab, 512 * sizeof(int16_t), cudaMemcpyHostToDevice));
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));            // the stage itself runs on the auxiliary stream
-    b->fec = f;
+    b->fec = std::move(f);
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
 // called by bpsk_receive after the bit-timing stage; like that stage it runs on the auxiliary stream
 int jsdr_fec_after_bits(jsdr_bpsk *b)
 {
-    jsdr_fec_state *f = b->fec;
+    jsdr_fec_state *f = b->fec.get();
     jsdr_ctx *ctx = b->ctx;
     const int nchan = b->nchan, max_bits = b->max_bits;
-    JSDR_CUDA(cudaMemsetAsync(f->d_nframes, 0, sizeof(int), ctx->aux));
+    int8_t *const bits = b->stage.d_bits.get();
+    int8_t *const hist = f->d_hist[f->cur].get(), *const hist_next = f->d_hist[f->cur ^ 1].get();
+    int32_t *const nbits = b->d_nbits.get();
+    JSDR_CUDA(cudaMemsetAsync(f->d_nframes.get(), 0, sizeof(int), ctx->aux));
     if (max_bits > 0) {
         dim3 grid((max_bits + 255) / 256, nchan);
         // cntBit lives at the end of each TimingState
         const long long *cnt_bit = reinterpret_cast<const long long *>(
-            reinterpret_cast<const char *>(b->d_ts) + offsetof(jsdr::bpsk::TimingState, cntBit));
+            reinterpret_cast<const char *>(b->d_ts.get()) + offsetof(jsdr::bpsk::TimingState, cntBit));
         ProfScope prof(ctx, JSDR_K_SYNC, ctx->aux);
-        fec::k_sync<<<grid, 256, 0, ctx->aux>>>(f->d_hist[f->cur], b->d_bits, b->d_nbits, max_bits, nchan, cnt_bit,
-                                                   (int)(sizeof(jsdr::bpsk::TimingState) / sizeof(long long)), f->d_frames,
-                                                   f->d_nframes, f->max_frames, f->d_cnt);
+        fec::k_sync<<<grid, 256, 0, ctx->aux>>>(hist, bits, nbits, max_bits, nchan, cnt_bit,
+                                                   (int)(sizeof(jsdr::bpsk::TimingState) / sizeof(long long)), f->d_frames.get(),
+                                                   f->d_nframes.get(), f->max_frames, f->d_cnt.get());
         JSDR_TRY(launched(ctx, "k_sync"));
     }
     const size_t smem = sizeof(fec::DecodeSmem);
@@ -553,26 +551,16 @@ int jsdr_fec_after_bits(jsdr_bpsk *b)
     }));
     {
         ProfScope prof(ctx, JSDR_K_FEC, ctx->aux);
-        fec::k_fec_decode<<<f->max_frames, 32, smem, ctx->aux>>>(f->d_hist[f->cur], b->d_bits, max_bits, f->d_frames,
-                                                                   f->d_nframes, f->max_frames, f->d_data, f->d_cnt + nchan,
-                                                                   f->d_mettab, f->d_rs_par);
+        fec::k_fec_decode<<<f->max_frames, 32, smem, ctx->aux>>>(hist, bits, max_bits, f->d_frames.get(),
+                                                                   f->d_nframes.get(), f->max_frames, f->d_data.get(),
+                                                                   f->d_cnt.get() + nchan, f->d_mettab.get(), f->d_rs_par);
         JSDR_TRY(launched(ctx, "k_fec_decode"));
     }
     dim3 g2((fec::HIST + 255) / 256, nchan);
-    fec::k_sync_shift<<<g2, 256, 0, ctx->aux>>>(f->d_hist[f->cur], f->d_hist[f->cur ^ 1], b->d_bits, b->d_nbits, max_bits);
+    fec::k_sync_shift<<<g2, 256, 0, ctx->aux>>>(hist, hist_next, bits, nbits, max_bits);
     JSDR_TRY(launched(ctx, "k_sync_shift"));
     f->cur ^= 1;
     return JSDR_OK;
-}
-
-void jsdr_fec_destroy(jsdr_bpsk *b)
-{
-    jsdr_fec_state *f = b->fec;
-    if (!f) return;
-    void *ptrs[] = {f->d_hist[0], f->d_hist[1], f->d_frames, f->d_nframes, f->d_data, f->d_cnt, f->d_mettab};
-    for (void *p : ptrs) cudaFree(p);
-    delete f;
-    b->fec = nullptr;
 }
 
 extern "C" int jsdr_bpsk_read_frames(jsdr_bpsk *b, int32_t *nframes, int32_t *chan, int64_t *bit_index,
@@ -580,18 +568,18 @@ extern "C" int jsdr_bpsk_read_frames(jsdr_bpsk *b, int32_t *nframes, int32_t *ch
 try {
     JSDR_REQUIRE(b && nframes, JSDR_EINVAL, "null argument");
     JSDR_REQUIRE(b->fec, JSDR_ESTATE, "jsdr_bpsk_enable_fec has not been called");
-    jsdr_fec_state *f = b->fec;
+    jsdr_fec_state *f = b->fec.get();
     jsdr_ctx *ctx = b->ctx;
     JSDR_TRY(ctx->bind());
     int n = 0;
-    JSDR_CUDA(cudaMemcpyAsync(&n, f->d_nframes, sizeof(int), cudaMemcpyDeviceToHost, ctx->aux));
+    JSDR_CUDA(cudaMemcpyAsync(&n, f->d_nframes.get(), sizeof(int), cudaMemcpyDeviceToHost, ctx->aux));
     JSDR_CUDA(cudaStreamSynchronize(ctx->aux));
     const int have = std::min(n, f->max_frames);
     std::vector<fec::FrameMeta> meta(have);
     std::vector<uint8_t> dat((size_t)have * 256);
     if (have > 0) {
-        JSDR_CUDA(cudaMemcpyAsync(meta.data(), f->d_frames, sizeof(fec::FrameMeta) * have, cudaMemcpyDeviceToHost, ctx->aux));
-        JSDR_CUDA(cudaMemcpyAsync(dat.data(), f->d_data, (size_t)have * 256, cudaMemcpyDeviceToHost, ctx->aux));
+        JSDR_CUDA(cudaMemcpyAsync(meta.data(), f->d_frames.get(), sizeof(fec::FrameMeta) * have, cudaMemcpyDeviceToHost, ctx->aux));
+        JSDR_CUDA(cudaMemcpyAsync(dat.data(), f->d_data.get(), (size_t)have * 256, cudaMemcpyDeviceToHost, ctx->aux));
         JSDR_CUDA(cudaStreamSynchronize(ctx->aux));
     }
     // detection order on the device is not deterministic: report by (channel, bit)
@@ -620,8 +608,8 @@ try {
     jsdr_ctx *ctx = b->ctx;
     JSDR_TRY(ctx->bind());
     const size_t nc = (size_t)b->nchan;
-    JSDR_CUDA(cudaMemcpyAsync(cnt_fec, b->fec->d_cnt, sizeof(long long) * nc, cudaMemcpyDeviceToHost, ctx->aux));
-    JSDR_CUDA(cudaMemcpyAsync(cnt_dec, b->fec->d_cnt + nc, sizeof(long long) * nc, cudaMemcpyDeviceToHost, ctx->aux));
+    JSDR_CUDA(cudaMemcpyAsync(cnt_fec, b->fec->d_cnt.get(), sizeof(long long) * nc, cudaMemcpyDeviceToHost, ctx->aux));
+    JSDR_CUDA(cudaMemcpyAsync(cnt_dec, b->fec->d_cnt.get() + nc, sizeof(long long) * nc, cudaMemcpyDeviceToHost, ctx->aux));
     JSDR_CUDA(cudaStreamSynchronize(ctx->aux));
     return JSDR_OK;
 } JSDR_CATCH_ALL

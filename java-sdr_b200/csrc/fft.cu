@@ -3,7 +3,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
-
+#include <memory>
 #include <vector>
 
 #include "fft_fourstep.cuh"
@@ -137,18 +137,16 @@ static int launch_fourstep(jsdr_fft *f, const Args &a, int in_fmt, int out_mode,
         chunk_mb = e ? std::max(1, atoi(e)) : 32;
     }
     const int chunk = std::max(1, std::min(f->max_batch, (int)(((long)chunk_mb << 20) / ((long)N * 8))));
-    if (!f->d_work[0]) {
-        cudaError_t e = cudaMalloc(&f->d_work[0], (size_t)chunk * N * sizeof(float2));
-        if (e == cudaSuccess) e = cudaMalloc(&f->d_work[1], (size_t)chunk * N * sizeof(float2));
-        if (e == cudaSuccess) e = cudaMalloc(&f->d_best, sizeof(unsigned long long) * (size_t)f->max_batch);
-        if (e != cudaSuccess) {
-            set_error("fft workspace: %s", cudaGetErrorString(e));
-            cudaGetLastError();
-            return JSDR_ENOMEM;
-        }
+    if (!f->work.best) {
+        jsdr_fft::Work w;
+        JSDR_TRY(w.z[0].alloc((size_t)chunk * N * sizeof(float2), "fft workspace"));
+        JSDR_TRY(w.z[1].alloc((size_t)chunk * N * sizeof(float2), "fft workspace"));
+        JSDR_TRY(w.best.alloc(sizeof(unsigned long long) * (size_t)f->max_batch, "fft workspace"));
+        f->work = std::move(w);
     }
+    unsigned long long *best = f->work.best.get();
     if (out_mode == OUT_PSD)
-        JSDR_CUDA(cudaMemsetAsync(f->d_best, 0, sizeof(unsigned long long) * (size_t)a.nblocks, st));
+        JSDR_CUDA(cudaMemsetAsync(best, 0, sizeof(unsigned long long) * (size_t)a.nblocks, st));
     // Chunks alternate between two streams (and two Z buffers): while one chunk's row kernel
     // drains, the next chunk's column kernel already fills the SMs.
     const bool two = a.nblocks > chunk && st != ctx->aux;
@@ -163,9 +161,9 @@ static int launch_fourstep(jsdr_fft *f, const Args &a, int in_fmt, int out_mode,
         FsArgs fa;
         fa.nblocks = std::min(chunk, a.nblocks - b0);
         fa.in = reinterpret_cast<const char *>(a.in) + (size_t)b0 * N * in_el;
-        fa.z = f->d_work[ci & 1];
+        fa.z = f->work.z[ci & 1].get();
         fa.out = (out_mode == OUT_PSD) ? a.out + (size_t)b0 * (N + 2) : a.out + (size_t)b0 * N * 2;
-        fa.best = f->d_best + b0;
+        fa.best = best + b0;
         fa.tw = a.tw;
         fa.cf = a.cf;
         fa.db_off = a.db_off;
@@ -189,7 +187,7 @@ static int launch_fourstep(jsdr_fft *f, const Args &a, int in_fmt, int out_mode,
         JSDR_CUDA(cudaStreamWaitEvent(st, ctx->ev_aux_join, 0));
     }
     if (out_mode == OUT_PSD) {
-        k_fs_finish<<<(a.nblocks + 127) / 128, 128, 0, st>>>(f->d_best, a.out, a.peak_bin, N, a.rate, a.nblocks);
+        k_fs_finish<<<(a.nblocks + 127) / 128, 128, 0, st>>>(best, a.out, a.peak_bin, N, a.rate, a.nblocks);
         JSDR_TRY(launched(ctx, "k_fs_finish"));
     }
     return JSDR_OK;
@@ -199,21 +197,18 @@ static int launch_generic(jsdr_fft *f, const Args &a, int in_fmt, int out_mode, 
 {
     jsdr_ctx *ctx = f->ctx;
     const size_t need = (size_t)f->max_batch * (size_t)f->n * sizeof(float2);
-    if (!f->d_work[0]) {
-        for (int i = 0; i < 2; i++) {
-            cudaError_t e = cudaMalloc(&f->d_work[i], need);
-            if (e != cudaSuccess) {
-                set_error("fft workspace: cudaMalloc(%zu): %s", need, cudaGetErrorString(e));
-                cudaGetLastError();
-                return JSDR_ENOMEM;
-            }
-        }
+    if (!f->work.z[0]) {
+        jsdr_fft::Work w;
+        JSDR_TRY(w.z[0].alloc(need, "fft workspace"));
+        JSDR_TRY(w.z[1].alloc(need, "fft workspace"));
+        f->work = std::move(w);
     }
+    float2 *z0 = f->work.z[0].get(), *z1 = f->work.z[1].get();
     const long long total = (long long)a.nblocks * f->n;
-    k_generic_load<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(a.in, f->d_work[0], total, in_fmt, a.ic, a.qc);
+    k_generic_load<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(a.in, z0, total, in_fmt, a.ic, a.qc);
     JSDR_TRY(launched(ctx, "k_generic_load"));
     int rc = JSDR_OK;
-    float2 *res = fftg::run<float>(ctx, st, f->d_work[0], f->d_work[1], f->n, a.nblocks, -1, &rc);
+    float2 *res = fftg::run<float>(ctx, st, z0, z1, f->n, a.nblocks, -1, &rc);
     if (rc != JSDR_OK) return rc;
     if (out_mode == OUT_SPECTRUM) {
         JSDR_CUDA(cudaMemcpyAsync(a.out, res, (size_t)total * sizeof(float2), cudaMemcpyDeviceToDevice, st));
@@ -230,7 +225,7 @@ int launch(jsdr_fft *f, const void *d_in, int in_fmt, int batch, float *d_out, i
     a.in = d_in;
     a.out = d_out;
     a.peak_bin = d_peak;
-    a.tw = f->d_tw;
+    a.tw = f->d_tw.get();
     a.nblocks = batch;
     a.rate = f->rate;
     // fft.java:199-200  cf = 2f/(float)N; cf = cf*cf  (float arithmetic)
@@ -255,9 +250,9 @@ int launch(jsdr_fft *f, const void *d_in, int in_fmt, int batch, float *d_out, i
     }
     if (f->split) {
         a.nblocks = 2 * batch;                    // half blocks
-        a.tw2 = f->d_tw2;
-        a.best = f->d_best;
-        a.cnt = f->d_cnt;
+        a.tw2 = f->d_tw2.get();
+        a.best = f->d_best.get();
+        a.cnt = f->d_cnt.get();
         return reinterpret_cast<launch_fn>(f->launch)(f->ctx, a, in_fmt, out_mode, st);
     }
     if (f->fs_n1) return launch_fourstep(f, a, in_fmt, out_mode, st);
@@ -287,8 +282,8 @@ try {
         return JSDR_EUNSUPPORTED;
     }
     JSDR_TRY(ctx->bind());
-    jsdr_fft *f = new jsdr_fft();
-    f->ctx = ctx;
+    const char *what = "jsdr_fft_create";
+    std::unique_ptr<jsdr_fft> f(new jsdr_fft(ctx));
     f->n = n;
     f->rate = rate;
     f->max_batch = max_batch;
@@ -306,54 +301,34 @@ try {
         double ang = 2.0 * M_PI * (double)t / (double)m;
         tw[t] = make_float2((float)cos(ang), (float)-sin(ang));
     }
-    cudaError_t e = cudaMalloc(&f->d_tw, sizeof(float2) * m);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(f->d_tw, tw.data(), sizeof(float2) * m, cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess && f->split) {                          // the radix-2 step's twiddles and the halves' meeting point
+    JSDR_TRY(f->d_tw.alloc(sizeof(float2) * m, what));
+    JSDR_CUDA(cudaMemcpyAsync(f->d_tw.get(), tw.data(), sizeof(float2) * m, cudaMemcpyHostToDevice, ctx->stream));
+    if (f->split) {                                              // the radix-2 step's twiddles and the halves' meeting point
         for (int t = 0; t < m; t++) {
             double ang = 2.0 * M_PI * (double)t / (double)n;
             tw[t] = make_float2((float)cos(ang), (float)-sin(ang));
         }
-        e = cudaMalloc(&f->d_tw2, sizeof(float2) * m);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(f->d_tw2, tw.data(), sizeof(float2) * m, cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess) e = cudaMalloc(&f->d_best, sizeof(unsigned long long) * (size_t)max_batch);
-        if (e == cudaSuccess) e = cudaMalloc(&f->d_cnt, sizeof(unsigned) * (size_t)max_batch);
-        if (e == cudaSuccess) e = cudaMemsetAsync(f->d_best, 0, sizeof(unsigned long long) * (size_t)max_batch, ctx->stream);
-        if (e == cudaSuccess) e = cudaMemsetAsync(f->d_cnt, 0, sizeof(unsigned) * (size_t)max_batch, ctx->stream);
+        JSDR_TRY(f->d_tw2.alloc(sizeof(float2) * m, what));
+        JSDR_CUDA(cudaMemcpyAsync(f->d_tw2.get(), tw.data(), sizeof(float2) * m, cudaMemcpyHostToDevice, ctx->stream));
+        JSDR_TRY(f->d_best.alloc_zeroed(sizeof(unsigned long long) * (size_t)max_batch, ctx->stream, what));
+        JSDR_TRY(f->d_cnt.alloc_zeroed(sizeof(unsigned) * (size_t)max_batch, ctx->stream, what));
     }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-        set_error("jsdr_fft_create: %s", cudaGetErrorString(e));
-        cudaGetLastError();
-        jsdr_fft_destroy(f);
-        return e == cudaErrorMemoryAllocation ? JSDR_ENOMEM : JSDR_ECUDA;
-    }
-    *out = f;
+    JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
+    *out = f.release();
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
 extern "C" int jsdr_fft_destroy(jsdr_fft *f)
 try {
-    if (!f) return JSDR_OK;
-    f->ctx->bind();
-    cudaFree(f->d_tw);
-    cudaFree(f->d_in);
-    cudaFree(f->d_pix);
-    cudaFree(f->d_out);
-    cudaFree(f->d_peak);
-    cudaFree(f->d_work[0]);
-    cudaFree(f->d_work[1]);
-    cudaFree(f->d_best);
-    cudaFree(f->d_tw2);
-    cudaFree(f->d_cnt);
     delete f;
     return JSDR_OK;
 } JSDR_CATCH_ALL
 
 int jsdr::fft::ensure_staging(jsdr_fft *f, size_t in_bytes, size_t out_bytes)
 {
-    JSDR_TRY(grow(&f->d_in, &f->in_cap, in_bytes));
-    JSDR_TRY(grow(reinterpret_cast<void **>(&f->d_out), &f->out_cap, out_bytes));
-    if (!f->d_peak) JSDR_CUDA(cudaMalloc(&f->d_peak, sizeof(int32_t) * (size_t)f->max_batch));
+    JSDR_TRY(f->d_in.grow(in_bytes, "fft staging"));
+    JSDR_TRY(f->d_out.grow(out_bytes, "fft staging"));
+    return f->d_peak.grow(sizeof(int32_t) * (size_t)f->max_batch, "fft staging");
     return JSDR_OK;
 }
 
@@ -376,11 +351,11 @@ int fft_run(jsdr_fft *f, const void *in, int in_fmt, int batch, int ic, int qc, 
         return fft::launch(f, in, in_fmt, batch, out, peak_bin, out_mode, ic, qc, ctx->stream);
     }
     JSDR_TRY(fft::ensure_staging(f, in_bytes, out_elems * sizeof(float)));
-    JSDR_CUDA(cudaMemcpyAsync(f->d_in, in, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    JSDR_TRY(fft::launch(f, f->d_in, in_fmt, batch, f->d_out, f->d_peak, out_mode, ic, qc, ctx->stream));
-    JSDR_CUDA(cudaMemcpyAsync(out, f->d_out, out_elems * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    JSDR_CUDA(cudaMemcpyAsync(f->d_in.get(), in, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    JSDR_TRY(fft::launch(f, f->d_in.get(), in_fmt, batch, f->d_out.get(), f->d_peak.get(), out_mode, ic, qc, ctx->stream));
+    JSDR_CUDA(cudaMemcpyAsync(out, f->d_out.get(), out_elems * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     if (peak_bin && out_mode == fft::OUT_PSD)
-        JSDR_CUDA(cudaMemcpyAsync(peak_bin, f->d_peak, sizeof(int32_t) * (size_t)batch,
+        JSDR_CUDA(cudaMemcpyAsync(peak_bin, f->d_peak.get(), sizeof(int32_t) * (size_t)batch,
                                   cudaMemcpyDeviceToHost, ctx->stream));
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     return JSDR_OK;

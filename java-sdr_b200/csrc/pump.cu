@@ -61,8 +61,8 @@ int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int
         // stream) starts beside this FFT and not behind it; the demod kernels follow the FFT, ahead
         // of the bank's wait for this block's tuner-phase replay.
         if (px) JSDR_TRY(fft::ensure_staging(f, 0, psd_bytes));
-        float *d_psd = px ? f->d_out : psd;
-        int32_t *d_peak = (px && !peak_bin) ? f->d_peak : peak_bin;
+        float *d_psd = px ? f->d_out.get() : psd;
+        int32_t *d_peak = (px && !peak_bin) ? f->d_peak.get() : peak_bin;
         const void *d_in;
         JSDR_TRY(bpsk::receive_begin(b, raw, bpsk::FMT_S16, S, S, mem, true, &d_in));
         JSDR_TRY(fft::launch(f, d_in, fft::IN_S16, batch, d_psd, d_peak, fft::OUT_PSD, ic, qc, ctx->stream));
@@ -78,8 +78,11 @@ int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int
     }
 
     JSDR_TRY(fft::ensure_staging(f, 0, psd_bytes));
-    JSDR_TRY(grow(&b->d_in, &b->in_cap, (size_t)b->nchan * (size_t)S * 4));
-    if (px) JSDR_TRY(grow(reinterpret_cast<void **>(&f->d_pix), &f->pix_cap, (size_t)batch * px->width * sizeof(int32_t)));
+    JSDR_TRY(b->d_in.grow((size_t)b->nchan * (size_t)S * 4, "tuner bank staging"));
+    if (px) JSDR_TRY(f->d_pix.grow((size_t)batch * px->width * sizeof(int32_t), "pixel staging"));
+    char *d_raw = static_cast<char *>(b->d_in.get());   // the batch, resident for all handlers
+    float *d_psd = f->d_out.get();
+    int32_t *d_peak = f->d_peak.get(), *d_pix = f->d_pix.get();
     // Host path, pipelined over channel chunks: PCIe is full duplex, so the upload of chunk
     // c+1 (copy_in stream) runs beside the FFT of chunk c (main stream) and the download of
     // the results of chunk c-1 (copy_out stream).  The tuner bank runs once the whole batch is in.
@@ -91,28 +94,28 @@ int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int
         if (c1 == c0) continue;
         const size_t in_off = (size_t)c0 * (size_t)S * 4, in_len = (size_t)(c1 - c0) * (size_t)S * 4;
         const size_t blk0 = (size_t)c0 * nblocks, nblk = (size_t)(c1 - c0) * nblocks;
-        JSDR_CUDA(cudaMemcpyAsync((char *)b->d_in + in_off, (const char *)raw + in_off, in_len,
+        JSDR_CUDA(cudaMemcpyAsync(d_raw + in_off, (const char *)raw + in_off, in_len,
                                   cudaMemcpyHostToDevice, ctx->copy_in));
         JSDR_CUDA(cudaEventRecord(ctx->ev_chunk_in[c], ctx->copy_in));
         JSDR_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_chunk_in[c], 0));
-        JSDR_TRY(fft::launch(f, (const char *)b->d_in + in_off, fft::IN_S16, (int)nblk, f->d_out + blk0 * N2,
-                             f->d_peak + blk0, fft::OUT_PSD, ic, qc, ctx->stream));
+        JSDR_TRY(fft::launch(f, d_raw + in_off, fft::IN_S16, (int)nblk, d_psd + blk0 * N2, d_peak + blk0, fft::OUT_PSD,
+                             ic, qc, ctx->stream));
         if (px)
-            JSDR_TRY(jsdr_launch_waterfall(ctx, f->d_out + blk0 * N2, f->n, (int)nblk, px->width, px->rgb,
-                                           f->d_pix + blk0 * px->width, ctx->stream));
+            JSDR_TRY(jsdr_launch_waterfall(ctx, d_psd + blk0 * N2, f->n, (int)nblk, px->width, px->rgb,
+                                           d_pix + blk0 * px->width, ctx->stream));
         JSDR_CUDA(cudaEventRecord(ctx->ev_chunk_done[c], ctx->stream));
         JSDR_CUDA(cudaStreamWaitEvent(ctx->copy_out, ctx->ev_chunk_done[c], 0));
         if (px) {
-            JSDR_CUDA(cudaMemcpyAsync(px->pixels + blk0 * px->width, f->d_pix + blk0 * px->width,
+            JSDR_CUDA(cudaMemcpyAsync(px->pixels + blk0 * px->width, d_pix + blk0 * px->width,
                                       nblk * px->width * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->copy_out));
-            JSDR_CUDA(cudaMemcpy2DAsync(px->peak + blk0 * 2, 2 * sizeof(float), f->d_out + blk0 * N2 + f->n, N2 * sizeof(float),
+            JSDR_CUDA(cudaMemcpy2DAsync(px->peak + blk0 * 2, 2 * sizeof(float), d_psd + blk0 * N2 + f->n, N2 * sizeof(float),
                                         2 * sizeof(float), nblk, cudaMemcpyDeviceToHost, ctx->copy_out));
         } else {
-            JSDR_CUDA(cudaMemcpyAsync(psd + blk0 * N2, f->d_out + blk0 * N2, nblk * N2 * sizeof(float),
+            JSDR_CUDA(cudaMemcpyAsync(psd + blk0 * N2, d_psd + blk0 * N2, nblk * N2 * sizeof(float),
                                       cudaMemcpyDeviceToHost, ctx->copy_out));
         }
         if (peak_bin)
-            JSDR_CUDA(cudaMemcpyAsync(peak_bin + blk0, f->d_peak + blk0, sizeof(int32_t) * nblk,
+            JSDR_CUDA(cudaMemcpyAsync(peak_bin + blk0, d_peak + blk0, sizeof(int32_t) * nblk,
                                       cudaMemcpyDeviceToHost, ctx->copy_out));
     }
     if (dm) {   // the whole batch is in (the main stream waited for every chunk): demod, audio down beside the bank
@@ -120,7 +123,7 @@ int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int
         int16_t *d_audio = nullptr;
         float *d_ma = nullptr;
         JSDR_TRY(jsdr_pump_demod_staging(d, S, nblocks, &d_audio, &d_ma));
-        JSDR_TRY(jsdr_pump_demod_run(d, static_cast<const int16_t *>(b->d_in), S, f->n, ic, qc, d_audio,
+        JSDR_TRY(jsdr_pump_demod_run(d, reinterpret_cast<const int16_t *>(d_raw), S, f->n, ic, qc, d_audio,
                                      dm->max_avg ? d_ma : nullptr));
         JSDR_CUDA(cudaEventRecord(d->ev_audio_ready, ctx->stream));
         JSDR_CUDA(cudaStreamWaitEvent(ctx->copy_out, d->ev_audio_ready, 0));
@@ -130,7 +133,7 @@ int pump_receive(jsdr_fft *f, jsdr_bpsk *b, const int16_t *raw, int nblocks, int
             JSDR_CUDA(cudaMemcpyAsync(dm->max_avg, d_ma, sizeof(float) * 2 * (size_t)b->nchan * nblocks,
                                       cudaMemcpyDeviceToHost, ctx->copy_out));
     }
-    JSDR_TRY(bpsk::receive(b, b->d_in, bpsk::FMT_S16, S, S, ic, qc, JSDR_MEM_DEVICE, true));
+    JSDR_TRY(bpsk::receive(b, d_raw, bpsk::FMT_S16, S, S, ic, qc, JSDR_MEM_DEVICE, true));
     JSDR_CUDA(cudaStreamSynchronize(ctx->copy_out));
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     return JSDR_OK;

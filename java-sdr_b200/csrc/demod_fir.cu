@@ -59,15 +59,17 @@ __device__ __forceinline__ float2 mul2(float2 a, float2 b)
     return *reinterpret_cast<float2 *>(&r);
 }
 
-// (float)Math.sin(car), (float)Math.cos(car) for the NCO (:425-426).  car is a float in [0, 2 pi]
-// (:427-429), so the binary64 sine and cosine need no large-argument path: one Cody-Waite step by
-// k*(pi/2) (k <= 5, the product is exact inside the fma), the two minimax kernels of the classic
-// binary64 libm on [-pi/4, pi/4] (absolute error below 2.3e-16, so the float results differ from a
-// correctly rounded libm's in about one sample in 2^28 and then by one float ulp), quadrant by
-// selects on the rounded floats.  Coefficients sit in constant memory and enter the DFMAs as
-// operands; the library's sincos() spent as many instructions moving its constants into uniform
-// registers and testing for its slow path as on arithmetic.  Arguments beyond |x| <= 8 (never
-// produced by the phase recurrence; NaN) go to the library.
+// (float)Math.sin(car), (float)Math.cos(car) for the NCO (:425-426).  For 0 <= phi < 2 pi car stays
+// in [0, 2 pi] (:427-429), where the binary64 sine and cosine need no large-argument path: one
+// Cody-Waite step by k*(pi/2) (|k| <= 5, the product is exact inside the fma), the two minimax
+// kernels of the classic binary64 libm on [-pi/4, pi/4], quadrant by selects on the rounded floats.
+// Over every float in [-8, 8] the float results equal the correctly rounded sin and cos
+// (tools/nco_scan.py; tests/test_nco_model.py, tests/test_gpu_nco.py).  Coefficients sit in
+// constant memory and enter the DFMAs as operands; the library's sincos() spent as many
+// instructions moving its constants into uniform registers and testing for its slow path as on
+// arithmetic.  Arguments beyond |x| <= 8 and NaN go to the library, out of line: car reaches them
+// for flo < 0 (phi < 0: car grows until car - phi rounds back to car, near 2^24 |phi|) and for
+// flo > rate (phi > 2 pi: car runs negative), as in the reference.
 __constant__ double c_trig[15] = {
     -1.66666666666666324348e-01, 8.33333333332248946124e-03, -1.98412698298579493134e-04,
     2.75573137070700676789e-06, -2.50507602534068634195e-08, 1.58969099521155010221e-10,

@@ -159,6 +159,14 @@ class Demod:
         return out
 
 
+def demod_phases(phi, car0, n: int) -> np.ndarray:
+    """demod.java:427-429 alone: float32[n + 1], the car of each of n samples from car0 and the
+    value carried after them."""
+    out = np.empty(n + 1, dtype=np.float32)
+    lib().orc_demod_phases(C.c_float(phi), C.c_float(car0), int(n), _p(out, C.c_float))
+    return out
+
+
 def demod_detect(sam: np.ndarray, mode: int, rate: int, doagc: bool, lilq: np.ndarray):
     """demod.java:405-481 on the FIR/NCO output; lilq (float32[2]) is updated in place.
     Returns (audio int16[n], max_avg float32[2])."""

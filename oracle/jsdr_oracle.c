@@ -535,6 +535,19 @@ void orc_demod_receive(orc_demod *s, const float *buf, int nsamples, float *out)
     }
 }
 
+/* The value of car seen by each of n samples of orc_demod_receive (:425-426), from car0 on, and
+ * the carried value after them in out[n]: the two lines of :427-429 on their own. */
+void orc_demod_phases(float phi, float car0, int n, float *out)
+{
+    float car = car0;
+    for (int k = 0; k < n; k++) {
+        out[k] = car;
+        car -= phi;
+        if (car < 0.0f) car += (float)(2 * M_PI);
+    }
+    out[n] = car;
+}
+
 static int j_f2i(float f)                    /* Java (int)float */
 {
     if (f != f) return 0;

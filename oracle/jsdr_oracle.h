@@ -90,6 +90,9 @@ void orc_demod_weights(orc_demod *s, int flo, int fhi); /* flo==INT32_MIN -> all
 /* out = the value of sam[] after the FIR and down-shift stages
  * (what demod.java:436-437 copies to dbg[]) */
 void orc_demod_receive(orc_demod *s, const float *buf, int nsamples, float *out);
+/* The NCO phase alone (:427-429): out[k] = car used by sample k (k < n) from car0, out[n] = the
+ * value carried to the next call.  out holds n + 1 floats. */
+void orc_demod_phases(float phi, float car0, int n, float *out);
 
 /* The rest of demod.receive (demod.java:405-481) on the FIR/NCO output `sam` (2n floats):
  * detector per mode (0 off, 1 raw, 2 AM, 3 NFM, 4 WFM; :439-463), max/avg, AGC, s16

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import jsdrcuda as J
+import nco_phase as N
 import oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -116,8 +117,8 @@ def test_s16_and_f32_blocks_alternate_on_one_handle(ctx):
 
 @pytest.mark.parametrize("mode", [0, 1, 2, 3, 4])
 def test_audio_raw_against_the_oracle(ctx, mode):
-    """Without the NCO every s16 sample equals the oracle's; with it (cos/sin from another libm)
-    within one LSB."""
+    """Every s16 sample and max/avg pair equal to the oracle's detectors, without the NCO on the
+    oracle's FIR output, with it on the NCO model of tests/nco_phase.py."""
     nchan = 2
     rng = np.random.default_rng(200 + mode)
     for dodwn in (False, True):
@@ -126,19 +127,18 @@ def test_audio_raw_against_the_oracle(ctx, mode):
         orc, lilq = [], [np.zeros(2, np.float32) for _ in range(nchan)]
         for c in range(nchan):
             d.weights(9000 + 1000 * c, 15000, chan=c)
-            o = O.Demod(RATE, True, dodwn)
+            o = N.RefDemod(RATE, True, dodwn)
             o.weights(9000 + 1000 * c, 15000)
             orc.append(o)
         for n in LENGTHS:
             raw = (rng.standard_normal((nchan, 2 * n)) * 6000).astype(np.int16)
             audio, ma = d.receive_audio_raw(raw, ic=9, qc=-9)
             for c in range(nchan):
-                ref, rma = O.demod_detect(orc[c].receive(O.s16_to_float(raw[c], 9, -9)), mode, RATE, True, lilq[c])
-                if dodwn:
-                    assert np.max(np.abs(audio[c].astype(np.int32) - ref.astype(np.int32))) <= 1, (n, c)
-                else:
-                    assert np.array_equal(audio[c], ref), (n, c)
-                    assert np.array_equal(ma[c], rma, equal_nan=True), (n, c)
+                mixed, allowed = orc[c].receive(O.s16_to_float(raw[c], 9, -9))
+                assert not allowed, (n, c)
+                ref, rma = O.demod_detect(mixed, mode, RATE, True, lilq[c])
+                assert np.array_equal(audio[c], ref), (dodwn, n, c)
+                assert np.array_equal(ma[c], rma, equal_nan=True), (dodwn, n, c)
         d.close()
 
 

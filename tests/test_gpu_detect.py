@@ -4,6 +4,7 @@ import numpy as np
 import pytest
 
 import jsdrcuda as J
+import nco_phase as N
 import oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -66,21 +67,24 @@ def test_am_running_mean_special_operands(ctx, doagc):
     d.close()
 
 
-def test_demod_audio_with_nco_within_one_lsb(ctx):
-    """With the down-shift on, cos/sin come from different libms: one s16 LSB."""
+def test_demod_audio_with_nco_bit_exact(ctx):
+    """With the down-shift on: every s16 sample and max/avg pair equal to the oracle's detectors on
+    the NCO model of tests/nco_phase.py (the kernel's own sine / cosine, emulated bit for bit)."""
     rate = 96000
     rng = np.random.default_rng(3)
     d = J.demod(ctx, J.AudioDescriptor(rate), max_block=9600)
     d.weights(9000, 15000)
     d.set_mode(J.demod.MODE_NFM, False)
-    o = O.Demod(rate, True, True)
+    o = N.RefDemod(rate)
     o.weights(9000, 15000)
     lilq = np.zeros(2, np.float32)
     for _ in range(3):
         x = (rng.standard_normal(2 * 9600) * 0.2).astype(np.float32)
-        audio, _ = d.receive_audio(x)
-        ref, _ = O.demod_detect(o.receive(x), 3, rate, False, lilq)
-        assert np.max(np.abs(audio[0].astype(np.int32) - ref.astype(np.int32))) <= 1
+        audio, ma = d.receive_audio(x)
+        mixed, allowed = o.receive(x)
+        assert not allowed
+        ref, rma = O.demod_detect(mixed, 3, rate, False, lilq)
+        assert np.array_equal(audio[0], ref) and np.array_equal(ma[0], rma)
     d.close()
 
 

@@ -10,6 +10,7 @@ bit-exactly.
 import numpy as np
 import pytest
 
+import nco_phase as N
 import oracle as O
 from oracle import siggen
 from conftest import load_s16
@@ -321,14 +322,14 @@ def test_demod_fir_and_nco(ctx, golden):
     w = d.weights(3000, 6000)
     assert np.array_equal(w, golden["demod_w"])                   # host formula, demod.java:356-366
     d.set_flags(True, True)
-    o = O.Demod(44100, True, True)
+    o = N.RefDemod(44100)                                         # the oracle's FIR, the NCO of tests/nco_phase.py
     o.weights(3000, 6000)
     for k in range(3):                                            # carried FIR history and NCO phase
         y = d.receive(buf)[0]
-        r = o.receive(buf)
-        assert np.max(np.abs(y - r)) <= 1e-6                      # float path; full scale is 1
+        r, allowed = o.receive(buf)
+        assert not allowed and np.array_equal(y, r)               # every float, bit for bit
         if k < 2:
-            assert np.max(np.abs(y - golden[f"demod_out{k + 1}"])) <= 1e-6
+            assert np.array_equal(y, golden[f"demod_out{k + 1}"])
     # FIR alone is exact (no transcendental): float mul/add in the reference order
     d2 = J.demod(ctx, adsc, dofir=True, dodwn=False)
     d2.weights(3000, 6000)
@@ -351,14 +352,15 @@ def test_demod_many_channels_ragged(ctx):
     for c in range(nchan):
         lo = -20000 + 9000 * c
         d.weights(lo, lo + 6000, chan=c)
-        o = O.Demod(rate, True, True)
+        o = N.RefDemod(rate)
         o.weights(lo, lo + 6000)
         os_.append(o)
     for n in (5000, 1, 19, 20, 21, 1023, 1024, 1025, 33):
         x = rng.uniform(-1, 1, (nchan, 2 * n)).astype(np.float32)
         y = d.receive(x)
         for c in range(nchan):
-            assert np.max(np.abs(y[c] - os_[c].receive(x[c]))) <= 1e-6, (n, c)
+            r, allowed = os_[c].receive(x[c])
+            assert N.matches(y[c], r, allowed), (n, c)
     d.close()
 
 

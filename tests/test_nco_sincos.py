@@ -4,7 +4,8 @@ as demod.java:425-426 does with Math.cos / Math.sin.  The coefficients are read 
 source, the routine is restated in numpy binary64 (fused multiply-adds become a multiply and an add:
 a difference of an ulp of binary64, far below the float rounding this test looks at) and compared
 with libm over the phase range of the recurrence (:427-429) and beyond it up to the routine's own
-limit.  No GPU needed; the kernel itself is checked against the oracle in tests/test_gpu_parity.py."""
+limit.  No GPU needed; tests/test_nco_model.py holds the same routine to exact arithmetic and the
+correctly rounded float, and tests/test_gpu_nco.py the kernel to that model."""
 import os
 import re
 

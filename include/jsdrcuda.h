@@ -102,7 +102,8 @@ int jsdr_timer_stop_ms(jsdr_ctx *ctx, float *ms);
  * (:223-226).  peak_bin (nullable, int32 per block) additionally exports the
  * arg-max bin (-1 if no bin compared greater), because the Hz value wraps
  * beyond +-53.7 kHz at 192 kS/s (SURVEY Q2).
- * No window is applied (fft.java never applies win[]; SURVEY Q1).
+ * No window is applied unless jsdr_fft_set_window sets one (fft.java never applies
+ * win[]; SURVEY Q1).
  */
 int jsdr_fft_supported(int n);   /* 1 if a plan exists for n */
 int jsdr_fft_create(jsdr_ctx *ctx, int n, int rate, int max_batch, jsdr_fft **out);
@@ -113,6 +114,20 @@ int jsdr_fft_receive_s16(jsdr_fft *f, const int16_t *raw, int batch, int ic, int
                          float *psd, int32_t *peak_bin, int mem);
 /* the spectrum itself (what complexForward leaves in dat[]): float[2n] per block */
 int jsdr_fft_forward_f32(jsdr_fft *f, const float *iq, int batch, float *spec, int mem);
+/* Multiply each block's sample t (I and Q alike) by win[t] before the transform: what fft.java
+ * would publish if receive() applied its win[] (fft.java:72-73) to dat[] ahead of complexForward.
+ * win is host memory, float[n]; NULL removes the window.  No gain correction: cf stays (2/n)^2.
+ * Applies to jsdr_fft_receive_f32/_s16, jsdr_fft_forward_f32 and the fft part of the three pumps;
+ * the bank and the demod handler of a pump still see unwindowed samples.
+ *   - stream-ordered on the context's stream: work already enqueued with JSDR_MEM_DEVICE uses the
+ *     window in force when it was enqueued, calls after this one use the new window.
+ *   - a non-finite entry (JSDR_EINVAL, the message names the first one) or a failed allocation
+ *     (JSDR_ENOMEM) leaves the previous window in force.
+ *   - arithmetic: one binary32 multiply per component on the converted sample, before any
+ *     butterfly: RN(x*win[t]) for float input, RN((float)s*win[t]) for s16 input, s the value after
+ *     the ic / qc correction (the 1/32767 stays folded into cf).  Java's order, RN(RN(s/32767f)*w),
+ *     differs from this by a few ulps per sample, far inside the 1e-4 parity bar. */
+int jsdr_fft_set_window(jsdr_fft *f, const float *win);
 
 /* ------------------------------------------------------- FUNcubeBPSKDemod.java
  * A bank of `nchan` independent FUNcube tuners.  One receive call is one

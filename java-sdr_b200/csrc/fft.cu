@@ -48,8 +48,10 @@ static const PlanEntry *find_plan(int n)
 static launch_fn split_plan(int n) { return n == 32768 ? launch_split_n16384 : nullptr; }
 
 // ---- lengths without a single-CTA plan: fft_generic.cuh stages + a PSD pass -------------
+// WIN: sample i times win[i mod n] (apply_win, fft_kernels.cuh)
+template <bool WIN>
 __global__ void __launch_bounds__(256) k_generic_load(const void *__restrict__ in, float2 *__restrict__ out, long long total,
-                                                     int in_fmt, int ic, int qc)
+                                                     int in_fmt, int ic, int qc, const float *__restrict__ win, int n)
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
@@ -61,6 +63,7 @@ __global__ void __launch_bounds__(256) k_generic_load(const void *__restrict__ i
         const short si = (short)((int)(w & 0xffffu) + ic), sq = (short)((int)(w >> 16) + qc);
         out[i] = make_float2((float)si, (float)sq);
     }
+    if constexpr (WIN) out[i] = apply_win(out[i], win, (int)(i % n));
 }
 
 // fft.java:199-224 on a finished spectrum: one CTA per block
@@ -111,18 +114,26 @@ __global__ void __launch_bounds__(256) k_generic_psd(const float2 *__restrict__ 
 
 
 // ---- 32768 / 65536: the four-step pair (fft_fourstep.cuh), chunked so that Z stays in L2 ----
-template <int N1, int IN, int OUT>
+template <int N1, int IN, int OUT, bool WIN>
 static int launch_fourstep_chunk(jsdr_ctx *ctx, const FsArgs &fa, cudaStream_t st)
 {
     constexpr int N2 = 256;
     {
         ProfScope prof(ctx, JSDR_K_FFT, st);
-        k_fs_cols<N1, N2, IN><<<(unsigned)((long)fa.nblocks * (N2 / 16)), 256, 0, st>>>(fa);
+        k_fs_cols<N1, N2, IN, WIN><<<(unsigned)((long)fa.nblocks * (N2 / 16)), 256, 0, st>>>(fa);
         JSDR_TRY(launched(ctx, "k_fs_cols"));
     }
     ProfScope prof(ctx, JSDR_K_FFT, st);
     k_fs_rows<N1, N2, OUT><<<(unsigned)((long)fa.nblocks * (N1 / 16)), 256, 0, st>>>(fa);
     return launched(ctx, "k_fs_rows");
+}
+
+template <int N1, bool WIN>
+static int launch_fourstep_fmt(jsdr_ctx *ctx, const FsArgs &fa, int in_fmt, int out_mode, cudaStream_t st)
+{
+    if (out_mode == OUT_SPECTRUM) return launch_fourstep_chunk<N1, IN_F32, OUT_SPECTRUM, WIN>(ctx, fa, st);
+    if (in_fmt == IN_F32) return launch_fourstep_chunk<N1, IN_F32, OUT_PSD, WIN>(ctx, fa, st);
+    return launch_fourstep_chunk<N1, IN_S16, OUT_PSD, WIN>(ctx, fa, st);
 }
 
 static int launch_fourstep(jsdr_fft *f, const Args &a, int in_fmt, int out_mode, cudaStream_t st)
@@ -169,16 +180,14 @@ static int launch_fourstep(jsdr_fft *f, const Args &a, int in_fmt, int out_mode,
         fa.db_off = a.db_off;
         fa.ic = a.ic;
         fa.qc = a.qc;
+        fa.win = a.win;
         int rc;
-        if (out_mode == OUT_SPECTRUM) {
-            rc = (N1 == 128) ? launch_fourstep_chunk<128, IN_F32, OUT_SPECTRUM>(ctx, fa, cs)
-                             : launch_fourstep_chunk<256, IN_F32, OUT_SPECTRUM>(ctx, fa, cs);
-        } else if (in_fmt == IN_F32) {
-            rc = (N1 == 128) ? launch_fourstep_chunk<128, IN_F32, OUT_PSD>(ctx, fa, cs)
-                             : launch_fourstep_chunk<256, IN_F32, OUT_PSD>(ctx, fa, cs);
+        if (fa.win) {
+            rc = (N1 == 128) ? launch_fourstep_fmt<128, true>(ctx, fa, in_fmt, out_mode, cs)
+                             : launch_fourstep_fmt<256, true>(ctx, fa, in_fmt, out_mode, cs);
         } else {
-            rc = (N1 == 128) ? launch_fourstep_chunk<128, IN_S16, OUT_PSD>(ctx, fa, cs)
-                             : launch_fourstep_chunk<256, IN_S16, OUT_PSD>(ctx, fa, cs);
+            rc = (N1 == 128) ? launch_fourstep_fmt<128, false>(ctx, fa, in_fmt, out_mode, cs)
+                             : launch_fourstep_fmt<256, false>(ctx, fa, in_fmt, out_mode, cs);
         }
         JSDR_TRY(rc);
     }
@@ -205,7 +214,9 @@ static int launch_generic(jsdr_fft *f, const Args &a, int in_fmt, int out_mode, 
     }
     float2 *z0 = f->work.z[0].get(), *z1 = f->work.z[1].get();
     const long long total = (long long)a.nblocks * f->n;
-    k_generic_load<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(a.in, z0, total, in_fmt, a.ic, a.qc);
+    const unsigned grid = (unsigned)((total + 255) / 256);
+    if (a.win) k_generic_load<true><<<grid, 256, 0, st>>>(a.in, z0, total, in_fmt, a.ic, a.qc, a.win, f->n);
+    else k_generic_load<false><<<grid, 256, 0, st>>>(a.in, z0, total, in_fmt, a.ic, a.qc, nullptr, f->n);
     JSDR_TRY(launched(ctx, "k_generic_load"));
     int rc = JSDR_OK;
     float2 *res = fftg::run<float>(ctx, st, z0, z1, f->n, a.nblocks, -1, &rc);
@@ -244,6 +255,7 @@ int launch(jsdr_fft *f, const void *d_in, int in_fmt, int batch, float *d_out, i
     a.tw2 = nullptr;
     a.best = nullptr;
     a.cnt = nullptr;
+    a.win = f->win_on ? f->d_win.get() : nullptr;
     if (out_mode == OUT_SPECTRUM && in_fmt != IN_F32) {
         set_error("spectrum output needs float input");
         return JSDR_EINVAL;
@@ -315,6 +327,38 @@ try {
     }
     JSDR_CUDA(cudaStreamSynchronize(ctx->stream));
     *out = f.release();
+    return JSDR_OK;
+} JSDR_CATCH_ALL
+
+// The window is checked whole before anything is enqueued.  The first window is uploaded into a
+// buffer of its own that is installed only once the copy is enqueued; later ones are copied over
+// it on the context's stream, so that every call enqueued before this one keeps the window it was
+// enqueued with and every call after it sees the new one.  Removing the window keeps the buffer.
+extern "C" int jsdr_fft_set_window(jsdr_fft *f, const float *win)
+try {
+    JSDR_REQUIRE(f, JSDR_EINVAL, "null handle");
+    if (!win) {
+        f->win_on = false;
+        return JSDR_OK;
+    }
+    for (int t = 0; t < f->n; t++) {
+        if (!isfinite(win[t])) {
+            set_error("jsdr_fft_set_window: win[%d] = %g is not finite", t, (double)win[t]);
+            return JSDR_EINVAL;
+        }
+    }
+    jsdr_ctx *ctx = f->ctx;
+    JSDR_TRY(ctx->bind());
+    const size_t bytes = sizeof(float) * (size_t)f->n;
+    if (f->d_win) {
+        JSDR_CUDA(cudaMemcpyAsync(f->d_win.get(), win, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    } else {
+        DevBuf<float> w;
+        JSDR_TRY(w.alloc(bytes, "fft window"));
+        JSDR_CUDA(cudaMemcpyAsync(w.get(), win, bytes, cudaMemcpyHostToDevice, ctx->stream));
+        f->d_win = std::move(w);
+    }
+    f->win_on = true;
     return JSDR_OK;
 } JSDR_CATCH_ALL
 

@@ -27,6 +27,7 @@ struct FsArgs {
     int nblocks;
     float cf, db_off;
     int ic, qc;
+    const float *win;      // [N] window of jsdr_fft_set_window, read by k_fs_cols<..., true> only
 };
 
 constexpr int kFsPitch = 18;                     // float2 per 16-element row (16 + 2 pad)
@@ -49,8 +50,14 @@ __device__ __forceinline__ float2 fs_load(const FsArgs &a, long idx)
 }
 
 // grid = nblocks * N2/16 CTAs of 256 threads; thread = (g = n2 within the CTA's 16, c)
-template <int N1, int N2, int IN>
-__global__ void __launch_bounds__(256) k_fs_cols(const FsArgs a)
+// WIN: each sample times a.win[t] as it is loaded (apply_win, fft_kernels.cuh).  Left alone, ptxas
+// holds the 16 window values beside the 16 samples and the CTAs per SM drop by one (N1 = 256: 48
+// -> 50..54 registers, four CTAs instead of five); the bound keeps the CTAs per SM of the
+// unwindowed kernel: five, six for N1 = 128 with float input (40 registers there).
+template <int N1, int IN>
+constexpr int fs_cols_win_ctas() { return (N1 == 128 && IN == IN_F32) ? 6 : 5; }
+template <int N1, int N2, int IN, bool WIN = false>
+__global__ void __launch_bounds__(256, WIN ? fs_cols_win_ctas<N1, IN>() : 0) k_fs_cols(const FsArgs a)
 {
     constexpr int N = N1 * N2, R1 = N1 / 16;
     __shared__ __align__(16) float2 sm[16 * kFsGroup];
@@ -63,6 +70,10 @@ __global__ void __launch_bounds__(256) k_fs_cols(const FsArgs a)
         float2 v[16];
 #pragma unroll
         for (int m = 0; m < 16; m++) v[m] = fs_load<IN>(a, base + (long)(c + m * R1) * N2 + n2);
+        if constexpr (WIN) {
+#pragma unroll
+            for (int m = 0; m < 16; m++) v[m] = apply_win(v[m], a.win, (c + m * R1) * N2 + n2);
+        }
         Dft<16>::run(v);
         float4 *dst = reinterpret_cast<float4 *>(sm + g * kFsGroup + c * kFsPitch);
 #pragma unroll

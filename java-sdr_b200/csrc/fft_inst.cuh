@@ -8,11 +8,11 @@
 namespace jsdr {
 namespace fft {
 
-template <class P, int IN, int OUT, int SPLIT = 1>
+template <class P, int IN, int OUT, int SPLIT, bool WIN>
 static int launch_one(jsdr_ctx *ctx, const Args &a, cudaStream_t st)
 {
     static PerDeviceFlag attr_done;
-    auto kern = fft_kernel<P, IN, OUT, SPLIT>;
+    auto kern = fft_kernel<P, IN, OUT, SPLIT, WIN>;
     constexpr size_t smem = (P::PERSIST && IN == IN_S16 && SPLIT == 1) ? P::SMEM_PERSIST
                           : (P::TW_SMEM_NP && SPLIT == 1) ? P::SMEM_TW : P::SMEM;   // + twiddle tables
     JSDR_TRY(attr_done.once(ctx->device, [&]() -> int {
@@ -34,15 +34,23 @@ static int launch_one(jsdr_ctx *ctx, const Args &a, cudaStream_t st)
     return launched(ctx, "fft_kernel");
 }
 
-template <class P, int SPLIT = 1>
-static int launch_plan(jsdr_ctx *ctx, const Args &a, int in_fmt, int out_mode, cudaStream_t st)
+template <class P, int SPLIT, bool WIN>
+static int launch_fmt(jsdr_ctx *ctx, const Args &a, int in_fmt, int out_mode, cudaStream_t st)
 {
     if (out_mode == OUT_SPECTRUM) {
         if (in_fmt != IN_F32) { set_error("spectrum output needs float input"); return JSDR_EINVAL; }
-        return launch_one<P, IN_F32, OUT_SPECTRUM, SPLIT>(ctx, a, st);
+        return launch_one<P, IN_F32, OUT_SPECTRUM, SPLIT, WIN>(ctx, a, st);
     }
-    if (in_fmt == IN_F32) return launch_one<P, IN_F32, OUT_PSD, SPLIT>(ctx, a, st);
-    return launch_one<P, IN_S16, OUT_PSD, SPLIT>(ctx, a, st);
+    if (in_fmt == IN_F32) return launch_one<P, IN_F32, OUT_PSD, SPLIT, WIN>(ctx, a, st);
+    return launch_one<P, IN_S16, OUT_PSD, SPLIT, WIN>(ctx, a, st);
+}
+
+// a handle with a window (a.win set) runs the windowed instantiations of the same plan
+template <class P, int SPLIT = 1>
+static int launch_plan(jsdr_ctx *ctx, const Args &a, int in_fmt, int out_mode, cudaStream_t st)
+{
+    return a.win ? launch_fmt<P, SPLIT, true>(ctx, a, in_fmt, out_mode, st)
+                 : launch_fmt<P, SPLIT, false>(ctx, a, in_fmt, out_mode, st);
 }
 
 }  // namespace fft

@@ -428,6 +428,7 @@ struct Args {
     const float2 *tw2;          // exp(-2*pi*i*c/(2N)), c in [0, N)
     unsigned long long *best;   // [real blocks] packed (dB key, ~bin) of the halves seen so far; zero between launches
     unsigned *cnt;              // [real blocks] halves that have reported; zero between launches
+    const float *win;           // [N * SPLIT] window of jsdr_fft_set_window, read by the WIN instantiations only
 };
 
 __device__ __forceinline__ unsigned ordered_key(float v)
@@ -478,6 +479,16 @@ __device__ __forceinline__ float2 load_sample(const Args &a, long blk, int n)
     }
 }
 
+// jsdr_fft_set_window: sample t of the block times win[t], one binary32 rounding per component.
+// __fmul_rn and not '*': under nvcc's default -fmad=true ptxas may fuse a plain product into the
+// first butterfly's add, which would round once where the contract (jsdrcuda.h) rounds twice.
+// The table is the same for every block, so the loads hit in L1.
+__device__ __forceinline__ float2 apply_win(float2 v, const float *win, int t)
+{
+    const float w = __ldg(win + t);
+    return make_float2(__fmul_rn(v.x, w), __fmul_rn(v.y, w));
+}
+
 template <int R, int M>
 __device__ __forceinline__ void load_strided(float2 *v, const float2 *p)
 {
@@ -516,7 +527,9 @@ __device__ __forceinline__ void middle_pass(float2 *sm, const float2 *__restrict
 // SM that drift apart.  The block maximum is combined through one 64-bit atomicMax per half
 // (dB key in the high word, complemented bin in the low one: first strict maximum as at
 // fft.java:208-211) and the half that reports last publishes peak Hz / dB (:214-224).
-template <class P, int IN, int OUT, int SPLIT = 1>
+// WIN: every converted sample of pass 0 times a.win[t] (apply_win) before the first butterfly; a
+// handle without a window runs the WIN = false instantiations, which carry no code for it.
+template <class P, int IN, int OUT, int SPLIT = 1, bool WIN = false>
 __global__ void __launch_bounds__(P::T, P::MINB) fft_kernel(const Args a)
 {
     static_assert(SPLIT == 1 || (SPLIT == 2 && P::G == 1), "split plans take one half block per CTA");
@@ -695,6 +708,13 @@ __global__ void __launch_bounds__(P::T, P::MINB) fft_kernel(const Args a)
                             vb[i] = ldg_stream_f2(src + N + (m0 + i) * NB0);
                         }
                     }
+                    if constexpr (WIN) {                // samples n and n + N of the whole block
+#pragma unroll
+                        for (int i = 0; i < CHK; i++) {
+                            va[i] = apply_win(va[i], a.win, c + (m0 + i) * NB0);
+                            vb[i] = apply_win(vb[i], a.win, N + c + (m0 + i) * NB0);
+                        }
+                    }
                     if (h == 0) {
 #pragma unroll
                         for (int i = 0; i < CHK; i++) v[m0 + i] = cadd(va[i], vb[i]);
@@ -725,9 +745,17 @@ __global__ void __launch_bounds__(P::T, P::MINB) fft_kernel(const Args a)
                 }
 #pragma unroll
                 for (int m = 0; m < R0; m++) v[m] = s16_bits_to_float(w[m]);
+                if constexpr (WIN) {
+#pragma unroll
+                    for (int m = 0; m < R0; m++) v[m] = apply_win(v[m], a.win, c + m * NB0);
+                }
             } else {
 #pragma unroll
                 for (int m = 0; m < R0; m++) v[m] = load_sample<P, IN>(a, blk, c + m * NB0);
+                if constexpr (WIN) {
+#pragma unroll
+                    for (int m = 0; m < R0; m++) v[m] = apply_win(v[m], a.win, c + m * NB0);
+                }
             }
             Dft<R0>::run(v);
             int pos;

@@ -26,6 +26,8 @@ struct jsdr_fft {
     jsdr::DevBuf<float2> d_tw2;               // split plan: exp(-2*pi*i*c/n), c in [0, n/2)
     jsdr::DevBuf<unsigned long long> d_best;  // split plan: [max_batch] packed block maxima
     jsdr::DevBuf<unsigned> d_cnt;             // split plan: halves reported per block (zero between launches)
+    jsdr::DevBuf<float> d_win;                // [n] window of jsdr_fft_set_window (kept when the window is removed)
+    bool win_on = false;                      // the kernels multiply by d_win
     // staging for host-pointer calls (allocated on first use)
     jsdr::DevBuf<void> d_in;
     jsdr::DevBuf<float> d_out;

@@ -78,6 +78,7 @@ _SIGS = {
     "jsdr_fft_receive_f32": [_vp, _vp, _i, _vp, _vp, _i],
     "jsdr_fft_receive_s16": [_vp, _vp, _i, _i, _i, _vp, _vp, _i],
     "jsdr_fft_forward_f32": [_vp, _vp, _i, _vp, _i],
+    "jsdr_fft_set_window": [_vp, _vp],
     "jsdr_bpsk_create": [_vp, _i, _i, _vp, _i, _pp],
     "jsdr_bpsk_destroy": [_vp],
     "jsdr_bpsk_set_stages": [_vp, _i],
@@ -373,6 +374,18 @@ class fft:
         out = np.empty_like(a)
         _ck(lib().jsdr_fft_forward_f32(self.h, _ptr(a), a.shape[0], _ptr(out), MEM_HOST))
         return out.view(np.complex64).reshape(a.shape[0], self.n)
+
+    def set_window(self, win):
+        """fft.java's win[] (:72-73) applied ahead of the transform (jsdr_fft_set_window): every
+        later call multiplies sample t of each block by win[t], float[N]; None removes it.
+        Stream-ordered: device-memory calls already enqueued keep the window they were enqueued with."""
+        if win is None:
+            _ck(lib().jsdr_fft_set_window(self.h, None))
+            return
+        w = np.ascontiguousarray(win, dtype=np.float32).ravel()
+        if w.size != self.n:
+            raise ValueError("win must hold N floats")
+        _ck(lib().jsdr_fft_set_window(self.h, _ptr(w)))
 
     # device-resident entry points (bench.py)
     def receive_dev(self, d_in, batch: int, d_psd, d_peak=None, s16: bool = True, ic: int = 0, qc: int = 0):

@@ -6,6 +6,7 @@
   python tools/kbench.py demod [nchan] [S]      demod FIR+NCO and NFM / AM audio, f32 against s16 input, alternated
   python tools/kbench.py pumpdemod [nchan] [nblk] [n]   the pump with and without the demod handler, alternated
   python tools/kbench.py duty                   the reference's duty: fft + demod (NFM) + two tuners, per 100 ms block
+  python tools/kbench.py window [n ...]         FFT+PSD with and without jsdr_fft_set_window, alternated (s16 and f32)
 Prints achieved GB/s of algorithmic bytes and the fraction of MEASURED_PEAKS.json."""
 import json
 import os
@@ -462,6 +463,81 @@ def duty(rate=192000, calls=230, warm=30):
     ctx.close()
 
 
+def card():
+    """The device's name and power limit, read in the same run as the numbers they qualify."""
+    import subprocess
+    import torch
+    name = torch.cuda.get_device_name(0)
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=60).stdout.strip()
+    except Exception as e:
+        q = f"unknown ({e})"
+    return f"{name}, power limit / max SM clock: {q}"
+
+
+def window(ns, total=1 << 31, rounds=4, reps=5):
+    """jsdr_fft_set_window: the windowed FFT + PSD against the unwindowed one on the same
+    device-resident batch of `total` samples (s16 and f32 input), alternated round by round so
+    that both see the same clocks; per call the CUDA-event time of the FFT kernels (JSDR_K_FFT,
+    summed over the launches of one call) and of the whole call on the stream."""
+    print(f"window: {card()}", flush=True)
+    ctx = J.Context(0)
+    rng = np.random.default_rng(7)
+    tile = rng.integers(-20000, 20000, 1 << 25).astype(np.int16)          # 64 MB
+    res = {}
+    for n in ns:
+        batch = max(1, total // n)
+        d_in = ctx.dev_alloc(batch * n * 8)
+        for off in range(0, batch * n * 8, tile.nbytes):
+            d_in.upload(tile[: min(tile.size, (batch * n * 8 - off) // 2)], offset=off)
+        d_psd, d_pk = ctx.dev_alloc(batch * (n + 2) * 4), ctx.dev_alloc(batch * 4)
+        adsc = J.AudioDescriptor(192000)
+        plain = J.fft(ctx, None, adsc, max_batch=batch, n=n)
+        win = J.fft(ctx, None, adsc, max_batch=batch, n=n)
+        t = np.arange(n)
+        win.set_window((0.54 - 0.46 * np.cos(2.0 * np.pi * t / n)).astype(np.float32))
+        legs = {"plain": plain, "hamming": win}
+        for r in range(rounds):
+            for s16 in (True, False):
+                for name in (list(legs) if r % 2 == 0 else list(legs)[::-1]):
+                    f = legs[name]
+                    fn = lambda: f.receive_dev(d_in, batch, d_psd, d_pk, s16=s16)
+                    for _ in range(2):
+                        fn()
+                    ctx.sync()
+                    ctx.profile(True)
+                    ctx.profile_read()
+                    ctx.timer_start()
+                    for _ in range(reps):
+                        fn()
+                    ms = ctx.timer_stop_ms() / reps
+                    prof = ctx.profile_read()
+                    ctx.profile(False)
+                    kms = prof["fft"][0] / reps
+                    fmt = "s16" if s16 else "f32"
+                    res.setdefault((n, fmt, name), []).append((kms, ms))
+                    print(f"round {r} n={n:6d} batch={batch:7d} {fmt} {name:8s}: FFT kernels {kms:8.3f} ms  call {ms:8.3f} ms",
+                          flush=True)
+        for d in (d_in, d_psd, d_pk):
+            d.free()
+        plain.close()
+        win.close()
+    # (the four-step pair of 65536 runs its chunks on two streams: there the summed kernel time
+    # exceeds the call, and the call time is the one to compare)
+    print(f"summary ({total} samples per call; min .. max over {rounds} rounds of {reps} calls; {card()}):")
+    for n in ns:
+        for fmt in ("s16", "f32"):
+            for i, what in ((0, "FFT kernels"), (1, "call")):
+                p = [v[i] for v in res[(n, fmt, "plain")]]
+                w = [v[i] for v in res[(n, fmt, "hamming")]]
+                b = (total // n) * n * ((4 if fmt == "s16" else 8) + 4)
+                print(f"  n={n:6d} {fmt} {what:11s}: unwindowed {min(p):8.3f} .. {max(p):8.3f} ms   windowed {min(w):8.3f} .. "
+                      f"{max(w):8.3f} ms   ratio of minima {min(w) / min(p):.3f}   windowed {b / min(w) / 1e6:7.1f} GB/s of input + PSD",
+                      flush=True)
+    ctx.close()
+
+
 if __name__ == "__main__":
     what = sys.argv[1] if len(sys.argv) > 1 else "mix"
     if what == "mix":
@@ -481,6 +557,8 @@ if __name__ == "__main__":
         pumpdemod(*[int(x) for x in sys.argv[2:]])
     elif what == "duty":
         duty(*[int(x) for x in sys.argv[2:]])
+    elif what == "window":
+        window([int(x) for x in sys.argv[2:]] or [4096, 19200, 65536])
     else:
         fft([int(x) for x in sys.argv[2:]] or [256, 1024, 4096, 9600, 16384, 19200])
 
